@@ -2,6 +2,7 @@
 """bench.py -- compress + decompress throughput of the aligned-read coding path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..5] [--impl b200|reference] [--replicas]
+                    [--dump-outputs DIR]
 
 A step is one pass of the hot path over one batch of synthetic reads: compress the batch (K1 edit
 extraction -> K2 block coder -> container index), then decompress it (K2 block decoder -> K3 read
@@ -54,6 +55,23 @@ CFG_TEXT = {
     5: "config5: 50-250 bp reads at 30x over 15.07 Mbp, 2 % indels, soft clips, 0.5 % substitutions",
 }
 DEFAULT_SCALE = {1: 1.0, 2: 1.0, 3: 1.0, 4: 0.1, 5: 1.0}
+# --dump-outputs: elements kept per array (float32, 4 bytes each: 56 MB for both at most). Config 2's container
+# (5 054 923 bytes) is written whole; its decoded text (3 014 484 lines of 150 bases + newline, 455 MB) is sampled.
+DUMP_CAP = {"container": 6_000_000, "decoded": 8_000_000}
+DUMP_SEED = 20240601
+
+
+def dump_outputs(outdir: str, outputs: dict):
+    """Writes each uint8 array of `outputs` as <outdir>/<name>.npy in float32 (every byte value is exact there): whole when
+    it has at most DUMP_CAP[name] elements, else the elements at DUMP_CAP[name] distinct positions drawn with DUMP_SEED, in
+    ascending order, the same positions for the same length in every run. <outdir>/lengths.npy holds the full lengths, in
+    the order of `outputs`."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, arr in outputs.items():
+        if arr.size > DUMP_CAP[name]:
+            arr = arr[np.sort(np.random.default_rng(DUMP_SEED).choice(arr.size, DUMP_CAP[name], replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), arr.astype(np.float32))
+    np.save(os.path.join(outdir, "lengths.npy"), np.array([a.size for a in outputs.values()], np.float64))
 
 
 def peaks():
@@ -466,6 +484,8 @@ def run_b200_arm(args):
     dev_ms = ev0.elapsed_time(ev1)
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
+    if args.dump_outputs and rank == 0:                       # batch 0's last timed round trip, before anything below codes it again
+        dump_outputs(args.dump_outputs, {"container": codec.fetch_container(), "decoded": codec.fetch_decoded()})
     step_ms = max_over_ranks(dev_ms) / args.steps
     value = KB * total_reads / (step_ms * 1e-3)
     for k in range(KB):
@@ -781,7 +801,14 @@ def main():
     ap.add_argument("--scale", type=float, default=0.0, help="shrink the workload; default 1.0 (config 4: 0.1, stated in config.workload)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline / blocking-overhead / CLI legs")
     ap.add_argument("--no-cli", action="store_true", help="skip the file-to-file CLI leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the container and decoded text of the last one as DIR/<name>.npy "
+                         "(float32; a seeded sample where an array is larger than DUMP_CAP; rank 0's shard when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 arm computed: it needs --impl b200")
     args.warmup = max(args.warmup, 0)
     subprocess.run(["make", "-s", "-C", ROOT, "host"], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     if args.impl == "reference":

@@ -112,9 +112,8 @@ def test_single_block_stream_is_byte_identical_to_reference(codec, meta_path):
 
 def test_single_block_stream_past_the_rescale_thresholds(codec):
     """300 k reads in the one warp of the single-block mode: FLAG, POS and SNP-count models pass rescale = 2^20 several
-    times. The CPU restatement writes the reference encoder's bytes for this very input
-    (tests/test_oracle_vs_reference.py::test_live_reference_past_the_rescale_thresholds); the GPU must write them too,
-    and read them back."""
+    times. The CPU restatement wrote the reference encoder's bytes for this very input when it was checked against the
+    reference binary (DESIGN.md section 2); the GPU must write them too, and read them back."""
     cfg = synth.SynthConfig(seed=104, genome_len=1_500_000, n_reads=300_000, len_min=150, len_max=150, p_sub=0.005)
     g = synth.make_genome(cfg)
     b = synth.make_reads(cfg, g)
@@ -329,9 +328,9 @@ def test_config2_slice_roundtrip_and_resident_path(codec):
 
 
 def test_cigar_operations_beyond_midS_on_the_gpu(codec):
-    """K1 reads a CIGAR as written -- H and P skipped, = and X counted as M -- like the restatement (which is pinned to the
-    reference where the reference's own parser survives them: tests/test_oracle_vs_reference.py); a skipped region (N)
-    is an input error."""
+    """K1 reads a CIGAR as written -- H and P skipped, = and X counted as M -- like the restatement (which was checked against the
+    reference binary where the reference's own parser survives them: DESIGN.md section 2); a skipped region (N) is an
+    input error."""
     from test_oracle_vs_reference import _rewrite_cigars, _eqx_from_md
     from cbc_b200.codec import CbcgError
     g, plain = _synth(seed=131, genome_len=200_000, n_reads=6_000, len_min=100, len_max=100, p_sub=0.01, p_indel=0.004)
@@ -394,8 +393,8 @@ def test_more_distinct_flags_than_a_block_adapts(codec, n_distinct, random_head)
     distinct values -- more than a block and more than any snapshot holds; with random_head the blocks of one generation
     adapt different values, so that their merge has to drop some (F2) -- in cold, generation-primed, one-stream,
     four-substream and default-layout containers: the restatement's bytes, and the input back. The single-block mode is
-    the reference's own stream, whose model adapts every value (tests/test_oracle_vs_reference.py pins the restatement to
-    the reference binary on 700 values): byte-identical there too."""
+    the reference's own stream, whose model adapts every value (the restatement was checked against the
+    reference binary on 700 values: DESIGN.md section 2): byte-identical there too."""
     g, b0 = _synth(seed=32, genome_len=150_000, n_reads=24_000, len_min=100, len_max=100, p_sub=0.01, p_indel=0.0)
     b = _with_flags(b0, n_distinct, 8, random_head)
     codec.set_reference(g)
