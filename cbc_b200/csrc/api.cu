@@ -1005,21 +1005,6 @@ extern "C" int cbcg_encode_resident(cbcg_ctx *ctx, const cbcg_encode_opts *opts)
     cudaEventElapsedTime(&S.ms_gather, ctx->ev[3], ctx->ev[4]);
     cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[4]);
 
-    if (getenv("CBCG_BLOCK_TIMES") && !ctx->gens.empty()) {  /* with -DK2_BLOCK_TIMES: balance of the last generation */
-        const uint32_t f0 = ctx->gens.back().first, cnt = ctx->gens.back().second;
-        std::vector<double> t;
-        for (uint32_t k = f0; k < f0 + cnt; k++) if (ctx->hblocks[k].n_reads == ctx->hblocks[f0].n_reads) t.push_back((double)ctx->hblocks[k].sym_off * 1e-6);
-        std::sort(t.begin(), t.end());
-        double sum = 0; for (double x : t) sum += x;
-        double init = 0; for (uint32_t k = f0; k < f0 + cnt; k++) init += (double)ctx->hblocks[k].pa_touched * 1e-6;
-        fprintf(stderr, "[cbcg] mean block set-up (workspace, models from the snapshot, coder init): %.4f ms\n", init / cnt);
-        if (getenv("CBCG_BLOCK_DUMP")) {
-            FILE *f = fopen(getenv("CBCG_BLOCK_DUMP"), "w");
-            if (f) { for (uint32_t k = f0; k < f0 + cnt; k++) fprintf(f, "%u %u %u %llu\n", ctx->hblocks[k].n_reads, ctx->hblocks[k].n_symbols, ctx->hblocks[k].n_edits, (unsigned long long)ctx->hblocks[k].sym_off); fclose(f); }
-        }
-        if (!t.empty()) fprintf(stderr, "[cbcg] last generation, %zu full blocks of %u reads: block time mean %.3f ms, median %.3f, p90 %.3f, p99 %.3f, max %.3f ms\n",
-                                t.size(), ctx->hblocks[f0].n_reads, sum / t.size(), t[t.size() / 2], t[t.size() * 9 / 10], t[t.size() * 99 / 100], t.back());
-    }
     finish_encode(ctx, opts, legacy, fixed, n, n_edits, nb, payload_total);
     return CBCG_OK;
 }
@@ -1092,13 +1077,6 @@ static const double PIPE_MULT[PIPE_CHUNKS] = { 1.3, 1.2, 1.0, 0.6, 0.45 };
 /* a compact batch is on the device after a third of the time: the encoder no longer waits for the link, a flatter ramp
    (which the decoder still wants: small blocks decode first and their text goes out while the large ones run) */
 static const double PIPE_MULT_COMPACT[PIPE_CHUNKS] = { 1.15, 1.1, 1.0, 0.8, 0.6 };
-static bool pipe_ramp(double *hi, double *lo) {             /* CBCG_PIPE_RAMP="hi,lo": a linear ramp instead (tuning) */
-    const char *e = getenv("CBCG_PIPE_RAMP");
-    if (!e) return false;
-    double a = 0, b = 0;
-    if (sscanf(e, "%lf,%lf", &a, &b) == 2 && a >= b && b > 0.05 && a < 8.0) { *hi = a; *lo = b; return true; }
-    return false;
-}
 static int pipe_init(cbcg_ctx *ctx) {
     if (ctx->pipe_ready) return 0;
     CU(cudaStreamCreateWithFlags(&ctx->cs, cudaStreamNonBlocking));
@@ -1162,16 +1140,9 @@ static int encode_pipelined(cbcg_ctx *ctx, const BatchSrc &src, const cbcg_encod
     uint64_t slots = 0;
     cbcg_encode_opts used = *opts;
     used.block_reads = auto_block_reads(ctx, n, 1, &slots);
-    double hi = 0, lo = 0;
     std::vector<SizeStep> ramp;
-    double mult[PIPE_CHUNKS], inv = 0;
-    const bool linear = pipe_ramp(&hi, &lo);
-    for (uint32_t c = 0; c < PIPE_CHUNKS; c++) mult[c] = linear ? hi - (hi - lo) * (double)c / (double)(PIPE_CHUNKS - 1) : (src.compact ? PIPE_MULT_COMPACT[c] : PIPE_MULT[c]);
-    if (const char *e = getenv("CBCG_PIPE_MULTS")) {        /* tuning: one multiplier per chunk instead of the linear ramp */
-        double m[PIPE_CHUNKS]; int k = 0; const char *q = e;
-        while (k < (int)PIPE_CHUNKS) { char *end; m[k] = strtod(q, &end); if (end == q || m[k] < 0.05 || m[k] > 8.0) break; k++; if (*end != ',') break; q = end + 1; }
-        if (k == (int)PIPE_CHUNKS) for (uint32_t c = 0; c < PIPE_CHUNKS; c++) mult[c] = m[c];
-    }
+    const double *mult = src.compact ? PIPE_MULT_COMPACT : PIPE_MULT;
+    double inv = 0;
     for (uint32_t c = 0; c < PIPE_CHUNKS; c++) inv += PIPE_SHARE[c] / mult[c];
     /* inv > 1: more blocks than resident slots, the last ones would queue */
     for (uint32_t c = 1; c <= PIPE_CHUNKS; c++) {

@@ -83,7 +83,7 @@ struct CoderParams {
     const uint8_t *snap;                   /* snapshot S_{g-1} (snapshot_bytes(L) bytes); blocked containers always start from one */
     uint8_t *fin;                          /* per block (absolute index): its image of the small models (WarpModels), read by the merges */
     struct K2Tri *tri;                       /* encode, one-stream blocks: the symbols' intervals, written by the model kernel and coded by the
-                                              interval kernel (k2_tri_off / K2_TRI_*); NULL: the one-kernel encoder */
+                                              interval kernel (k2_tri_off / K2_TRI_*) */
 };
 struct alignas(16) K2Tri { uint32_t lo, cnt, n, flags; };   /* moved as one 16-byte word (uint4) by the kernels */
 /* Interval buffer of a two-kernel encode, in slots of 16 bytes (cumulative count, count, total, flags). Block b owns
@@ -128,10 +128,9 @@ int launch_plan(const CoderParams &p, uint32_t n_reads_total, uint64_t n_edits_t
                 uint64_t payload_cap, uint64_t *totals, cudaStream_t st,
                 const uint64_t *carry_in = nullptr, const uint64_t *n_edits_dev = nullptr);
 int launch_coder(const CoderParams &p, cudaStream_t st);
-uint32_t coder_resident_blocks(int device);     /* blocks (warps) of the encode kernel the whole GPU holds at once */
+uint32_t coder_resident_blocks(int device);     /* blocks (warps) of the warp kernel the whole GPU holds at once */
 int launch_gather(BlockDesc *blocks, uint32_t n_blocks, const uint8_t *scratch, uint8_t *out,
                   uint64_t *out_off, int blocked, uint32_t layout_mode, cudaStream_t st);   /* blocked: CBCG_BLOCK_NSUB(layout_mode, gen) pieces per block */
-uint32_t roles_launches(uint32_t mode);         /* kernel launches one launch_coder call makes for a four-substream generation */
 uint32_t coder_launches(const CoderParams &p);  /* kernel launches launch_coder(p) makes */
 uint64_t coder_ws_bytes_bound(uint32_t L, uint64_t n_reads, uint64_t n_edits, uint64_t n_blocks, int legacy, int primed);
 /* generation snapshots (gen_mode 1) */
@@ -140,7 +139,6 @@ uint64_t fin_stride_bytes(void);
 int launch_snapshot_init(uint8_t *snap, uint32_t L, cudaStream_t st);
 int launch_merge(const BlockDesc *blocks, uint32_t block_begin, uint32_t n_blocks, uint32_t L, const uint8_t *prev,
                  uint8_t *next, const uint8_t *fin, const uint8_t *ws, unsigned long long *err, uint32_t flag_target, cudaStream_t st);
-int launch_roles(const CoderParams &p, cudaStream_t st);      /* k2_blocks.cu: blocked containers, encode / decode */
 int launch_code_kernel(const CoderParams &p, cudaStream_t st); /* k2_blocks.cu: the interval half of a two-kernel encode */
 void set_carveout_all(int pct);                 /* -1: driver default per kernel; 0..100: one split for every kernel */
 int launch_copy16(void *dst, const void *src, uint64_t bytes, cudaStream_t st);

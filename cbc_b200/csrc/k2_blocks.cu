@@ -1,48 +1,14 @@
 /*
- * k2_blocks.cu -- K2 for blocked containers: the substream roles of k2_roles.cuh as kernels.
+ * k2_blocks.cu -- K2 for blocked containers, the one-thread-per-block kernels built on the scalar coder of
+ * k2_roles.cuh (K2Ac): the interval half of a two-kernel encode, and the initial generation snapshot.
  *
- * One thread per (block, substream); a warp (one CTA) holds the same substream of 32 consecutive blocks, so its lanes
- * run the same code. Encode: one launch over all four substreams (the long one, var + bases, first in the grid).
- * Decode: three launches on the same stream, {POS, FLAG} -> {match, counts} -> {var, bases} (cbcg_format.h).
- * The kernel is latency-bound integer work with a few hundred warps in flight: one warp per CTA lets the hardware
- * spread them over all SMs (one warp per scheduler runs its dependent chain at the full issue rate).
+ * The interval kernel is latency-bound integer work with a few hundred warps in flight: one warp per CTA lets the
+ * hardware spread them over all SMs (one warp per scheduler runs its dependent chain at the full issue rate).
  */
-#include <stdlib.h>
 #include "common.cuh"
 #include "k2_roles.cuh"
 
 #define K2R_LANES 32u
-
-/* grid order of the substreams of an encode launch: the longest chain (var + bases) is scheduled first */
-__constant__ uint32_t k2r_enc_order[CBCG_N_SUB] = { CBCG_SUB_EDITS, CBCG_SUB_COUNTS, CBCG_SUB_POS, CBCG_SUB_FLAG };
-
-template <int MODE>
-__global__ void __launch_bounds__(K2R_LANES)
-k2_roles_kernel(CoderParams P, uint32_t first, uint32_t n_subs) {
-    if (*reinterpret_cast<volatile unsigned long long *>(P.err)) return;    /* an earlier stage failed: offsets may be out of range */
-    const uint32_t groups = (P.n_blocks + K2R_LANES - 1u) / K2R_LANES;
-    const uint32_t which = blockIdx.x / groups;
-    const uint32_t bl = (blockIdx.x - which * groups) * K2R_LANES + threadIdx.x;
-    if (which >= n_subs || bl >= P.n_blocks) return;
-    const uint32_t q = MODE == MODE_ENC ? k2r_enc_order[which] : first + which;
-    uint64_t item = 0;
-    const int rc = k2_run_role<MODE>(P, q, P.block_begin + bl, &item);
-    if (rc) dev_set_error(P.err, rc, item);
-}
-
-int launch_roles(const CoderParams &p, cudaStream_t st) {
-    if (p.n_blocks == 0) return 0;
-    const unsigned groups = (p.n_blocks + K2R_LANES - 1u) / K2R_LANES;
-    if (p.mode == MODE_ENC) {
-        k2_roles_kernel<MODE_ENC><<<groups * CBCG_N_SUB, K2R_LANES, 0, st>>>(p, 0u, CBCG_N_SUB);
-    } else {
-        k2_roles_kernel<MODE_DEC><<<groups * 2u, K2R_LANES, 0, st>>>(p, CBCG_SUB_POS, 2u);        /* POS, FLAG */
-        k2_roles_kernel<MODE_DEC><<<groups, K2R_LANES, 0, st>>>(p, CBCG_SUB_COUNTS, 1u);
-        k2_roles_kernel<MODE_DEC><<<groups, K2R_LANES, 0, st>>>(p, CBCG_SUB_EDITS, 1u);
-    }
-    return cudaGetLastError() == cudaSuccess ? 0 : -1;
-}
-uint32_t roles_launches(uint32_t mode) { static const bool scalar = getenv("CBCG_SCALAR_ROLES") != nullptr; return (scalar && mode != MODE_ENC) ? 3u : 1u; }
 
 /* ------------------------------------------------------------------------------------------------
  * The interval half of a two-kernel encode (k2_coder.cu, k2_model_kernel): ONE THREAD PER BLOCK walks the block's
@@ -199,9 +165,7 @@ int launch_snapshot_init(uint8_t *snap, uint32_t L, cudaStream_t st) {
     k2_snapshot_init_kernel<<<1, 32, 0, st>>>(snap, L);
     return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
-void roles_set_carveout(int pct) {
-    cudaFuncSetAttribute(k2_roles_kernel<MODE_ENC>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-    cudaFuncSetAttribute(k2_roles_kernel<MODE_DEC>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+void blocks_set_carveout(int pct) {
     cudaFuncSetAttribute(k2_snapshot_init_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k2_code_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
 }

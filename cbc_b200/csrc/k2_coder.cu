@@ -134,11 +134,11 @@ __device__ __noinline__ void emit_long(BitSink *bs, uint32_t b0, uint32_t run, u
 /* TRI: the encoder's model half on its own (k2_model_kernel): every coder step is replaced by a store of the symbol's
    interval (cumulative count, count, model total) for the interval kernel (k2_code_kernel) to code. */
 #define TRI_ESC 1u                             /* on a POS interval: the escape's four byte symbols follow (in the block's escape list) */
-/* The decoder's coder step as ONE copy of code (K2_SHARED_DEC_STEP): interval update, renormalisation shape, the next
- * k + m stream bits, the tag -- 40 % of the instructions the decoder executes, which the direct call sites of the state
- * machine would otherwise each hold inline (six hot sites: a hot loop of 24 KB walked by warps that are rarely at the
- * same place, 23 % of the decoder's stall samples waiting for instruction fetch). State travels by value in registers
- * (whole-program compilation: ptxas gives a non-inlined device function its own register convention, no stack). */
+/* The decoder's coder step as ONE copy of code: interval update, renormalisation shape, the next k + m stream bits, the
+ * tag -- 40 % of the instructions the decoder executes, which the direct call sites of the state machine would otherwise
+ * each hold inline (six hot sites: a hot loop of 24 KB walked by warps that are rarely at the same place, 23 % of the
+ * decoder's stall samples waiting for instruction fetch). State travels by value in registers (whole-program
+ * compilation: ptxas gives a non-inlined device function its own register convention, no stack). */
 struct AcDecState { uint32_t l, u, t, dcnt, in_pos; uint64_t dbuf; };
 __device__ __noinline__ AcDecState ac_decode_step_shared(AcDecState s, uint32_t lo, uint32_t cnt, uint32_t n, double rn, const WarpCold *cold) {
     AcInterval a = { s.l, s.u };
@@ -319,19 +319,8 @@ struct Coder {
         a = nx;
     }
     __device__ __forceinline__ void ac_decode_step(uint32_t lo, uint32_t cnt, uint32_t n, double rn) {
-#ifdef K2_SHARED_DEC_STEP
         const AcDecState r = ac_decode_step_shared(AcDecState{ a.l, a.u, t, dcnt, in_pos, dbuf }, lo, cnt, n, rn, coldp);
         a.l = r.l; a.u = r.u; t = r.t; dcnt = r.dcnt; in_pos = r.in_pos; dbuf = r.dbuf;
-        return;
-#endif
-        ac_narrow_r(a, lo, lo + cnt, n, rn);
-        uint32_t k, bits, m; AcInterval nx;
-        ac_renorm_shape(a, k, bits, m, nx);
-        uint32_t s = k + m;                                                   /* up to 51 bits; the tag keeps the last 26 */
-        uint64_t in64 = 0;
-        do { const uint32_t take = s < 32u ? s : 32u; in64 = (in64 << take) | get_bits(take); s -= take; } while (s);
-        t = ac_tag_shift(t, k, m, (uint32_t)in64);
-        a = nx;
     }
     /* encoder_last_step (:348-364) */
     __device__ __forceinline__ void ac_flush() {
@@ -837,13 +826,8 @@ enum : uint32_t { ST_HDR, ST_READ, ST_SAMEREF, ST_RNAME, ST_RLEN0, ST_RLENK, ST_
                   ST_INDELS, ST_DEL, ST_SNPVAR, ST_SNPCHAR, ST_INSVAR, ST_INSCHAR, ST_READ_END, ST_ENDMARK, ST_DONE };
 enum : uint32_t { K_NONE, K_DENSE, K_RLENK, K_FLAG, K_POS };
 
-#ifdef K2_MAXNREG
-#define K2_KERNEL_BOUNDS __maxnreg__(K2_MAXNREG)
-#else
-#define K2_KERNEL_BOUNDS __launch_bounds__(K2_THREADS, K2_MIN_CTAS)
-#endif
 template <int MODE, bool LEGACY>
-__global__ void K2_KERNEL_BOUNDS
+__global__ void __launch_bounds__(K2_THREADS, K2_MIN_CTAS)
 k2_coder_kernel(CoderParams P) {
     __shared__ __align__(16) WarpShared sshared[K2_WARPS];
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
@@ -858,9 +842,6 @@ k2_coder_kernel(CoderParams P) {
     constexpr bool lean = !LEGACY && MODE != MODE_LIST;  /* blocked containers never code same_ref / length bytes 1..3 */
     const bool fixed = lean && P.fixed_len != 0;         /* ... nor length byte 0 when every read is L bases long */
 
-#ifdef K2_BLOCK_TIMES
-    unsigned long long k2_t0; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(k2_t0));
-#endif
     Coder<MODE> C;
     C.lane = lane; C.err = 0; C.n_symbols = 0; C.M = &sshared[warp].m; C.coldp = &sshared[warp].c;
     C.primed = primed; C.lean = lean;
@@ -896,9 +877,6 @@ k2_coder_kernel(CoderParams P) {
     if (!legacy && MODE != MODE_LIST && !primed) C.init_L_models();
     if (!legacy && MODE == MODE_DEC && B.chr >= P.genome.n_chr) C.err = CBCG_ERR_NO_REFERENCE;
 
-#ifdef K2_BLOCK_TIMES
-    unsigned long long k2_t_init; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(k2_t_init));
-#endif
     /* ---- machine state */
     uint32_t state = legacy ? ST_HDR : ST_READ;
     uint32_t k = 0;                                      /* sub-index inside a state (header byte, edit ordinal ...) */
@@ -1275,9 +1253,6 @@ M_DONE:
         if (lane < C.pos_card) { C.pos_gval()[lane] = C.pos_rv; C.pos_gcnt()[lane] = C.pos_rc; }
         if (lane == 0) { B.pos_card = C.pos_card; B.n_rows = C.n_rows; B.pa_touched = C.pa_init ? 1u : 0u; }
     }
-#ifdef K2_BLOCK_TIMES                                       /* experiment: how long each block took (ns), for the balance of a generation */
-    if (lane == 0 && MODE != MODE_LIST) { unsigned long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1)); B.sym_off = t1 - k2_t0; if (!P.fin) B.pa_touched = (uint32_t)(k2_t_init - k2_t0); }
-#endif
     if (lane == 0) {
         B.n_symbols = (MODE == MODE_LIST) ? C.list_n : C.n_symbols;
         if (MODE == MODE_ENC) { B.payload_bytes = C.out_pos; B.sub_bytes[0] = C.out_pos; }
@@ -1299,12 +1274,9 @@ M_DONE:
  * follow one read behind them, the edits one read behind the counts; a block takes the time of its longest substream
  * instead of their sum. Lanes cooperate inside a symbol exactly as in round 1 (Coder<>: strided cumulative counts,
  * 32-wide hash probe, POS slots in registers). The block's small models live once in shared memory, each field
- * owned by one role. The scalar twin of these loops (k2_roles.cuh) is what the CPU harness checks against the oracle
- * and what CBCG_SCALAR_ROLES=1 runs on the GPU as a cross-check. */
+ * owned by one role. The scalar twin of these loops (k2_roles.cuh) is what the CPU harness checks against the oracle. */
 #define K2B_WARPS 4u
-#ifndef K2B_MIN_CTAS
 #define K2B_MIN_CTAS 5
-#endif
 #define K2B_RING 256u
 struct K2BEntry { uint32_t pos, flaglen, counts; };
 struct K2BShared {
@@ -1630,9 +1602,9 @@ int launch_block_kernel(const CoderParams &p, cudaStream_t st) {
  * Encode of one-stream blocks in TWO KERNELS: models (here), then intervals (k2_code_kernel, k2_blocks.cu).
  *
  * An encoder knows every symbol and every context before it codes anything: the adaptive models (stream_model.c
- * :31-76) never look at the coder's interval, only the coder (Arithmetic_stream.c:274-345) does. The one-kernel encoder
- * above runs both behind each other, 175 warp instructions per symbol, all 32 lanes repeating the interval arithmetic,
- * every block one chain of ~4 700 dependent symbols. Here
+ * :31-76) never look at the coder's interval, only the coder (Arithmetic_stream.c:274-345) does. The warp kernel above,
+ * as a one-kernel encoder, ran both behind each other, 175 warp instructions per symbol, all 32 lanes repeating the
+ * interval arithmetic, every block one chain of ~4 700 dependent symbols. Here
  *   - the model half runs as FOUR INDEPENDENT CHAINS per block (POS | length + FLAG | match + counts | var + bases: the
  *     model groups of cbcg_format.h), a warp each, lanes cooperating inside a symbol as before; a chain is a short loop
  *     over one kind of symbol -- no state machine, no interval arithmetic, no bit packer -- and writes each symbol's
@@ -1640,12 +1612,10 @@ int launch_block_kernel(const CoderParams &p, cudaStream_t st) {
  *     (slot = running sum over the reads' symbol counts, which every chain forms for itself from the records);
  *   - the interval half is one THREAD per block: 32 blocks per warp run the same ~60 instructions per symbol on
  *     different data (closed-form renormalisation: no data-dependent loop), reading their slots in order.
- * Same models, same order, same intervals: the container is byte-identical to the one-kernel encoder's (and to the
- * oracle's). POS escapes are the one symbol whose presence the other chains cannot know: the POS triple carries a flag
- * and the four byte symbols go to an escape list that the interval kernel splices in. */
-#ifndef K2M_MIN_CTAS
+ * Same models, same order, same intervals: the container is byte-identical to the oracle's. POS escapes are the one
+ * symbol whose presence the other chains cannot know: the POS triple carries a flag and the four byte symbols go to an
+ * escape list that the interval kernel splices in. */
 #define K2M_MIN_CTAS 8
-#endif
 /* chains of a block: POS | length + FLAG | match + counts | edit positions + bases (CBCG_SUB_*; the grid runs them from
    the last to the first: the longest chain is scheduled first) */
 #define K2M_ROLES      CBCG_N_SUB
@@ -2080,7 +2050,8 @@ static int launch_split_encode(const CoderParams &p, cudaStream_t st) {
 uint32_t coder_resident_blocks(int device) {
     int sms = 0, per_sm = 0;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) return 148u * 16u;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k2_coder_kernel<MODE_ENC, false>, (int)K2_THREADS, 0) != cudaSuccess || per_sm <= 0) per_sm = K2_MIN_CTAS;
+    /* the blocked warp decoder: its launch bounds and shared memory, and so its occupancy, are the warp encoder's */
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k2_coder_kernel<MODE_DEC, false>, (int)K2_THREADS, 0) != cudaSuccess || per_sm <= 0) per_sm = K2_MIN_CTAS;
     if (per_sm > 5) per_sm = 5;                              /* the cut (and with it the container) does not follow a build with more resident CTAs */
     return (uint32_t)sms * (uint32_t)per_sm * K2_WARPS;
 }
@@ -2102,51 +2073,41 @@ __global__ void merge_var_finish_kernel(MergeParams P);
  * kernel on the same split; one-stream calls keep the driver's choices, which are 0.3 ms better for the block coder. */
 void extract_set_carveout(int pct);        /* k1_extract.cu */
 void reconstruct_set_carveout(int pct);    /* k3_reconstruct.cu */
-void roles_set_carveout(int pct);          /* k2_blocks.cu */
+void blocks_set_carveout(int pct);         /* k2_blocks.cu */
 void unpack_set_carveout(int pct);         /* k0_unpack.cu */
 template <class K> static void set_carveout(K kernel, int pct) { cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct); }
 /* pct = -1: every kernel gets the split the driver prefers for it (best for each kernel on its own: the one-stream
  * calls); 0..100: that share of shared memory for all of them (the pipelined calls). */
 void set_carveout_all(int pct) {
     static int current = -1;
-    const char *e = getenv("CBCG_CARVEOUT");               /* tuning: force one value everywhere */
-    if (e) pct = atoi(e);
     if (pct == current) return;
     current = pct;
-    set_carveout(k2_coder_kernel<MODE_ENC, false>, pct); set_carveout(k2_coder_kernel<MODE_DEC, false>, pct); set_carveout(k2_coder_kernel<MODE_LIST, false>, pct);
+    set_carveout(k2_coder_kernel<MODE_DEC, false>, pct); set_carveout(k2_coder_kernel<MODE_LIST, false>, pct);
     set_carveout(k2_block_kernel<MODE_ENC>, pct); set_carveout(k2_block_kernel<MODE_DEC>, pct); set_carveout(k2_model_kernel<true>, pct); set_carveout(k2_model_kernel<false>, pct);
     set_carveout(k2_coder_kernel<MODE_ENC, true>, pct); set_carveout(k2_coder_kernel<MODE_DEC, true>, pct); set_carveout(k2_coder_kernel<MODE_LIST, true>, pct);
     set_carveout(k2_plan_kernel, pct); set_carveout(k2_payload_scan_kernel, pct); set_carveout(k2_gather_kernel, pct);
     set_carveout(snapshot_copy_kernel, pct);
     set_carveout(merge_prep_kernel, pct); set_carveout(merge_add_kernel, pct); set_carveout(merge_finish_kernel, pct); set_carveout(merge_var_finish_kernel, pct);
-    extract_set_carveout(pct); reconstruct_set_carveout(pct); roles_set_carveout(pct); unpack_set_carveout(pct);
+    extract_set_carveout(pct); reconstruct_set_carveout(pct); blocks_set_carveout(pct); unpack_set_carveout(pct);
 }
 
-static bool split_encode(const CoderParams &p) {
-    static const bool one_kernel = getenv("CBCG_ONE_KERNEL_ENCODE") != nullptr;   /* cross-check: the one-kernel encoder */
-    return !one_kernel && !p.legacy && p.mode == MODE_ENC && p.tri && p.primed && p.n_sub <= 1u;
-}
+static bool split_encode(const CoderParams &p) { return !p.legacy && p.mode == MODE_ENC && p.n_sub <= 1u; }
 uint32_t coder_launches(const CoderParams &p) {
     if (p.n_blocks == 0) return 0u;
-    if (!p.legacy && p.mode != MODE_LIST && p.n_sub > 1u) return roles_launches(p.mode);
     return split_encode(p) ? 2u : 1u;
 }
 int launch_block_kernel(const CoderParams &p, cudaStream_t st);
 int launch_coder(const CoderParams &p, cudaStream_t st) {
     if (p.n_blocks == 0) return 0;
-    if (!p.legacy && p.mode != MODE_LIST && p.n_sub > 1u) { /* four-substream containers: a CTA per block, a warp per substream */
-        static const bool scalar = getenv("CBCG_SCALAR_ROLES") != nullptr;   /* cross-check: the scalar twin (k2_blocks.cu) */
-        return scalar ? launch_roles(p, st) : launch_block_kernel(p, st);
-    }
-    if (split_encode(p)) return launch_split_encode(p, st);
+    if (!p.legacy && p.mode != MODE_LIST && p.n_sub > 1u) return launch_block_kernel(p, st);   /* four-substream containers: a CTA per block, a warp per substream */
+    if (split_encode(p)) return p.tri ? launch_split_encode(p, st) : -1;                      /* no interval buffer: a caller bug */
     const unsigned grid = (p.n_blocks + K2_WARPS - 1) / K2_WARPS;
     if (p.legacy) {
         if (p.mode == MODE_ENC) k2_coder_kernel<MODE_ENC, true><<<grid, K2_THREADS, 0, st>>>(p);
         else if (p.mode == MODE_DEC) k2_coder_kernel<MODE_DEC, true><<<grid, K2_THREADS, 0, st>>>(p);
         else k2_coder_kernel<MODE_LIST, true><<<grid, K2_THREADS, 0, st>>>(p);
     } else {
-        if (p.mode == MODE_ENC) k2_coder_kernel<MODE_ENC, false><<<grid, K2_THREADS, 0, st>>>(p);
-        else if (p.mode == MODE_DEC) k2_coder_kernel<MODE_DEC, false><<<grid, K2_THREADS, 0, st>>>(p);
+        if (p.mode == MODE_DEC) k2_coder_kernel<MODE_DEC, false><<<grid, K2_THREADS, 0, st>>>(p);
         else k2_coder_kernel<MODE_LIST, false><<<grid, K2_THREADS, 0, st>>>(p);
     }
     return cudaGetLastError() == cudaSuccess ? 0 : -1;

@@ -1,6 +1,6 @@
 /*
- * k2_layout.h -- memory layouts of the block coder shared by its kernels (k2_coder.cu: the single-block / symbol-list
- * warp kernel; k2_blocks.cu: the substream roles of blocked containers), the generation merges and the host API:
+ * k2_layout.h -- memory layouts of the block coder shared by its kernels (k2_coder.cu: the warp kernels; k2_blocks.cu:
+ * the interval kernel of a two-kernel encode), its scalar twin (k2_roles.cuh), the generation merges and the host API:
  * per-block model workspace, per-block image of the small models, generation snapshot. Plain C++ (host + device).
  */
 #pragma once
@@ -14,33 +14,20 @@
 #define K2_HD inline
 #endif
 
-#ifndef K2_WARPS
 #define K2_WARPS    4u
-#endif
-#ifndef K2_MIN_CTAS
 #define K2_MIN_CTAS 5          /* resident CTAs per SM the register allocation is held to: 96 registers, no spills
                                   (cold per-warp values live in shared memory, WarpCold); 6 spills and is slower */
-#endif
 #define K2_THREADS  (K2_WARPS * 32u)
-#ifndef K2_INLINE_DEC_STEP
-#define K2_SHARED_DEC_STEP 1   /* the decoder's coder step as one non-inlined copy (k2_coder.cu, ac_decode_step_shared); -DK2_INLINE_DEC_STEP: inline at every site */
-#endif
 #define LIKELY(c)   __builtin_expect(!!(c), 1)
 #define UNLIKELY(c) __builtin_expect(!!(c), 0)
-#ifndef FLAG_CAP
 #define FLAG_CAP    CBCG_FLAG_ADAPT_MAX   /* distinct FLAG values a block / a snapshot adapts (the sparse table's size, a format constant: rules F1 / F2 in cbcg_format.h; 128 -> 256 measured time-neutral) */
-#endif
 #define PA_STRIDE   260u              /* words per 256-symbol model row: 256 counts, n, padding to 16 bytes */
 #define VAR_DIRECT_MIN_EDITS 32768u       /* blocks with more edits index var rows directly by context */
 #define VAR_DEFERRED 0x80000000u           /* hash value: row not built yet, low 16 bits = the one symbol coded in it */
 
 enum { MODE_ENC = 0, MODE_DEC = 1, MODE_LIST = 2 };
 
-#ifdef K2_FENCE
-#define SYNCW() do { __syncwarp(); __threadfence_block(); } while (0)
-#else
 #define SYNCW() __syncwarp()
-#endif
 
 /* ------------------------------------------------------------------------------------------------
  * per-block workspace layout in HBM (u32 units unless noted) */

@@ -10,19 +10,16 @@
  *                        compute_delta_to_first_snp :703-718
  *   read_decompression.c decompress_read :59-86 and the decoding half of reconstruct_read :339-458
  *
- * Why scalar. Round 1 ran one warp per block with all 32 lanes carrying the same coder: 175 (encode) / 209 (decode)
- * warp instructions per symbol, every block one serial chain through all models, and the kernel was bound by
- * instruction issue at 55 % of the slots. Here a block's symbols are split by model group into four independent
- * arithmetic-coded substreams (POS | FLAG | match + counts | var + bases), and each (block, substream) is coded by ONE
- * THREAD: a warp holds the same substream of 32 different blocks, so its lanes run the same code on different data
- * (the rare paths -- POS escapes, rescales, row builds -- diverge briefly) and a warp instruction does 32 coder steps'
- * worth of work instead of one. Encode: all (block, substream) pairs are independent, one launch. Decode: three
- * launches, {POS, FLAG} -> {match, counts} -> {var, bases}: the match context needs samePos, the edit loops need the
- * counts, and the base context needs the reference base under the decoded position. Models live where the merge
- * kernels expect them (the block's WarpModels image, its workspace: k2_layout.h) and are reached through L1.
+ * A block's symbols are split by model group into four independent arithmetic-coded substreams (POS | FLAG |
+ * match + counts | var + bases), and each (block, substream) is coded here by one scalar coder. Encode: the four are
+ * independent. Decode runs {POS, FLAG} -> {match, counts} -> {var, bases}: the match context needs samePos, the edit
+ * loops need the counts, and the base context needs the reference base under the decoded position. Models live where
+ * the merge kernels expect them (the block's WarpModels image, its workspace: k2_layout.h).
  *
- * Everything here is plain scalar C++ marked host + device: tests/native/test_k2_roles.cpp runs the very same code on
- * the CPU against the oracle's containers (the warp-cooperative round-1 coder could only be checked on a GPU).
+ * Everything here is plain scalar C++ marked host + device. It is the reference the GPU's substream kernels are held
+ * to: tests/native/test_k2_roles.cpp runs it on the CPU against the oracle's containers (the warp-cooperative kernels
+ * can only be checked on a GPU). On the device, the interval kernel of a two-kernel encode (k2_blocks.cu) codes with
+ * K2Ac, and k2_snapshot_init writes the initial generation snapshot.
  */
 #pragma once
 #include <string.h>
