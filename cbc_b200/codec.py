@@ -41,7 +41,42 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_encode", "cbcg_encode_bound", "cbcg_decode", "cbcg_decoded_size", "cbcg_decode_edits",
            "cbcg_reconstruct", "cbcg_batch_upload", "cbcg_encode_resident", "cbcg_decode_resident",
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
-           "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack"]
+           "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
+           "cbcg_region_plan", "cbcg_decode_region"]
+
+
+UINT64_MAX = (1 << 64) - 1
+
+
+class Region(C.Structure):
+    """Mirror of ``cbcg_region`` (include/cbcg.h): 1-based, both ends inclusive; end UINT64_MAX = to the end of the record."""
+    _fields_ = [("name", C.c_char_p), ("start", C.c_uint64), ("end", C.c_uint64)]
+
+
+def _region_array(regions):
+    """(name,), (name, start) or (name, start, end) tuples -> a ctypes array of Region (the names stay referenced by it)."""
+    regions = list(regions)
+    arr = (Region * max(len(regions), 1))()
+    for k, r in enumerate(regions):
+        name = r[0].encode() if isinstance(r[0], str) else bytes(r[0])
+        start = int(r[1]) if len(r) > 1 else 1
+        end = int(r[2]) if len(r) > 2 else UINT64_MAX
+        arr[k] = Region(name, start, end)
+    return arr, len(regions)
+
+
+def region_plan(data: bytes, regions, legacy: bool = False) -> dict:
+    """What ``Codec.decompress_region`` would decode, from the container's header and block index alone (no device):
+    n_blocks, n_reads (decoded, not returned), payload_bytes read and max_seq_bytes (a bound on the text returned).
+    A legacy stream does not store its read count: n_reads and max_seq_bytes are UINT64_MAX there."""
+    lib = load_library()
+    src = np.frombuffer(data, np.uint8)
+    arr, n = _region_array(regions)
+    out = [C.c_uint64(0) for _ in range(4)]
+    rc = lib.cbcg_region_plan(src.ctypes.data, src.nbytes, int(legacy), arr, n, *[C.byref(v) for v in out])
+    if rc:
+        raise CbcgError(rc, lib.cbcg_strerror(rc).decode())
+    return dict(zip(("n_blocks", "n_reads", "payload_bytes", "max_seq_bytes"), (v.value for v in out)))
 
 
 class EncodeOpts(C.Structure):
@@ -108,6 +143,8 @@ def load_library():
         lib.cbcg_cigar_bound.argtypes = [P(CBatch)]; lib.cbcg_cigar_bound.restype = u64
         lib.cbcg_cigar_pack.argtypes = [vp, P(CBatch), vp, u64, P(u64)]
         lib.cbcg_cigar_unpack.argtypes = [vp, vp, u64, C.c_int, vp, u64, vp, u64, P(u64), P(u64)]
+        lib.cbcg_region_plan.argtypes = [vp, u64, C.c_int, P(Region), u32, P(u64), P(u64), P(u64), P(u64)]
+        lib.cbcg_decode_region.argtypes = [vp, vp, u64, C.c_int, P(Region), u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -301,6 +338,28 @@ class Codec:
                 rc = self.lib.cbcg_fetch_decoded(self.h, out.ctypes.data, out.nbytes, C.byref(n))
             self._check(rc)
             return out[:n.value].tobytes(), nr.value
+
+    def decompress_region(self, data: bytes, regions, legacy: bool = False) -> Tuple[bytes, np.ndarray]:
+        """The reads that overlap at least one region, each once, in container order: (SEQ + '\\n' per read, their
+        ordinals in the container as uint64). regions: (name,), (name, start) or (name, start, end), 1-based, inclusive."""
+        src = np.frombuffer(data, np.uint8)
+        arr, n_regions = _region_array(regions)
+        if legacy:
+            size, n_ids = 1 << 20, 1 << 16
+        else:
+            p = region_plan(data, regions)
+            size, n_ids = p["max_seq_bytes"], p["n_reads"]
+        while True:
+            out = np.empty(max(size, 1), np.uint8)
+            ids = np.empty(max(n_ids, 1), np.uint64)
+            n, nr = C.c_uint64(0), C.c_uint64(0)
+            rc = self.lib.cbcg_decode_region(self.h, src.ctypes.data, src.nbytes, int(legacy), arr, n_regions,
+                                             out.ctypes.data, out.nbytes, C.byref(n), ids.ctypes.data, ids.size, C.byref(nr))
+            if rc == -5 and (n.value > out.nbytes or nr.value > ids.size):
+                size, n_ids = max(size, n.value), max(n_ids, nr.value)
+                continue
+            self._check(rc)
+            return out[:n.value].tobytes(), ids[:nr.value].copy()
 
     def cigar_pack(self, batch: Batch) -> bytes:
         """The CIGAR side section of a batch (SURVEY.md 8f row 4, cbcg.h): reads whose CIGAR is not the one their indels

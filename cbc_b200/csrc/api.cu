@@ -41,6 +41,7 @@ struct Words {
     uint32_t ticket;
     uint32_t pad;
     uint64_t chain[2];                        /* pipelined encode: edit entries so far, ping-pong between K1 launches */
+    uint64_t n_selected;                      /* region decode: reads K5 kept */
 };
 
 struct cbcg_ctx {
@@ -79,6 +80,7 @@ struct cbcg_ctx {
     DevBuf recs, edits, chr_out, tile_desc, words, blocks, ws, scratch, payload, out_off, symbols, seq_out;
     DevBuf cig_cls, cig_exc, cig_out;          /* CIGAR recovery (k4_cigar.cu): classes, verbatim texts, emitted text */
     DevBuf tri;                                /* two-kernel encode: the symbols' intervals between the model and the interval kernel */
+    DevBuf reg, sel_recs, sel_chr, sel_ids;    /* region decode (k5_region.cu): intervals + ordinal runs, and the kept reads */
     DevBuf snap_a, snap_b, fin;                /* generation snapshots and per-block final states (gen_mode 1) */
     std::vector<std::pair<uint32_t, uint32_t>> gens;   /* (first block, block count) per generation of the last cut */
     uint32_t layout = 1;                       /* the call in progress: 1 = one stream per block, 4 = four substreams, 0 = four in the narrow early generations */
@@ -206,7 +208,8 @@ extern "C" void cbcg_destroy(cbcg_ctx *ctx) {
     if (ctx->hw) cudaFreeHost(ctx->hw);
     if (ctx->hblocks) cudaFreeHost(ctx->hblocks);
     if (ctx->h_tile) cudaFreeHost(ctx->h_tile);
-    for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec }) free_buf(*d);
+    for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec,
+                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids }) free_buf(*d);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->mark) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->kev) if (e) cudaEventDestroy(e);
@@ -1471,12 +1474,13 @@ static uint32_t ref_window_from_blocks(const cbcg_ctx *ctx, uint32_t max_len) {
     return want > 1e9 ? 0u : (uint32_t)want;
 }
 /* fixed_len != 0: every record is that long (CBCG_MODE_FIXED_LEN container, or checked by the caller). */
-static int run_reconstruct(cbcg_ctx *ctx, uint64_t n_reads, uint32_t max_len, uint32_t fixed_len, const uint32_t *chr_dev, uint32_t ref_cap_hint = 0) {
+static int run_reconstruct(cbcg_ctx *ctx, uint64_t n_reads, uint32_t max_len, uint32_t fixed_len, const uint32_t *chr_dev, uint32_t ref_cap_hint = 0,
+                           const cbcg_read_rec *recs_dev = nullptr) {
     const uint64_t out_cap = n_reads * ((uint64_t)max_len + 1u);
     TRY(ensure(ctx, ctx->seq_out, out_cap + 64));
     TRY(ensure(ctx, ctx->tile_desc, (reconstruct_num_tiles(n_reads) + 1) * 8));
     CU(cudaMemsetAsync(wptr<unsigned long long>(ctx, W_OFF(err)), 0, 8, ctx->st));
-    if (launch_reconstruct(n_reads, ctx->recs.as<cbcg_read_rec>(), chr_dev, ctx->edits.as<uint16_t>(), ctx->dg,
+    if (launch_reconstruct(n_reads, recs_dev ? recs_dev : ctx->recs.as<cbcg_read_rec>(), chr_dev, ctx->edits.as<uint16_t>(), ctx->dg,
                            ctx->seq_out.as<uint8_t>(), out_cap, max_len, fixed_len, ctx->tile_desc.as<uint64_t>(),
                            wptr<uint32_t>(ctx, W_OFF(ticket)), wptr<uint64_t>(ctx, W_OFF(total_bytes)),
                            wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st, ctx->kev[2], ctx->kev[3], ref_cap_hint))
@@ -1795,6 +1799,252 @@ extern "C" int cbcg_decode_edits(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_l
     if (nr && chr) CU(cudaMemcpyAsync(chr, ctx->chr_out.p, nr * 4, cudaMemcpyDeviceToHost, ctx->st));
     if (ne && edits) CU(cudaMemcpyAsync(edits, ctx->edits.p, ne * 2, cudaMemcpyDeviceToHost, ctx->st));
     CU(cudaStreamSynchronize(ctx->st));
+    return CBCG_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------ region decode
+ * cbcg_region_plan / cbcg_decode_region (DESIGN.md, "Region decode"). The blocks of generation g start from the snapshot
+ * that merges every block of the generations before g, so the blocks a query touches are decoded after every block of
+ * every generation before the latest touched one (g*), and of g* only the touched blocks are. One host routine walks the
+ * header and the index once and returns that selection; the decode hands it to the block decoder as a reduced descriptor
+ * table (each block keeps its generation, the FLAG target comes from the whole index), K5 keeps the reads that overlap
+ * a region and K3 rebuilds only those. */
+static int check_regions(cbcg_ctx *ctx, const cbcg_region *regions, uint32_t n_regions) {
+    if (!regions || !n_regions) return fail(ctx, CBCG_ERR_ARG, "no regions");
+    for (uint32_t k = 0; k < n_regions; k++)
+        if (!regions[k].name || regions[k].start == 0 || regions[k].start > regions[k].end)
+            return fail(ctx, CBCG_ERR_ARG, "region %u: NULL name, start 0 or start > end", k);
+    return 0;
+}
+/* sorted by (chr, start), overlapping or adjacent intervals merged: their ends ascend too */
+static void merge_intervals(std::vector<RegionIv> &iv) {
+    std::sort(iv.begin(), iv.end(), [](const RegionIv &a, const RegionIv &b) { return a.chr != b.chr ? a.chr < b.chr : a.start < b.start; });
+    size_t n = 0;
+    for (size_t k = 0; k < iv.size(); k++) {
+        if (n && iv[n - 1].chr == iv[k].chr && (iv[n - 1].end == UINT64_MAX || iv[k].start <= iv[n - 1].end + 1)) {
+            iv[n - 1].end = std::max(iv[n - 1].end, iv[k].end);
+            continue;
+        }
+        iv[n++] = iv[k];
+    }
+    iv.resize(n);
+}
+/* the regions whose name is in `names`, by ordinal into it; other names match nothing */
+static std::vector<RegionIv> region_intervals(const cbcg_region *regions, uint32_t n_regions, const std::vector<std::string> &names) {
+    std::vector<RegionIv> iv;
+    for (uint32_t k = 0; k < n_regions; k++) {
+        const size_t nl = strlen(regions[k].name);
+        for (size_t g = 0; g < names.size(); g++)
+            if (names[g].size() == nl && !memcmp(names[g].data(), regions[k].name, nl)) { iv.push_back({ (uint32_t)g, 0u, regions[k].start, regions[k].end }); break; }
+    }
+    merge_intervals(iv);
+    return iv;
+}
+
+struct RegionPlan {
+    Container c;
+    std::vector<BlockDesc> blocks;             /* the whole index (container chromosome ordinals); first_read / payload_off within the container */
+    std::vector<uint32_t> sel;                 /* blocks to decode, ascending */
+    std::vector<RegionIv> iv;                  /* the regions by container chromosome ordinal */
+    uint32_t max_block_reads = 0;              /* longest block of the whole index: the FLAG target of the merged snapshots */
+    uint64_t n_reads = 0, n_edits = 0, payload_bytes = 0, max_seq_bytes = 0;
+};
+
+/* Header + index -> the blocks to decode. A block's reads start within [its base_pos, the next block's base_pos on the same
+ * chromosome] (no upper bound for a chromosome's last block), and a read that starts up to max_len + 255 bases before a
+ * region (<= 255 deletions per read) can still reach into it: the selection is generous, K5 is exact. Reads no payload. */
+static int plan_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, const cbcg_region *regions, uint32_t n_regions, RegionPlan &P,
+                       const std::vector<std::string> *genome = nullptr) {   /* genome: fills P.c.chr_map */
+    TRY(check_regions(ctx, regions, n_regions));
+    Container &c = P.c;
+    if (parse_container(in, in_len, genome, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
+    std::vector<std::string> names(c.n_chr);
+    for (uint64_t o = 40, k = 0; k < c.n_chr; k++) {           /* parse_container has checked the name table */
+        const uint32_t nl = rd32(in + o); o += 4;
+        names[k].assign(reinterpret_cast<const char *>(in + o), nl);
+        o += nl + ((4 - (nl & 3)) & 3);
+    }
+    P.iv = region_intervals(regions, n_regions, names);
+    P.blocks.resize(c.n_blocks);
+    IndexState st = index_state(c.block_reads);
+    uint64_t o = c.index_off, first = 0, pay = 0;
+    uint32_t prev_gen = 0;
+    for (uint32_t k = 0; k < c.n_blocks; k++) {
+        BlockDesc &b = P.blocks[k];
+        if (!index_get(in, c.index_off + c.index_bytes, o, st, b, c.layout_mode)) return fail(ctx, CBCG_ERR_FORMAT, "block index entry %u malformed", k);
+        if (b.chr >= c.n_chr) return fail(ctx, CBCG_ERR_FORMAT, "block %u names chromosome %u of %u", k, b.chr, c.n_chr);
+        if (b.gen < prev_gen || (c.gen_mode == 0 && b.gen != 0)) return fail(ctx, CBCG_ERR_FORMAT, "block %u: bad generation %u", k, b.gen);
+        prev_gen = b.gen;
+        b.first_read = (uint32_t)first; b.payload_off = pay;
+        first += b.n_reads; pay += b.payload_bytes;
+        P.max_block_reads = std::max(P.max_block_reads, b.n_reads);
+    }
+    if (first != c.n_reads) return fail(ctx, CBCG_ERR_FORMAT, "index holds %llu reads, header says %llu", (unsigned long long)first, (unsigned long long)c.n_reads);
+    if (c.payload_off + pay > in_len) return fail(ctx, CBCG_ERR_FORMAT, "payload truncated");
+    const uint64_t reach = (uint64_t)c.max_len + 255u;
+    std::vector<uint8_t> touched(c.n_blocks, 0);
+    bool any = false;
+    uint32_t g_star = 0;
+    for (uint32_t k = 0; k < c.n_blocks; k++) {
+        const BlockDesc &b = P.blocks[k];
+        const uint64_t lo = b.base_pos;
+        const uint64_t hi = (k + 1 < c.n_blocks && P.blocks[k + 1].chr == b.chr) ? P.blocks[k + 1].base_pos : UINT64_MAX;
+        /* the first interval of this chromosome that ends at or after lo: the only one that can start too early to matter */
+        const auto it = std::lower_bound(P.iv.begin(), P.iv.end(), b, [&](const RegionIv &v, const BlockDesc &) {
+            return v.chr < b.chr || (v.chr == b.chr && v.end < lo); });
+        if (it == P.iv.end() || it->chr != b.chr) continue;
+        if (hi != UINT64_MAX && hi + reach <= it->start) continue;
+        touched[k] = 1; any = true; g_star = std::max(g_star, b.gen);
+    }
+    uint64_t touched_reads = 0;
+    for (uint32_t k = 0; any && k < c.n_blocks; k++) {
+        const BlockDesc &b = P.blocks[k];
+        if (b.gen > g_star || (b.gen == g_star && !touched[k])) continue;
+        P.sel.push_back(k);
+        P.n_reads += b.n_reads; P.n_edits += b.n_edits; P.payload_bytes += b.payload_bytes;
+        if (touched[k]) touched_reads += b.n_reads;
+    }
+    P.max_seq_bytes = touched_reads * ((uint64_t)c.max_len + 1u);
+    return 0;
+}
+
+extern "C" int cbcg_region_plan(const uint8_t *in, uint64_t in_len, int legacy, const cbcg_region *regions, uint32_t n_regions,
+                                uint64_t *n_blocks, uint64_t *n_reads, uint64_t *payload_bytes, uint64_t *max_seq_bytes) {
+    for (uint64_t *p : { n_blocks, n_reads, payload_bytes, max_seq_bytes }) if (p) *p = 0;
+    if (legacy) {                                            /* one block, decoded whole; the stream does not store its read count */
+        TRY(check_regions(nullptr, regions, n_regions));
+        if (!in || in_len < 4) return CBCG_ERR_FORMAT;
+        if (n_blocks) *n_blocks = 1;
+        if (n_reads) *n_reads = UINT64_MAX;
+        if (payload_bytes) *payload_bytes = in_len;
+        if (max_seq_bytes) *max_seq_bytes = UINT64_MAX;
+        return CBCG_OK;
+    }
+    RegionPlan P;
+    TRY(plan_region(nullptr, in, in_len, regions, n_regions, P));
+    if (n_blocks) *n_blocks = P.sel.size();
+    if (n_reads) *n_reads = P.n_reads;
+    if (payload_bytes) *payload_bytes = P.payload_bytes;
+    if (max_seq_bytes) *max_seq_bytes = P.max_seq_bytes;
+    return CBCG_OK;
+}
+
+/* K5 over the nr decoded records in ctx->recs / ctx->chr_out: the kept reads -> ctx->sel_*, *n_sel their number */
+static int run_region_select(cbcg_ctx *ctx, uint64_t nr, const std::vector<RegionIv> &iv, const std::vector<uint64_t> &runs, uint64_t *n_sel) {
+    *n_sel = 0;
+    const uint64_t iv_bytes = iv.size() * sizeof(RegionIv);
+    TRY(ensure(ctx, ctx->reg, iv_bytes + runs.size() * 8 + 64));
+    TRY(ensure(ctx, ctx->sel_recs, (nr + 1) * sizeof(cbcg_read_rec)));
+    TRY(ensure(ctx, ctx->sel_chr, (nr + 1) * 4));
+    TRY(ensure(ctx, ctx->sel_ids, (nr + 1) * 8));
+    TRY(ensure(ctx, ctx->tile_desc, (region_num_tiles(nr) + 1) * 8));
+    CU(cudaMemcpyAsync(ctx->reg.p, iv.data(), iv_bytes, cudaMemcpyHostToDevice, ctx->st));
+    const uint64_t *d_runs = reinterpret_cast<const uint64_t *>(ctx->reg.as<uint8_t>() + iv_bytes);
+    CU(cudaMemcpyAsync(const_cast<uint64_t *>(d_runs), runs.data(), runs.size() * 8, cudaMemcpyHostToDevice, ctx->st));
+    if (launch_region_select(nr, ctx->recs.as<cbcg_read_rec>(), ctx->chr_out.as<uint32_t>(), ctx->reg.as<RegionIv>(), (uint32_t)iv.size(),
+                             d_runs, (uint32_t)(runs.size() / 2), ctx->sel_recs.as<cbcg_read_rec>(), ctx->sel_chr.as<uint32_t>(),
+                             ctx->sel_ids.as<uint64_t>(), ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)),
+                             wptr<uint64_t>(ctx, W_OFF(n_selected)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "region select launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    ctx->stats.kernel_launches++;
+    TRY(fetch_words(ctx));                                   /* synchronises: the host vectors may go */
+    TRY(device_error(ctx, "region select"));
+    *n_sel = ctx->hw->n_selected;
+    return 0;
+}
+
+extern "C" int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                                  const cbcg_region *regions, uint32_t n_regions,
+                                  uint8_t *seq_out, uint64_t seq_cap, uint64_t *seq_len,
+                                  uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
+    if (!ctx || !seq_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_region: bad argument");
+    *seq_len = 0; if (n_reads) *n_reads = 0;
+    TRY(check_regions(ctx, regions, n_regions));
+    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
+    uint64_t nr = 0, ne = 0; uint32_t max_len = 1, fixed_len = 0;
+    std::vector<RegionIv> iv;                                /* by genome ordinal */
+    std::vector<uint64_t> runs;                              /* (dense first read, container first read) per run of consecutive blocks */
+    cbcg_stats &S = ctx->stats;
+    if (legacy) {                                            /* one block: decoded whole, then filtered */
+        TRY(decode_to_records(ctx, in, in_len, 1, &nr, &ne, &max_len, &fixed_len));
+        max_len = CBCG_MAX_READ_LEN;                         /* per-read lengths are coded mod 256 (src/read_compression.c:29-33) */
+        iv = region_intervals(regions, n_regions, ctx->names);
+        runs = { 0ull, 0ull };
+    } else {
+        RegionPlan P;
+        TRY(plan_region(ctx, in, in_len, regions, n_regions, P, &ctx->names));
+        const Container &c = P.c;
+        const std::vector<uint32_t> &chr_map = c.chr_map;
+        CU(cudaSetDevice(ctx->device));
+        set_carveout_all(-1);
+        ctx->have_decoded = false;
+        ctx->have_encoded = false;                          /* ctx->payload and ctx->hblocks are about to hold another container */
+        S = cbcg_stats();
+        CU(cudaEventRecord(ctx->ev[0], ctx->st));
+        /* chromosomes: only the blocks that are decoded have to be in the loaded reference */
+        const uint64_t nb = P.sel.size();
+        TRY(ensure_hblocks(ctx, nb + 1));
+        for (uint64_t j = 0; j < nb; j++) {
+            BlockDesc b = P.blocks[P.sel[j]];
+            if (chr_map[b.chr] == 0xffffffffu) return fail(ctx, CBCG_ERR_NO_REFERENCE, "block %u: chromosome not in the loaded reference", P.sel[j]);
+            b.chr = chr_map[b.chr];
+            b.first_read = 0; b.payload_off = 0;             /* the plan kernel numbers the reduced table densely */
+            ctx->hblocks[j] = b;
+        }
+        for (RegionIv &v : P.iv) v.chr = chr_map[v.chr];
+        for (const RegionIv &v : P.iv) if (v.chr != 0xffffffffu) iv.push_back(v);
+        merge_intervals(iv);
+        ctx->layout_mode = c.layout_mode;
+        gens_from_blocks(ctx, nb);
+        ctx->max_block_reads = P.max_block_reads;           /* the encoder's FLAG target: the whole container's longest block */
+        max_len = c.max_len ? c.max_len : 1;
+        fixed_len = c.fixed_len ? c.L : 0u;
+        /* the payload of the selection: the prefix of the early generations and one run per group of adjacent blocks */
+        TRY(ensure(ctx, ctx->payload, P.payload_bytes + 64));
+        uint64_t dense = 0, at = 0;
+        for (uint64_t j = 0; j < nb;) {
+            uint64_t e = j + 1;
+            while (e < nb && P.sel[e] == P.sel[e - 1] + 1) e++;
+            const BlockDesc &a = P.blocks[P.sel[j]], &z = P.blocks[P.sel[e - 1]];
+            const uint64_t bytes = z.payload_off + z.payload_bytes - a.payload_off;
+            if (bytes) CU(cudaMemcpyAsync(ctx->payload.as<uint8_t>() + at, in + c.payload_off + a.payload_off, bytes, cudaMemcpyHostToDevice, ctx->st));
+            runs.push_back(dense); runs.push_back(a.first_read);
+            at += bytes;
+            for (uint64_t k = j; k < e; k++) dense += P.blocks[P.sel[k]].n_reads;
+            j = e;
+        }
+        S.h2d_bytes = P.payload_bytes + nb * sizeof(BlockDesc);
+        CU(cudaEventRecord(ctx->ev[1], ctx->st));
+        if (nb) TRY(run_decode_blocks(ctx, nb, c.L, 0, c.gen_mode == 1, c.fixed_len != 0, P.n_reads, P.n_edits, &nr, &ne));
+        CU(cudaEventRecord(ctx->ev[2], ctx->st));
+        S.n_blocks = nb; S.n_reads = nr; S.n_edits = ne;
+    }
+    uint64_t n_sel = 0, bytes = 0;
+    if (nr && !iv.empty()) TRY(run_region_select(ctx, nr, iv, runs, &n_sel));
+    if (n_sel) {
+        TRY(run_reconstruct(ctx, n_sel, max_len, fixed_len, ctx->sel_chr.as<uint32_t>(), 0u, ctx->sel_recs.as<cbcg_read_rec>()));
+        TRY(fetch_words(ctx));
+        TRY(device_error(ctx, "read reconstruction"));
+        cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
+        bytes = ctx->hw->total_bytes;
+    }
+    CU(cudaEventRecord(ctx->ev[3], ctx->st));
+    *seq_len = bytes; if (n_reads) *n_reads = n_sel;
+    ctx->dec_bytes = bytes; ctx->dec_n_reads = n_sel; ctx->have_decoded = true;
+    if (bytes > seq_cap || (!seq_out && bytes) || (read_ids && n_sel > ids_cap))
+        return fail(ctx, CBCG_ERR_CAPACITY, "%llu reads / %llu bytes of text selected, room for %llu / %llu", (unsigned long long)n_sel,
+                    (unsigned long long)bytes, (unsigned long long)ids_cap, (unsigned long long)seq_cap);
+    CU(cudaEventRecord(ctx->ev[4], ctx->st));
+    if (bytes) CU(cudaMemcpyAsync(seq_out, ctx->seq_out.p, bytes, cudaMemcpyDeviceToHost, ctx->st));
+    if (read_ids && n_sel) CU(cudaMemcpyAsync(read_ids, ctx->sel_ids.p, n_sel * 8, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaEventRecord(ctx->ev[5], ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    cudaEventElapsedTime(&S.ms_h2d, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&S.ms_code, ctx->ev[1], ctx->ev[2]);
+    cudaEventElapsedTime(&S.ms_reconstruct, ctx->ev[2], ctx->ev[3]);
+    cudaEventElapsedTime(&S.ms_d2h, ctx->ev[4], ctx->ev[5]);
+    cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[5]);
+    S.d2h_bytes = bytes + (read_ids ? n_sel * 8 : 0);
     return CBCG_OK;
 }
 

@@ -10,6 +10,10 @@
  *          -B MB    SAM text per batch (default 2048): memory is bounded by three batches whatever the file size
  *          -C       CIGAR recovery (SURVEY.md 8f row 4; cbcg_cigar_pack / cbcg_cigar_unpack): -c also writes <out>.cig, the side
  *                   sections of the batches (u64 length + section each); -d reads <in>.cig and writes "CIGAR<TAB>SEQ" lines
+ *          -r NAME[:START[-END]]   -d only, repeatable: write only the reads that overlap one of the regions (1-based, inclusive;
+ *                   cbcg_decode_region), each once, in file order. The region is split at the last ':', so record names that
+ *                   contain one still work. Every batch of a "CBCS" file gets the same regions; a batch that none of them
+ *                   touches (cbcg_region_plan: no blocks) makes no device call. Not with -C.
  *
  * Host C only: SAM/FASTA ingest (sam_ingest.c) and file I/O; the coding runs on the GPU through include/cbcg.h.
  * Where the reference's compress() (src/compression.c:112-170) reads a line, codes it and moves on, this driver
@@ -25,6 +29,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
+#include <sys/mman.h>
 
 #include "cbcg.h"
 #include "sam_ingest.h"
@@ -32,11 +37,13 @@
 #define MAX_DEV 16
 #define CBCS_MAGIC 0x53434243u
 
+static uint32_t rd_u32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
 static double now(void) { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t); return (double)t.tv_sec + 1e-9 * (double)t.tv_nsec; }
 
 static int usage(void) {
     fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
-                    "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n");
+                    "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
+                    "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n");
     return 2;
 }
 
@@ -66,6 +73,7 @@ typedef struct shared {
     /* run parameters */
     int mode, single, var_length, with_cigar; uint32_t block_reads;
     const cbch_fasta *fa; int fa_ready;
+    const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
     double t_gpu_ready;
 } shared;
 
@@ -121,6 +129,21 @@ static void *device_main(void *arg) {
                 }
             }
             if (J->have_compact) cbch_free_compact(&J->cb);
+        } else if (S->n_regions) {
+            uint64_t nb = 0, n_reads = 0, pb = 0, cap = 0, n = 0;
+            rc = cbcg_region_plan(J->in, J->in_len, J->legacy, S->regions, S->n_regions, &nb, &n_reads, &pb, &cap);
+            if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "region plan: %s", cbcg_strerror(rc)); }
+            else if (nb) {                                        /* a batch that no region touches costs no device call */
+                if (J->legacy) cap = 1u << 20;
+                tq = now();
+                J->out = (uint8_t *)malloc(cap ? cap : 1);
+                rc = J->out ? cbcg_decode_region(ctx, J->in, J->in_len, J->legacy, S->regions, S->n_regions, J->out, cap, &n, NULL, 0, &n_reads) : CBCG_ERR_NOMEM;
+                if (rc == CBCG_ERR_CAPACITY && n > cap) { free(J->out); J->out = (uint8_t *)malloc(n); rc = J->out ? cbcg_fetch_decoded(ctx, J->out, n, &n) : CBCG_ERR_NOMEM; }
+                if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "%s", ctx ? cbcg_last_error(ctx) : "no context"); }
+                J->out_len = n; J->n_reads = n_reads;
+                D->call_s += now() - tq;
+                cbcg_stats st; cbcg_get_stats(ctx, &st); J->device_ms = st.ms_total;
+            }
         } else {
             uint64_t n_reads = 0, cap = 0, n = 0;
             if (!J->legacy && cbcg_decoded_size(J->in, J->in_len, &n_reads, &cap) != CBCG_OK) { J->rc = CBCG_ERR_FORMAT; snprintf(J->err, sizeof J->err, "malformed container"); }
@@ -205,6 +228,28 @@ static void *ingest_main(void *arg) {
     return NULL;
 }
 
+/* NAME[:START[-END]], split at the last ':' when what follows it is START or START-END (else the whole text is the name) */
+static int parse_region(const char *a, cbcg_region *r) {
+    const char *c = strrchr(a, ':');
+    size_t name_len = strlen(a);
+    unsigned long long s = 1, t = UINT64_MAX;
+    if (c && c != a && c[1] >= '0' && c[1] <= '9') {
+        char *e;
+        const unsigned long long s1 = strtoull(c + 1, &e, 10);
+        unsigned long long t1 = UINT64_MAX;
+        int ok = !*e || *e == '-';
+        if (ok && *e == '-') { const char *q = e + 1; t1 = (*q >= '0' && *q <= '9') ? strtoull(q, &e, 10) : 0; ok = *q >= '0' && *q <= '9' && !*e; }
+        if (ok) {
+            if (s1 == 0 || t1 < s1) return -1;
+            name_len = (size_t)(c - a); s = s1; t = t1;
+        }
+    }
+    char *name = strndup(a, name_len);
+    if (!name) return -1;
+    r->name = name; r->start = s; r->end = t;
+    return 0;
+}
+
 static int parse_devices(const char *s, int *dev) {
     int n = 0;
     while (*s && n < MAX_DEV) {
@@ -222,6 +267,7 @@ int main(int argc, char **argv) {
     uint32_t block_reads = CBCG_BLOCK_AUTO;
     uint64_t batch_mb = 2048;
     const char *files[4]; int nfiles = 0;
+    cbcg_region *regions = NULL; uint32_t n_regions = 0;
     for (int i = 1; i < argc; i++) {
         const char *a = argv[i];
         if (!strcmp(a, "-c")) mode = 'c';
@@ -231,6 +277,13 @@ int main(int argc, char **argv) {
         else if (!strcmp(a, "-C")) with_cigar = 1;
         else if (!strcmp(a, "-b") && i + 1 < argc) block_reads = (uint32_t)strtoul(argv[++i], NULL, 10);
         else if (!strcmp(a, "-B") && i + 1 < argc) batch_mb = strtoull(argv[++i], NULL, 10);
+        else if (!strcmp(a, "-r") && i + 1 < argc) {
+            cbcg_region *g = (cbcg_region *)realloc(regions, (n_regions + 1) * sizeof *regions);
+            if (!g) return 1;
+            regions = g;
+            if (parse_region(argv[++i], &regions[n_regions])) { fprintf(stderr, "cbc: bad region '%s' (NAME[:START[-END]], 1 <= START <= END)\n", argv[i]); return 2; }
+            n_regions++;
+        }
         else if (!strcmp(a, "-g") && i + 1 < argc) { n_dev = parse_devices(argv[++i], dev); if (n_dev < 1) return usage(); }
         else if (a[0] == '-' && a[1]) return usage();
         else if (nfiles < 4) files[nfiles++] = a;
@@ -243,6 +296,8 @@ int main(int argc, char **argv) {
         files[0] = files[1]; files[1] = files[2]; files[2] = files[3]; nfiles = 3;
     }
     if (!mode || nfiles != 3) { fprintf(stderr, "Missing required filenames\n"); return usage(); }
+    if (n_regions && mode != 'd') { fprintf(stderr, "cbc: -r selects reads to decode: it goes with -d\n"); return usage(); }
+    if (n_regions && with_cigar) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
     if (!single && block_reads == 0) block_reads = CBCG_BLOCK_AUTO;
     if (batch_mb < 1) batch_mb = 1;
 
@@ -250,12 +305,13 @@ int main(int argc, char **argv) {
     shared S; memset(&S, 0, sizeof S);
     pthread_mutex_init(&S.mu, NULL); pthread_cond_init(&S.cv, NULL);
     S.mode = mode; S.single = single; S.var_length = var_length; S.block_reads = block_reads; S.with_cigar = with_cigar;
+    S.regions = regions; S.n_regions = n_regions;
     devthread D[MAX_DEV]; memset(D, 0, sizeof D);
 
     /* ---- the input, cut into jobs (before the device threads start: they index S.jobs) */
     cbch_mapped map; memset(&map, 0, sizeof map); map.fd = -1;
     const uint8_t **cut = NULL;
-    uint8_t *in = NULL, *cig_file = NULL; uint64_t in_len = 0;
+    const uint8_t *in = NULL; uint8_t *cig_file = NULL; uint64_t in_len = 0;
     if (mode == 'c') {
         printf("Compressing...\n");
         const uint64_t batch_bytes = batch_mb << 20;
@@ -269,12 +325,10 @@ int main(int argc, char **argv) {
         cut[S.n_jobs] = end;
     } else {
         printf("Decompressing...\n");
-        FILE *f = fopen(files[0], "rb");
-        if (!f) { fprintf(stderr, "cbc: cannot open %s\n", files[0]); return 1; }
-        fseek(f, 0, SEEK_END); long sz = ftell(f); fseek(f, 0, SEEK_SET);
-        in = (uint8_t *)malloc(sz > 0 ? (size_t)sz : 1); in_len = sz > 0 ? (uint64_t)sz : 0;
-        if (!in || fread(in, 1, (size_t)in_len, f) != (size_t)in_len) { fprintf(stderr, "cbc: cannot read %s\n", files[0]); return 1; }
-        fclose(f);
+        /* mapped, not read: the payload pages a region query does not need are never read from disk */
+        if (cbch_map(files[0], 0, &map)) { fprintf(stderr, "cbc: cannot open %s\n", files[0]); return 1; }
+        in = map.p; in_len = map.n;
+        if (n_regions && in_len) madvise((void *)map.p, (size_t)in_len, MADV_RANDOM);   /* no read-ahead past the blocks a query needs */
         uint32_t h[4] = { 0, 0, 0, 0 };
         if (in_len >= 16) memcpy(h, in, 16);
         S.n_jobs = (h[0] == CBCS_MAGIC && h[2] > 0 && 16 + 16ull * h[2] <= in_len) ? h[2] : 1;
@@ -283,7 +337,7 @@ int main(int argc, char **argv) {
     for (uint64_t k = 0; k < S.n_jobs; k++) { S.jobs[k] = (job *)calloc(1, sizeof(job)); S.jobs[k]->index = k; }
     if (mode == 'd') {
         uint64_t nr, cap;
-        if (S.n_jobs == 1 && !(in_len >= 16 && ((uint32_t *)in)[0] == CBCS_MAGIC)) {
+        if (S.n_jobs == 1 && !(in_len >= 16 && rd_u32(in) == CBCS_MAGIC)) {
             S.jobs[0]->in = in; S.jobs[0]->in_len = in_len;
             S.jobs[0]->legacy = cbcg_decoded_size(in, in_len, &nr, &cap) != CBCG_OK;            /* no "CBCB" header: a reference stream */
         } else for (uint64_t k = 0; k < S.n_jobs; k++) {
@@ -402,8 +456,10 @@ int main(int argc, char **argv) {
     if (getenv("CBC_TRACE")) for (int d = 0; d < n_dev; d++)
         fprintf(stderr, "[cbc] device %d: context %.3f s, reference upload %.3f s, coding calls %.3f s; writer done at %.3f s\n", dev[d], D[d].create_s, D[d].setref_s, D[d].call_s, t2 - t0);
     for (uint64_t k = 0; k < S.n_jobs; k++) { free(S.jobs[k]->out); free(S.jobs[k]->cig); free(S.jobs[k]); }
-    free(S.jobs); free(cut); free(in); free(cig_file); free(shard_off); free(shard_len);
-    if (mode == 'c') cbch_unmap(&map);
+    free(S.jobs); free(cut); free(cig_file); free(shard_off); free(shard_len);
+    for (uint32_t k = 0; k < n_regions; k++) free((void *)regions[k].name);
+    free(regions);
+    cbch_unmap(&map);
     cbch_free_fasta(&fa);
     printf("Total time elapsed: %f seconds.\n", now() - t0);
     return status;

@@ -145,3 +145,11 @@ int launch_copy16(void *dst, const void *src, uint64_t bytes, cudaStream_t st);
 int launch_d2h_bytes(void *dst_host, const void *src_dev, uint64_t bytes, cudaStream_t st);   /* dst: mapped pinned host memory, any alignment */
 int launch_copy_words(void *dst, const void *src, uint32_t n_words, cudaStream_t st);          /* <= 32 64-bit words */
 uint64_t coder_payload_bound(uint64_t n_reads, uint64_t n_edits, uint64_t n_blocks, int legacy);
+/* k5_region.cu: region select and compaction. iv: the query's intervals (genome ordinals), sorted by (chr, start), overlaps
+   merged; runs: n_runs pairs (dense ordinal of a run's first read, its ordinal in the container), ascending. *total
+   receives the number of reads kept. */
+struct RegionIv { uint32_t chr, pad; uint64_t start, end; };   /* 1-based, both ends inclusive */
+uint64_t region_num_tiles(uint64_t n_reads);
+int launch_region_select(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr, const RegionIv *iv, uint32_t n_iv,
+                         const uint64_t *runs, uint32_t n_runs, cbcg_read_rec *out_recs, uint32_t *out_chr, uint64_t *out_ids,
+                         uint64_t *tile_desc, uint32_t *ticket, uint64_t *total, unsigned long long *err, cudaStream_t st);

@@ -195,6 +195,42 @@ int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64
 int cbcg_cigar_unpack(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const uint8_t *section, uint64_t section_len,
                       uint8_t *cigar_out, uint64_t cigar_cap, uint64_t *cigar_len, uint64_t *n_reads);
 
+/* ---- region decode (DESIGN.md, "Region decode"): the reads of a blocked container that overlap genomic intervals,
+ * without decoding the whole container. The blocks of generation g start from the snapshot that merges every block of the
+ * generations before g, so the call decodes every block of every generation before the latest generation g* that a region
+ * touches, then only the touched blocks of g* (gen_mode 0: only the touched blocks). A legacy stream is one block: it is
+ * decoded whole and then filtered.
+ *   overlap: a read overlaps [start, end] on its chromosome if pos <= end and pos + span - 1 >= start, span = len - n_ins +
+ *     n_dels from the decoded record (deletions and insertions counted per base; the reference codes soft clips as
+ *     insertions, so clipped bases are not part of the span): the alignment end samtools computes for M/I/D/S CIGARs.
+ *   several regions give their union: a read is returned once however many regions it overlaps; they need not be sorted.
+ *     A name that is not in the container (legacy: not in the loaded reference) matches nothing; that is not an error.
+ *   errors: start == 0, start > end, a NULL name or n_regions == 0 -> CBCG_ERR_ARG; a malformed header or index ->
+ *     CBCG_ERR_FORMAT; a block that has to be decoded names a chromosome missing from the loaded reference ->
+ *     CBCG_ERR_NO_REFERENCE (blocks that are not decoded may).
+ *   capacity: as cbcg_decode. seq_cap or ids_cap too small -> CBCG_ERR_CAPACITY with *seq_len / *n_reads set to the sizes
+ *     needed; cbcg_fetch_decoded then returns the text.
+ *   statistics: cbcg_get_stats's n_blocks and n_reads are what the block decoder decoded (more than is returned);
+ *     the returned count is *n_reads.
+ *   state: a decode; it invalidates "the last encode" as cbcg_decode of a foreign container does. */
+/* A genomic interval: 1-based, both ends inclusive; end = UINT64_MAX means "to the end of the record".
+ * name: a reference record name as stored in the container. */
+typedef struct cbcg_region { const char *name; uint64_t start, end; } cbcg_region;
+
+/* What cbcg_decode_region would do with this container and these regions, computed on the host from the header and the
+ * block index alone (no context, no device, no payload bytes read): blocks and reads it decodes, payload bytes it
+ * reads, and an upper bound on the text it returns. A legacy stream does not store its read count: *n_blocks = 1,
+ * *payload_bytes = in_len, *n_reads = *max_seq_bytes = UINT64_MAX (unknown). */
+int cbcg_region_plan(const uint8_t *in, uint64_t in_len, int legacy, const cbcg_region *regions, uint32_t n_regions,
+                     uint64_t *n_blocks, uint64_t *n_reads, uint64_t *payload_bytes, uint64_t *max_seq_bytes);
+
+/* The reads that overlap at least one region, each once, in container order: SEQ + '\n' per read, like cbcg_decode,
+ * and (read_ids != NULL) each read's ordinal in the container. */
+int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                       const cbcg_region *regions, uint32_t n_regions,
+                       uint8_t *seq_out, uint64_t seq_cap, uint64_t *seq_len,
+                       uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
+
 /* ---- device-resident variants (inputs already in HBM when the timed region starts): upload once,
  * run many times. Results stay on the device until fetched. Used by bench.py for `value`. */
 int cbcg_batch_upload(cbcg_ctx *ctx, const cbcg_batch *batch);                 /* replaces the resident batch */
