@@ -308,6 +308,10 @@ k1_extract_kernel(DevBatch b, DevGenome g, cbcg_read_rec *__restrict__ recs, uin
         if (!bad && !(my_cnt >> 24)) {
             EditSink sink = { nullptr, 0u, 0u, 0u, 0u, 0u, 0, S.ecache[tid] };
             walk_read(s_seq + S.soff[tid], my_len, my_cig, my_clen, my_md, my_mlen, sink);
+            /* the bases the decoder takes from the reference (len - n_ins aligned, plus the deletions) must lie inside the
+               chromosome, as K3 requires: a read whose span runs past the end could not be rebuilt */
+            if (!sink.err && (sink.n_ins > my_len ||
+                              (uint64_t)(my_pos - 1u) + (my_len - sink.n_ins) + sink.n_dels > g.chr_len[my_chr])) sink.err = 1;
             if (sink.err) bad = true;
             else { my_cnt = sink.n_snps | (sink.n_dels << 8) | (sink.n_ins << 16); my_total = sink.n_snps + sink.n_dels + sink.n_ins; }
         }

@@ -1065,7 +1065,8 @@ S_POS:
     x = 0u;
     if (MODE != MODE_DEC) {
         if (pos == 0u || len == 0u || len > CBCG_MAX_READ_LEN) { C.err = CBCG_ERR_INPUT; goto M_DONE; }
-        if (pos < prev_pos || pos - prev_pos + 1u > CBCG_MAX_POS_X) { C.err = CBCG_ERR_INPUT; goto M_DONE; }
+        /* the reference's POS alphabet bounds the step of its own stream only; a blocked container codes any 32-bit step */
+        if (pos < prev_pos || (LEGACY && pos - prev_pos + 1u > CBCG_MAX_POS_X)) { C.err = CBCG_ERR_INPUT; goto M_DONE; }
         x = pos - prev_pos + 1u;
     }
     CODE_DIRECT(C.sym_pos_main(x, slot), CBCG_S_POS_X, 0u, x, P_POS);
@@ -1377,7 +1378,7 @@ k2_block_kernel(CoderParams P) {
             uint32_t x = 0, pos = 0, slot = 1u;
             if (MODE == MODE_ENC) {
                 pos = P.recs[r0 + i].pos;
-                if (pos == 0u || pos < prev_pos || pos - prev_pos + 1u > CBCG_MAX_POS_X) K2B_FAIL(CBCG_ERR_INPUT);
+                if (pos == 0u || pos < prev_pos) K2B_FAIL(CBCG_ERR_INPUT);
                 x = pos - prev_pos + 1u;
             } else if (!k2b_room(S, i, seen_d)) { bailed = true; break; }
             const uint32_t y = C.sym_pos_main(x, slot);
@@ -1683,7 +1684,7 @@ k2_model_kernel(CoderParams P, uint32_t role_mask) {
         for (; i < n_reads; i++) {
             const uint4 nx = (i + 1u < n_reads) ? recs[i + 1u] : v;        /* next read's record: off the chain */
             const uint32_t pos = v.x;
-            if (pos == 0u || pos < prev_pos || pos - prev_pos + 1u > CBCG_MAX_POS_X) K2M_FAIL(CBCG_ERR_INPUT);
+            if (pos == 0u || pos < prev_pos) K2M_FAIL(CBCG_ERR_INPUT);
             const uint32_t x = pos - prev_pos + 1u;
             uint32_t s = 1u;
             C.tri_at = slots + slot + lead;

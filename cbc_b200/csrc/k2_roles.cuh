@@ -311,7 +311,7 @@ K2_HD int k2_role_pos(const CoderParams &P, uint32_t block, uint64_t *err_item) 
         uint32_t x = 0, pos = 0, slot = 0, lo = 0, cnt = 0;
         if (MODE == MODE_ENC) {
             pos = P.recs[r0 + i].pos;
-            if (pos == 0u || pos < prev_pos || pos - prev_pos + 1u > CBCG_MAX_POS_X) { ac.err = CBCG_ERR_INPUT; break; }
+            if (pos == 0u || pos < prev_pos) { ac.err = CBCG_ERR_INPUT; break; }
             x = pos - prev_pos + 1u;
             for (slot = 1; slot < card; slot++) { if (valv[slot] == x) break; }
             if (slot < card) { lo = k2_cum_below(cntv, slot); cnt = cntv[slot]; }

@@ -31,8 +31,13 @@ typedef enum cbcg_status {
     CBCG_ERR_NOMEM       = -4,
     CBCG_ERR_CAPACITY    = -5,   /* caller's output buffer too small */
     CBCG_ERR_INPUT       = -6,   /* a read is outside what the reference can code (SURVEY.md 8c):
-                                    POS 0, length 0 or > 252, CIGAR '*'/'N'/junk, > 255 edits of a kind,
-                                    unsorted positions, zero-probability symbol (src/stream_model.c:71) */
+                                    POS 0, length 0 or > 252, reference span (length - insertions
+                                    + deletions) past the chromosome's end, CIGAR '*'/'N'/junk,
+                                    > 255 edits of a kind, unsorted positions, zero-probability symbol
+                                    (src/stream_model.c:71: e.g. L SNPs in a read at header length L), and,
+                                    in the single-block stream only, a POS step pos - prev_pos + 1 above
+                                    5 000 000 (CBCG_MAX_POS_X; the first read of a chromosome steps from 0).
+                                    Blocked containers code any POS step. */
     CBCG_ERR_NO_REFERENCE = -7,  /* cbcg_set_reference not called / chromosome ordinal out of range */
     CBCG_ERR_FORMAT      = -8,   /* container header / index malformed */
     CBCG_ERR_CORRUPT     = -9,   /* bitstream decodes to an impossible symbol */

@@ -607,10 +607,11 @@ static int md_walk(mdwalk *w, snp_t *snps, uint32_t *n_snps, uint32_t insertion_
     return 0;
 }
 
-/* One read. Returns 0, or <0 when the read is outside what the reference can code. */
+/* One read. Returns 0, or <0 when the read is outside what the reference can code (-2: its edits do not fit in
+ * edits_cap entries). */
 static int extract_read(const uint8_t *read, uint32_t len, const uint8_t *cigar, uint32_t cigar_len,
                         const uint8_t *md, uint32_t md_len, const uint8_t *ref, uint64_t ref_len,
-                        uint32_t pos, cbcg_read_rec *rec, uint16_t *edits, uint32_t *n_edits) {
+                        uint32_t pos, cbcg_read_rec *rec, uint16_t *edits, uint64_t edits_cap, uint32_t *n_edits) {
     *n_edits = 0;
     rec->match = 0; rec->n_snps = rec->n_dels = rec->n_ins = 0;
     if (pos == 0 || len == 0 || len > CBCG_MAX_READ_LEN) return -10;
@@ -678,6 +679,10 @@ static int extract_read(const uint8_t *read, uint32_t len, const uint8_t *cigar,
     if (last_snp) md_walk(&w, snps, &n_snps, len + 1, read, len);       /* :551-552 */
 
     if (n_snps > 255 || n_dels > 255 || n_ins > 255) return -14;
+    /* the reference span the decoder rebuilds from (rebuild_read below) must lie inside the chromosome; K1 refuses the
+       same reads. Insertions and clips may carry SEQ past the chromosome's end. */
+    if (n_ins > len || (uint64_t)pos - 1 + (len - n_ins) + n_dels > ref_len) return -15;
+    if ((uint64_t)n_dels + n_snps + n_ins > edits_cap) return -2;
     rec->n_snps = (uint8_t)n_snps; rec->n_dels = (uint8_t)n_dels; rec->n_ins = (uint8_t)n_ins;
     uint32_t e = 0;
     for (uint32_t k = 0; k < n_dels; k++) { if (dels[k] > 255) return -14; edits[e++] = CBCG_EDIT(dels[k], 0, 0); }
@@ -694,14 +699,13 @@ int64_t cbco_extract(const cbco_batch *b, const cbco_genome *g, cbcg_read_rec *r
         uint32_t chr = b->chr[r];
         if (chr >= g->n_chr) return -1;
         uint32_t len = b->seq_len[r];
-        if (total + 3ull * len + 8 > edits_cap) return -2;
         cbcg_read_rec *rec = &recs[r];
         rec->pos = b->pos[r]; rec->flag = b->flag[r]; rec->len = (uint16_t)len; rec->edit_off = (uint32_t)total;
         uint32_t ne = 0;
         int rc = extract_read(b->seq + b->seq_off[r], len,
                               b->cigar + b->cigar_off[r], (uint32_t)(b->cigar_off[r + 1] - b->cigar_off[r]),
                               b->md + b->md_off[r], (uint32_t)(b->md_off[r + 1] - b->md_off[r]),
-                              g->bases[chr], g->len[chr], b->pos[r], rec, edits + total, &ne);
+                              g->bases[chr], g->len[chr], b->pos[r], rec, edits + total, edits_cap - total, &ne);
         if (rc) return rc;
         total += ne;
     }
@@ -912,6 +916,11 @@ static int code_range(rstate *s, const cbco_batch *b, const cbco_genome *g, cons
             if (legacy) s->prev_pos = 0;
             snp_reset(&s->snp, g->len[chr] + 2048);
         }
+        /* single stream: the reference indexes alphaExist / alphaMap, CBCG_MAX_POS_X entries each (sam_block.h:54), by the
+           POS step, so a step above CBCG_MAX_POS_X is refused, as the GPU encoder refuses it. Whether the reference itself
+           survives a step of exactly CBCG_MAX_POS_X was never run against its binary. A blocked container codes any
+           32-bit step through the escape and has no such limit. */
+        if (legacy && recs[r].pos - s->prev_pos + 1u > CBCG_MAX_POS_X) return -16;
         put_read(s, &recs[r], edits + recs[r].edit_off);
         if (s->c.err) return s->c.err;
     }
@@ -920,7 +929,7 @@ static int code_range(rstate *s, const cbco_batch *b, const cbco_genome *g, cons
 
 int cbco_encode_legacy(const cbco_batch *b, const cbco_genome *g, uint32_t L, cbco_buf *out, cbco_buf *trace) {
     uint64_t cap = 16;
-    for (uint64_t r = 0; r < b->n_reads; r++) cap += 3ull * b->seq_len[r] + 8;
+    for (uint64_t r = 0; r < b->n_reads; r++) cap += CBCO_EDITS_PER_READ(b->seq_len[r]);
     cbcg_read_rec *recs = (cbcg_read_rec *)malloc(sizeof(cbcg_read_rec) * (b->n_reads + 1));
     uint16_t *edits = (uint16_t *)malloc(2 * cap);
     int64_t ne = cbco_extract(b, g, recs, edits, cap);
@@ -1124,7 +1133,7 @@ static int encode_cut(const cbco_batch *b, const cbco_genome *g, uint32_t L, uin
                       uint32_t gen_mode, cbco_buf *out) {
     if (block_reads == 0) return -30;
     uint64_t cap = 16;
-    for (uint64_t r = 0; r < b->n_reads; r++) cap += 3ull * b->seq_len[r] + 8;
+    for (uint64_t r = 0; r < b->n_reads; r++) cap += CBCO_EDITS_PER_READ(b->seq_len[r]);
     cbcg_read_rec *recs = (cbcg_read_rec *)malloc(sizeof(cbcg_read_rec) * (b->n_reads + 1));
     uint16_t *edits = (uint16_t *)malloc(2 * cap);
     int64_t ne = cbco_extract(b, g, recs, edits, cap);

@@ -49,8 +49,12 @@ typedef struct cbco_buf { uint8_t *data; uint64_t size, cap; } cbco_buf;
 void cbco_buf_free(cbco_buf *b);
 
 /* Edit extraction (compress_edits + add_snps_to_array, src/read_compression.c:265-701).
- * recs[n_reads]; edits needs room for sum(n_dels+n_snps+n_ins) entries (<= 3*len per read).
- * Returns number of edit entries, or <0 on an input outside the reference's contract. */
+ * recs[n_reads]; edits needs room for sum(n_dels+n_snps+n_ins) entries. A read carries up to 255
+ * deletions whatever its length, and, when its CIGAR and MD agree with its SEQ, at most len SNPs
+ * and insertions together: CBCO_EDITS_PER_READ(len) entries (8 spare) per read are always enough.
+ * Returns number of edit entries, -2 when they do not fit in edits_cap, or <0 on an input outside
+ * the reference's contract. Nothing is written past edits_cap. */
+#define CBCO_EDITS_PER_READ(len) ((uint64_t)(len) + 255u + 8u)
 int64_t cbco_extract(const cbco_batch *b, const cbco_genome *g, cbcg_read_rec *recs,
                      uint16_t *edits, uint64_t edits_cap);
 

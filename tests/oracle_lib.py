@@ -70,7 +70,7 @@ def extract(batch: Batch, genome: Genome):
     g = _G(genome)
     cb = batch.c_struct()
     recs = np.zeros(batch.n_reads, REC_DTYPE)
-    cap = int(batch.seq_len.astype(np.int64).sum()) * 3 + 8 * batch.n_reads + 64
+    cap = int(batch.seq_len.astype(np.int64).sum()) + (255 + 8) * batch.n_reads + 64    # CBCO_EDITS_PER_READ
     edits = np.zeros(cap, np.uint16)
     n = lib().cbco_extract(C.byref(cb), C.byref(g.s), recs.ctypes.data_as(C.c_void_p),
                            edits.ctypes.data_as(C.c_void_p), C.c_uint64(cap))

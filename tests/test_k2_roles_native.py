@@ -43,6 +43,9 @@ CASES = [
     "21 20000 300000 100 100 0.01 0 0 0 20000 1 3000",
     "22 60000 400000 100 100 0.01 0 0 1 4294967295 1 1500 1",   # the blocks of a generation adapt different values: the merge keeps 256 (F2)
     "23 200000 1000000 100 100 0.01 0 0 1 4294967295 1 400 1",
+    # 12 reads over 60 Mb in one block: POS steps of several Mb, above the single stream's 5 M limit
+    "24 12 60000000 100 100 0.01 0 0 0 12",
+    "25 12 60000000 100 100 0.01 0 0 1",
 ]
 
 
