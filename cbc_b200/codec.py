@@ -42,7 +42,7 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_reconstruct", "cbcg_batch_upload", "cbcg_encode_resident", "cbcg_decode_resident",
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
            "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
-           "cbcg_region_plan", "cbcg_decode_region"]
+           "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam"]
 
 
 UINT64_MAX = (1 << 64) - 1
@@ -77,6 +77,22 @@ def region_plan(data: bytes, regions, legacy: bool = False) -> dict:
     if rc:
         raise CbcgError(rc, lib.cbcg_strerror(rc).decode())
     return dict(zip(("n_blocks", "n_reads", "payload_bytes", "max_seq_bytes"), (v.value for v in out)))
+
+
+def sam_header(data: bytes) -> bytes:
+    """@HD and one @SQ line per chromosome of a blocked container's table, from its header alone (no device). The
+    container does not store record lengths, so the @SQ lines carry no LN (``Codec.decompress_sam`` adds it from the
+    loaded reference)."""
+    lib = load_library()
+    src = np.frombuffer(data, np.uint8)
+    n = C.c_uint64(0)
+    rc = lib.cbcg_sam_header(src.ctypes.data, src.nbytes, None, 0, C.byref(n))
+    out = np.empty(max(n.value, 1), np.uint8)
+    if rc == -5:
+        rc = lib.cbcg_sam_header(src.ctypes.data, src.nbytes, out.ctypes.data, out.nbytes, C.byref(n))
+    if rc:
+        raise CbcgError(rc, lib.cbcg_strerror(rc).decode())
+    return out[:n.value].tobytes()
 
 
 class EncodeOpts(C.Structure):
@@ -145,6 +161,8 @@ def load_library():
         lib.cbcg_cigar_unpack.argtypes = [vp, vp, u64, C.c_int, vp, u64, vp, u64, P(u64), P(u64)]
         lib.cbcg_region_plan.argtypes = [vp, u64, C.c_int, P(Region), u32, P(u64), P(u64), P(u64), P(u64)]
         lib.cbcg_decode_region.argtypes = [vp, vp, u64, C.c_int, P(Region), u32, vp, u64, P(u64), vp, u64, P(u64)]
+        lib.cbcg_sam_header.argtypes = [vp, u64, vp, u64, P(u64)]
+        lib.cbcg_decode_sam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -355,6 +373,37 @@ class Codec:
             n, nr = C.c_uint64(0), C.c_uint64(0)
             rc = self.lib.cbcg_decode_region(self.h, src.ctypes.data, src.nbytes, int(legacy), arr, n_regions,
                                              out.ctypes.data, out.nbytes, C.byref(n), ids.ctypes.data, ids.size, C.byref(nr))
+            if rc == -5 and (n.value > out.nbytes or nr.value > ids.size):
+                size, n_ids = max(size, n.value), max(n_ids, nr.value)
+                continue
+            self._check(rc)
+            return out[:n.value].tobytes(), ids[:nr.value].copy()
+
+    def decompress_sam(self, data: bytes, cigar_section: Optional[bytes] = None, regions=None, header: bool = True,
+                       legacy: bool = False) -> Tuple[bytes, np.ndarray]:
+        """SAM text of a container (include/cbcg.h, cbcg_decode_sam): the header (header=True), then one alignment record per
+        read in container order, or per read that overlaps one of the regions (as ``decompress_region``); and each line's read
+        ordinal in the container as uint64. cigar_section: the CIGAR side section (``cigar_pack``); None: implied CIGARs."""
+        src = np.frombuffer(data, np.uint8)
+        sec = np.frombuffer(cigar_section, np.uint8) if cigar_section is not None else None
+        if regions is not None:
+            arr, n_regions = _region_array(regions)                          # an empty list is CBCG_ERR_ARG
+        else:
+            arr, n_regions = None, 0
+        n_ids = 1 << 16
+        size = max(len(data) * 8, 1 << 20)
+        if not legacy:
+            n_reads, cap = C.c_uint64(0), C.c_uint64(0)
+            if self.lib.cbcg_decoded_size(src.ctypes.data, src.nbytes, C.byref(n_reads), C.byref(cap)) == 0:
+                size, n_ids = max(size, 2 * cap.value + 1024), max(n_reads.value, 1)
+        while True:
+            out = np.empty(size, np.uint8)
+            ids = np.empty(n_ids, np.uint64)
+            n, nr = C.c_uint64(0), C.c_uint64(0)
+            rc = self.lib.cbcg_decode_sam(self.h, src.ctypes.data, src.nbytes, int(legacy),
+                                          sec.ctypes.data if sec is not None else None, sec.nbytes if sec is not None else 0,
+                                          arr, n_regions, 1 if header else 0, out.ctypes.data, out.nbytes, C.byref(n),
+                                          ids.ctypes.data, ids.size, C.byref(nr))
             if rc == -5 and (n.value > out.nbytes or nr.value > ids.size):
                 size, n_ids = max(size, n.value), max(n_ids, nr.value)
                 continue

@@ -81,6 +81,7 @@ struct cbcg_ctx {
     DevBuf cig_cls, cig_exc, cig_out;          /* CIGAR recovery (k4_cigar.cu): classes, verbatim texts, emitted text */
     DevBuf tri;                                /* two-kernel encode: the symbols' intervals between the model and the interval kernel */
     DevBuf reg, sel_recs, sel_chr, sel_ids;    /* region decode (k5_region.cu): intervals + ordinal runs, and the kept reads */
+    DevBuf sam_aux, sam_out;                   /* SAM output (k6_sam.cu): name lengths, CIGAR classes and texts; the text */
     DevBuf snap_a, snap_b, fin;                /* generation snapshots and per-block final states (gen_mode 1) */
     std::vector<std::pair<uint32_t, uint32_t>> gens;   /* (first block, block count) per generation of the last cut */
     uint32_t layout = 1;                       /* the call in progress: 1 = one stream per block, 4 = four substreams, 0 = four in the narrow early generations */
@@ -209,7 +210,7 @@ extern "C" void cbcg_destroy(cbcg_ctx *ctx) {
     if (ctx->hblocks) cudaFreeHost(ctx->hblocks);
     if (ctx->h_tile) cudaFreeHost(ctx->h_tile);
     for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec,
-                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids }) free_buf(*d);
+                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out }) free_buf(*d);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->mark) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->kev) if (e) cudaEventDestroy(e);
@@ -1841,6 +1842,17 @@ static std::vector<RegionIv> region_intervals(const cbcg_region *regions, uint32
     return iv;
 }
 
+/* the chromosome table of a parsed container */
+static std::vector<std::string> container_names(const uint8_t *in, const Container &c) {
+    std::vector<std::string> names(c.n_chr);
+    for (uint64_t o = 40, k = 0; k < c.n_chr; k++) {                 /* parse_container has checked the name table */
+        const uint32_t nl = rd32(in + o); o += 4;
+        names[k].assign(reinterpret_cast<const char *>(in + o), nl);
+        o += nl + ((4 - (nl & 3)) & 3);
+    }
+    return names;
+}
+
 struct RegionPlan {
     Container c;
     std::vector<BlockDesc> blocks;             /* the whole index (container chromosome ordinals); first_read / payload_off within the container */
@@ -1858,13 +1870,7 @@ static int plan_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, const 
     TRY(check_regions(ctx, regions, n_regions));
     Container &c = P.c;
     if (parse_container(in, in_len, genome, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
-    std::vector<std::string> names(c.n_chr);
-    for (uint64_t o = 40, k = 0; k < c.n_chr; k++) {           /* parse_container has checked the name table */
-        const uint32_t nl = rd32(in + o); o += 4;
-        names[k].assign(reinterpret_cast<const char *>(in + o), nl);
-        o += nl + ((4 - (nl & 3)) & 3);
-    }
-    P.iv = region_intervals(regions, n_regions, names);
+    P.iv = region_intervals(regions, n_regions, container_names(in, c));
     P.blocks.resize(c.n_blocks);
     IndexState st = index_state(c.block_reads);
     uint64_t o = c.index_off, first = 0, pay = 0;
@@ -1953,12 +1959,10 @@ static int run_region_select(cbcg_ctx *ctx, uint64_t nr, const std::vector<Regio
     return 0;
 }
 
-extern "C" int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
-                                  const cbcg_region *regions, uint32_t n_regions,
-                                  uint8_t *seq_out, uint64_t seq_cap, uint64_t *seq_len,
-                                  uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
-    if (!ctx || !seq_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_region: bad argument");
-    *seq_len = 0; if (n_reads) *n_reads = 0;
+/* The region's reads of a container (or legacy stream) -> ctx->sel_recs / sel_chr / sel_ids (*n_sel of them), decoded as
+ * cbcg_decode_region describes; *nr and *ne: the reads and edits the block decoder decoded. Events ev[0..2] are recorded. */
+static int region_records(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const cbcg_region *regions, uint32_t n_regions,
+                          uint64_t *nr_out, uint64_t *ne_out, uint64_t *n_sel_out, uint32_t *max_len_out, uint32_t *fixed_len_out) {
     TRY(check_regions(ctx, regions, n_regions));
     if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
     uint64_t nr = 0, ne = 0; uint32_t max_len = 1, fixed_len = 0;
@@ -2019,8 +2023,21 @@ extern "C" int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_
         CU(cudaEventRecord(ctx->ev[2], ctx->st));
         S.n_blocks = nb; S.n_reads = nr; S.n_edits = ne;
     }
-    uint64_t n_sel = 0, bytes = 0;
+    uint64_t n_sel = 0;
     if (nr && !iv.empty()) TRY(run_region_select(ctx, nr, iv, runs, &n_sel));
+    *nr_out = nr; *ne_out = ne; *n_sel_out = n_sel; *max_len_out = max_len; *fixed_len_out = fixed_len;
+    return 0;
+}
+
+extern "C" int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                                  const cbcg_region *regions, uint32_t n_regions,
+                                  uint8_t *seq_out, uint64_t seq_cap, uint64_t *seq_len,
+                                  uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
+    if (!ctx || !seq_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_region: bad argument");
+    *seq_len = 0; if (n_reads) *n_reads = 0;
+    uint64_t nr = 0, ne = 0, n_sel = 0, bytes = 0; uint32_t max_len = 1, fixed_len = 0;
+    cbcg_stats &S = ctx->stats;
+    TRY(region_records(ctx, in, in_len, legacy, regions, n_regions, &nr, &ne, &n_sel, &max_len, &fixed_len));
     if (n_sel) {
         TRY(run_reconstruct(ctx, n_sel, max_len, fixed_len, ctx->sel_chr.as<uint32_t>(), 0u, ctx->sel_recs.as<cbcg_read_rec>()));
         TRY(fetch_words(ctx));
@@ -2093,6 +2110,36 @@ extern "C" int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *
     memcpy(out, sec.data(), sec.size());
     return CBCG_OK;
 }
+/* A CIGAR side section (layout above cbcg_cigar_bound) for a container of n reads -> a class per read and the class-4 texts. */
+static int parse_cigar_section(cbcg_ctx *ctx, const uint8_t *section, uint64_t section_len, uint64_t n, std::vector<uint8_t> &cls,
+                               std::vector<uint64_t> &exc_read, std::vector<uint64_t> &exc_off, std::vector<uint8_t> &exc_text) {
+    uint32_t magic = 0, version = 0; uint64_t sn = 0, entries = 0;
+    if (section_len < 24) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section too short");
+    memcpy(&magic, section, 4); memcpy(&version, section + 4, 4); memcpy(&sn, section + 8, 8); memcpy(&entries, section + 16, 8);
+    if (magic != CBCC_MAGIC || version != 1u) return fail(ctx, CBCG_ERR_FORMAT, "not a CIGAR section");
+    if (sn != n) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section of %llu reads beside a container of %llu", (unsigned long long)sn, (unsigned long long)n);
+    cls.assign(n, 0); exc_read.clear(); exc_off.assign(1, 0); exc_text.clear();
+    uint64_t o = 24, prev = 0;
+    for (uint64_t k = 0; k < entries; k++) {
+        uint64_t d = 0, l = 0;
+        if (!get_varint(section, section_len, o, d) || o >= section_len) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section truncated");
+        const uint64_t r = prev + d;
+        if (r >= n || (k && d == 0)) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section lists read %llu", (unsigned long long)r);
+        prev = r;
+        const uint8_t c = section[o++];
+        if (c == 0 || c > 4) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section: class %u", (unsigned)c);
+        cls[r] = c;
+        if (c == 4) {
+            if (!get_varint(section, section_len, o, l) || l > section_len - o) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section truncated");
+            exc_read.push_back(r);
+            exc_text.insert(exc_text.end(), section + o, section + o + l);
+            exc_off.push_back(exc_text.size());
+            o += l;
+        }
+    }
+    return 0;
+}
+
 /* container (or legacy stream) + its section -> the CIGAR of every read, '\n'-terminated, in read order. section == NULL:
  * every read gets the CIGAR its indels imply (soft clips read as insertions). */
 extern "C" int cbcg_cigar_unpack(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const uint8_t *section, uint64_t section_len,
@@ -2107,31 +2154,7 @@ extern "C" int cbcg_cigar_unpack(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_l
     std::vector<uint64_t> exc_read, exc_off(1, 0);
     std::vector<uint8_t> exc_text;
     uint64_t text_bound = 0;
-    if (section) {
-        uint32_t magic = 0, version = 0; uint64_t sn = 0, entries = 0;
-        if (section_len < 24) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section too short");
-        memcpy(&magic, section, 4); memcpy(&version, section + 4, 4); memcpy(&sn, section + 8, 8); memcpy(&entries, section + 16, 8);
-        if (magic != CBCC_MAGIC || version != 1u) return fail(ctx, CBCG_ERR_FORMAT, "not a CIGAR section");
-        if (sn != nr) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section of %llu reads beside a container of %llu", (unsigned long long)sn, (unsigned long long)nr);
-        uint64_t o = 24, prev = 0;
-        for (uint64_t k = 0; k < entries; k++) {
-            uint64_t d = 0, l = 0;
-            if (!get_varint(section, section_len, o, d) || o >= section_len) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section truncated");
-            const uint64_t r = prev + d;
-            if (r >= nr || (k && d == 0)) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section lists read %llu", (unsigned long long)r);
-            prev = r;
-            const uint8_t c = section[o++];
-            if (c == 0 || c > 4) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section: class %u", (unsigned)c);
-            cls[r] = c;
-            if (c == 4) {
-                if (!get_varint(section, section_len, o, l) || l > section_len - o) return fail(ctx, CBCG_ERR_FORMAT, "CIGAR section truncated");
-                exc_read.push_back(r);
-                exc_text.insert(exc_text.end(), section + o, section + o + l);
-                exc_off.push_back(exc_text.size());
-                o += l;
-            }
-        }
-    }
+    if (section) TRY(parse_cigar_section(ctx, section, section_len, nr, cls, exc_read, exc_off, exc_text));
     text_bound = exc_text.size() + nr * 4ull + ne * 12ull + nr * 8ull + 64;   /* per read: '\n' + <= 2 operations per indel event + 2 M runs, <= 6 bytes each */
     const uint64_t n_exc = exc_read.size();
     const uint64_t exc_bytes = (n_exc + 1) * 16 + exc_text.size() + 64;
@@ -2158,6 +2181,145 @@ extern "C" int cbcg_cigar_unpack(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_l
     if (bytes > cigar_cap || !cigar_out) return fail(ctx, CBCG_ERR_CAPACITY, "CIGAR text is %llu bytes, room for %llu", (unsigned long long)bytes, (unsigned long long)cigar_cap);
     CU(cudaMemcpyAsync(cigar_out, ctx->cig_out.p, bytes, cudaMemcpyDeviceToHost, ctx->st));
     CU(cudaStreamSynchronize(ctx->st));
+    return CBCG_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------ SAM output
+ * cbcg_sam_header / cbcg_decode_sam (DESIGN.md, "SAM output"; the line and the MD / NM rule: k6_sam.cu). The records come
+ * from the whole-container decode or from the region decode, K3 rebuilds SEQ, K6 formats the lines next to it. The CIGAR
+ * side section is parsed here into a class byte per container read and the class-4 texts; K6 looks a read up by its
+ * container ordinal, which is what lets a region decode recover the CIGARs. */
+
+/* @HD, then @SQ per name; lengths: LN per name (UINT64_MAX: unknown, not written) */
+static std::string sam_header_text(const std::vector<std::string> &names, const std::vector<uint64_t> *lengths) {
+    std::string h = "@HD\tVN:1.6\tSO:coordinate\n";
+    for (size_t k = 0; k < names.size(); k++) {
+        h += "@SQ\tSN:"; h += names[k];
+        if (lengths && (*lengths)[k] != UINT64_MAX) { h += "\tLN:"; h += std::to_string((unsigned long long)(*lengths)[k]); }
+        h += '\n';
+    }
+    return h;
+}
+extern "C" int cbcg_sam_header(const uint8_t *in, uint64_t in_len, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!out_len) return CBCG_ERR_ARG;
+    *out_len = 0;
+    Container c;
+    const int rc = parse_container(in, in_len, nullptr, c);
+    if (rc) return rc;
+    const std::string h = sam_header_text(container_names(in, c), nullptr);
+    *out_len = h.size();
+    if (!out || h.size() > out_cap) return CBCG_ERR_CAPACITY;
+    memcpy(out, h.data(), h.size());
+    return CBCG_OK;
+}
+
+extern "C" int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                               const uint8_t *section, uint64_t section_len,
+                               const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
+                               uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                               uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
+    if (!ctx || !out_len || (flags & ~CBCG_SAM_HEADER) || (!regions && n_regions) || (section && !section_len))
+        return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_sam: bad argument");
+    *out_len = 0; if (n_reads) *n_reads = 0;
+    if (regions) TRY(check_regions(ctx, regions, n_regions));
+    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
+    /* the chromosome table (legacy: the loaded reference) and the read count the section must match */
+    std::vector<std::string> table = ctx->names;
+    uint64_t cont_reads = 0;
+    if (!legacy) {
+        Container c;
+        if (parse_container(in, in_len, nullptr, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
+        table = container_names(in, c);
+        cont_reads = c.n_reads;
+    }
+    std::vector<uint8_t> cls;
+    std::vector<uint64_t> exc_read, exc_off(1, 0);
+    std::vector<uint8_t> exc_text;
+    if (section && !legacy) TRY(parse_cigar_section(ctx, section, section_len, cont_reads, cls, exc_read, exc_off, exc_text));
+    /* records: every read, or the region's (with their container ordinals) */
+    uint64_t nr = 0, ne = 0, n_sel = 0; uint32_t max_len = 1, fixed_len = 0;
+    const cbcg_read_rec *d_recs = ctx->recs.as<cbcg_read_rec>();
+    const uint32_t *d_chr = nullptr; const uint64_t *d_ids = nullptr;
+    uint32_t ref_hint = 0;
+    if (!regions) {
+        TRY(decode_to_records(ctx, in, in_len, legacy, &nr, &ne, &max_len, &fixed_len));
+        if (legacy) max_len = CBCG_MAX_READ_LEN;            /* per-read lengths are coded mod 256 (src/read_compression.c:29-33) */
+        else ref_hint = ref_window_from_blocks(ctx, max_len);
+        n_sel = nr;
+        d_recs = ctx->recs.as<cbcg_read_rec>(); d_chr = ctx->chr_out.as<uint32_t>();
+    } else {
+        TRY(region_records(ctx, in, in_len, legacy, regions, n_regions, &nr, &ne, &n_sel, &max_len, &fixed_len));
+        d_recs = ctx->sel_recs.as<cbcg_read_rec>(); d_chr = ctx->sel_chr.as<uint32_t>(); d_ids = ctx->sel_ids.as<uint64_t>();
+    }
+    if (section && legacy) TRY(parse_cigar_section(ctx, section, section_len, nr, cls, exc_read, exc_off, exc_text));   /* a legacy stream is decoded whole */
+    cbcg_stats &S = ctx->stats;
+    std::vector<uint64_t> lengths(table.size(), UINT64_MAX);
+    for (size_t k = 0; k < table.size(); k++)
+        for (size_t g = 0; g < ctx->names.size(); g++)
+            if (ctx->names[g] == table[k]) { lengths[k] = ctx->h_len[g]; break; }
+    const std::string head = (flags & CBCG_SAM_HEADER) ? sam_header_text(table, &lengths) : std::string();
+    uint64_t rec_bytes = 0;
+    if (n_sel) {
+        TRY(run_reconstruct(ctx, n_sel, max_len, fixed_len, d_chr, ref_hint, d_recs));
+        /* an upper bound on the lines (k6_sam.cu): per read 64 bytes of fields, the name, SEQ, 16 per edit (implied CIGAR +
+           MD), and per verbatim CIGAR its text, 4 per base and 5 per deleted base (<= 255) of MD */
+        size_t max_name = 0;
+        std::vector<uint32_t> name_len(ctx->names.size());
+        for (size_t g = 0; g < ctx->names.size(); g++) { name_len[g] = (uint32_t)ctx->names[g].size(); max_name = std::max(max_name, ctx->names[g].size()); }
+        const uint64_t bound = n_sel * (64u + max_name + max_len) + 16u * ne + exc_text.size() + exc_read.size() * (4u * max_len + 5u * 255u + 8u) + 64u;
+        const uint64_t n_exc = exc_read.size();
+        const uint64_t aux = name_len.size() * 4 + cls.size() + (2 * n_exc + 1) * 8 + exc_text.size() + 256;
+        TRY(ensure(ctx, ctx->sam_aux, aux));
+        TRY(ensure(ctx, ctx->sam_out, head.size() + bound + 64));
+        TRY(ensure(ctx, ctx->tile_desc, (2 * sam_num_tiles(n_sel) + 1) * 8));
+        uint8_t *a = ctx->sam_aux.as<uint8_t>();
+        uint64_t *d_read = reinterpret_cast<uint64_t *>(a), *d_off = d_read + n_exc;
+        uint32_t *d_nl = reinterpret_cast<uint32_t *>(d_off + n_exc + 1);
+        uint8_t *d_cls = reinterpret_cast<uint8_t *>(d_nl + name_len.size()), *d_text = d_cls + cls.size();
+        if (n_exc) CU(cudaMemcpyAsync(d_read, exc_read.data(), n_exc * 8, cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaMemcpyAsync(d_off, exc_off.data(), (n_exc + 1) * 8, cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaMemcpyAsync(d_nl, name_len.data(), name_len.size() * 4, cudaMemcpyHostToDevice, ctx->st));
+        if (!cls.empty()) CU(cudaMemcpyAsync(d_cls, cls.data(), cls.size(), cudaMemcpyHostToDevice, ctx->st));
+        if (!exc_text.empty()) CU(cudaMemcpyAsync(d_text, exc_text.data(), exc_text.size(), cudaMemcpyHostToDevice, ctx->st));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        if (launch_sam(n_sel, d_recs, d_chr, ctx->edits.as<uint16_t>(), ctx->dg, ctx->g_names.as<uint8_t>(), d_nl, ctx->seq_out.as<uint8_t>(),
+                       max_len, fixed_len, d_ids, section ? d_cls : nullptr, d_read, d_off, d_text, n_exc,
+                       ctx->sam_out.as<uint8_t>() + head.size(), bound, ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)),
+                       wptr<uint64_t>(ctx, W_OFF(total_bytes)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+            return fail(ctx, CBCG_ERR_CUDA, "K6 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        ctx->stats.kernel_launches++;
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+        TRY(fetch_words(ctx));                               /* synchronises: the host vectors above may go */
+        TRY(device_error(ctx, "SAM output"));
+        cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
+        rec_bytes = ctx->hw->total_bytes;
+    } else {
+        TRY(ensure(ctx, ctx->sam_out, head.size() + 64));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+    }
+    /* the SAM text becomes "the decoded text" that cbcg_fetch_decoded returns */
+    std::swap(ctx->seq_out, ctx->sam_out);
+    const uint64_t bytes = head.size() + rec_bytes;
+    *out_len = bytes; if (n_reads) *n_reads = n_sel;
+    ctx->dec_bytes = bytes; ctx->dec_n_reads = n_sel; ctx->have_decoded = true;
+    if (bytes > out_cap || (!out && bytes) || (read_ids && n_sel > ids_cap))
+        return fail(ctx, CBCG_ERR_CAPACITY, "%llu reads / %llu bytes of SAM, room for %llu / %llu", (unsigned long long)n_sel,
+                    (unsigned long long)bytes, (unsigned long long)ids_cap, (unsigned long long)out_cap);
+    CU(cudaEventRecord(ctx->ev[4], ctx->st));
+    if (bytes) CU(cudaMemcpyAsync(out, ctx->seq_out.p, bytes, cudaMemcpyDeviceToHost, ctx->st));
+    if (read_ids && n_sel) {
+        if (d_ids) CU(cudaMemcpyAsync(read_ids, d_ids, n_sel * 8, cudaMemcpyDeviceToHost, ctx->st));
+        else for (uint64_t r = 0; r < n_sel; r++) read_ids[r] = r;
+    }
+    CU(cudaEventRecord(ctx->ev[5], ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    cudaEventElapsedTime(&S.ms_h2d, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&S.ms_code, ctx->ev[1], ctx->ev[2]);
+    cudaEventElapsedTime(&S.ms_reconstruct, ctx->ev[2], ctx->ev[3]);
+    cudaEventElapsedTime(&S.ms_d2h, ctx->ev[4], ctx->ev[5]);
+    cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[5]);
+    S.d2h_bytes = bytes + (read_ids && d_ids ? n_sel * 8 : 0);
     return CBCG_OK;
 }
 

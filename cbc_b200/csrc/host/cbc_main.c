@@ -13,7 +13,13 @@
  *          -r NAME[:START[-END]]   -d only, repeatable: write only the reads that overlap one of the regions (1-based, inclusive;
  *                   cbcg_decode_region), each once, in file order. The region is split at the last ':', so record names that
  *                   contain one still work. Every batch of a "CBCS" file gets the same regions; a batch that none of them
- *                   touches (cbcg_region_plan: no blocks) makes no device call. Not with -C.
+ *                   touches (cbcg_region_plan: no blocks) makes no device call. Not with -C unless with -S.
+ *          -S       -d only: write SAM (cbcg_decode_sam): a header, then one alignment record per read (QNAME, MAPQ, mate fields
+ *                   and QUAL are not stored: `*`, 255, `*`, 0, 0, `*`), with NM and MD recomputed against the reference. The
+ *                   header is written once: for a "CBCB" or "CBCS" input from batch 0's chromosome table (cbcg_sam_header; a
+ *                   later batch whose table differs is an error), for a single-block stream from the reference; LN comes
+ *                   from the reference. With -C the CIGARs are the input's (<in>.cig), else the ones the indels imply.
+ *                   With -r only the region's records.
  *
  * Host C only: SAM/FASTA ingest (sam_ingest.c) and file I/O; the coding runs on the GPU through include/cbcg.h.
  * Where the reference's compress() (src/compression.c:112-170) reads a line, codes it and moves on, this driver
@@ -43,7 +49,8 @@ static double now(void) { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t);
 static int usage(void) {
     fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
                     "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
-                    "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n");
+                    "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n"
+                    "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n");
     return 2;
 }
 
@@ -71,7 +78,7 @@ typedef struct shared {
     uint64_t next_take;                         /* next job a device thread takes */
     int producer_failed;
     /* run parameters */
-    int mode, single, var_length, with_cigar; uint32_t block_reads;
+    int mode, single, var_length, with_cigar, sam; uint32_t block_reads;
     const cbch_fasta *fa; int fa_ready;
     const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
     double t_gpu_ready;
@@ -129,6 +136,25 @@ static void *device_main(void *arg) {
                 }
             }
             if (J->have_compact) cbch_free_compact(&J->cb);
+        } else if (S->sam) {                                      /* SAM records; the writer adds the header */
+            uint64_t nb = 1, n_reads = 0, pb = 0, cap = 0, n = 0;
+            if (S->n_regions) {
+                rc = cbcg_region_plan(J->in, J->in_len, J->legacy, S->regions, S->n_regions, &nb, &n_reads, &pb, &cap);
+                if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "region plan: %s", cbcg_strerror(rc)); nb = 0; }
+            }
+            if (nb) {                                             /* a batch that no region touches costs no device call */
+                if (J->legacy || cbcg_decoded_size(J->in, J->in_len, &n_reads, &cap) != CBCG_OK) cap = 1u << 20;
+                cap = 2 * cap + (1u << 16);                       /* SAM lines: about SEQ + 60 bytes */
+                tq = now();
+                J->out = (uint8_t *)malloc(cap);
+                rc = J->out ? cbcg_decode_sam(ctx, J->in, J->in_len, J->legacy, S->with_cigar ? J->cig_in : NULL, S->with_cigar ? J->cig_in_len : 0,
+                                              S->n_regions ? S->regions : NULL, S->n_regions, 0u, J->out, cap, &n, NULL, 0, &n_reads) : CBCG_ERR_NOMEM;
+                if (rc == CBCG_ERR_CAPACITY && n > cap) { free(J->out); J->out = (uint8_t *)malloc(n); rc = J->out ? cbcg_fetch_decoded(ctx, J->out, n, &n) : CBCG_ERR_NOMEM; }
+                if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "%s", ctx ? cbcg_last_error(ctx) : "no context"); }
+                J->out_len = n; J->n_reads = n_reads;
+                D->call_s += now() - tq;
+                cbcg_stats st; cbcg_get_stats(ctx, &st); J->device_ms = st.ms_total;
+            }
         } else if (S->n_regions) {
             uint64_t nb = 0, n_reads = 0, pb = 0, cap = 0, n = 0;
             rc = cbcg_region_plan(J->in, J->in_len, J->legacy, S->regions, S->n_regions, &nb, &n_reads, &pb, &cap);
@@ -228,6 +254,46 @@ static void *ingest_main(void *arg) {
     return NULL;
 }
 
+/* The SAM header: @HD and the @SQ lines of batch 0's chromosome table (a single-block stream: of the reference), each with
+ * LN from the reference when it holds the name. */
+static int write_sam_header(FILE *fo, const job *J0, const cbch_fasta *fa) {
+    uint8_t *h = NULL; uint64_t n = 0;
+    if (!J0->legacy) {
+        if (cbcg_sam_header(J0->in, J0->in_len, NULL, 0, &n) != CBCG_ERR_CAPACITY || !(h = (uint8_t *)malloc(n)) ||
+            cbcg_sam_header(J0->in, J0->in_len, h, n, &n) != CBCG_OK) { free(h); return 1; }
+    } else {
+        uint64_t cap = 64;
+        for (uint32_t k = 0; k < fa->n; k++) cap += strlen(fa->names[k]) + 16;
+        if (!(h = (uint8_t *)malloc(cap))) return 1;
+        n = (uint64_t)snprintf((char *)h, cap, "@HD\tVN:1.6\tSO:coordinate\n");
+        for (uint32_t k = 0; k < fa->n; k++) n += (uint64_t)snprintf((char *)h + n, cap - n, "@SQ\tSN:%s\n", fa->names[k]);
+    }
+    int rc = 0;
+    for (const uint8_t *l = h, *e = h + n; l < e && !rc;) {
+        const uint8_t *nl = (const uint8_t *)memchr(l, '\n', (size_t)(e - l));
+        if (!nl) nl = e;
+        if (fwrite(l, 1, (size_t)(nl - l), fo) != (size_t)(nl - l)) rc = 1;
+        if (nl - l > 7 && !memcmp(l, "@SQ\tSN:", 7))
+            for (uint32_t k = 0; k < fa->n; k++)
+                if (strlen(fa->names[k]) == (size_t)(nl - l - 7) && !memcmp(fa->names[k], l + 7, (size_t)(nl - l - 7))) {
+                    fprintf(fo, "\tLN:%llu", (unsigned long long)fa->len[k]); break;
+                }
+        if (fputc('\n', fo) == EOF) rc = 1;
+        l = nl + 1;
+    }
+    free(h);
+    return rc;
+}
+/* 1 when batch k's chromosome table differs from batch 0's */
+static int sam_table_differs(const job *J0, const job *J) {
+    uint64_t a = 0, b = 0;
+    if (cbcg_sam_header(J0->in, J0->in_len, NULL, 0, &a) != CBCG_ERR_CAPACITY || cbcg_sam_header(J->in, J->in_len, NULL, 0, &b) != CBCG_ERR_CAPACITY || a != b) return 1;
+    uint8_t *x = (uint8_t *)malloc(a), *y = (uint8_t *)malloc(b);
+    int d = !x || !y || cbcg_sam_header(J0->in, J0->in_len, x, a, &a) || cbcg_sam_header(J->in, J->in_len, y, b, &b) || memcmp(x, y, a);
+    free(x); free(y);
+    return d;
+}
+
 /* NAME[:START[-END]], split at the last ':' when what follows it is START or START-END (else the whole text is the name) */
 static int parse_region(const char *a, cbcg_region *r) {
     const char *c = strrchr(a, ':');
@@ -263,7 +329,7 @@ static int parse_devices(const char *s, int *dev) {
 }
 
 int main(int argc, char **argv) {
-    int mode = 0, single = 0, var_length = 0, with_cigar = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
+    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
     uint32_t block_reads = CBCG_BLOCK_AUTO;
     uint64_t batch_mb = 2048;
     const char *files[4]; int nfiles = 0;
@@ -275,6 +341,7 @@ int main(int argc, char **argv) {
         else if (!strcmp(a, "-1")) single = 1;
         else if (!strcmp(a, "-l")) var_length = 1;
         else if (!strcmp(a, "-C")) with_cigar = 1;
+        else if (!strcmp(a, "-S")) sam = 1;
         else if (!strcmp(a, "-b") && i + 1 < argc) block_reads = (uint32_t)strtoul(argv[++i], NULL, 10);
         else if (!strcmp(a, "-B") && i + 1 < argc) batch_mb = strtoull(argv[++i], NULL, 10);
         else if (!strcmp(a, "-r") && i + 1 < argc) {
@@ -297,7 +364,8 @@ int main(int argc, char **argv) {
     }
     if (!mode || nfiles != 3) { fprintf(stderr, "Missing required filenames\n"); return usage(); }
     if (n_regions && mode != 'd') { fprintf(stderr, "cbc: -r selects reads to decode: it goes with -d\n"); return usage(); }
-    if (n_regions && with_cigar) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
+    if (sam && mode != 'd') { fprintf(stderr, "cbc: -S writes SAM: it goes with -d\n"); return usage(); }
+    if (n_regions && with_cigar && !sam) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
     if (!single && block_reads == 0) block_reads = CBCG_BLOCK_AUTO;
     if (batch_mb < 1) batch_mb = 1;
 
@@ -305,7 +373,7 @@ int main(int argc, char **argv) {
     shared S; memset(&S, 0, sizeof S);
     pthread_mutex_init(&S.mu, NULL); pthread_cond_init(&S.cv, NULL);
     S.mode = mode; S.single = single; S.var_length = var_length; S.block_reads = block_reads; S.with_cigar = with_cigar;
-    S.regions = regions; S.n_regions = n_regions;
+    S.regions = regions; S.n_regions = n_regions; S.sam = sam;
     devthread D[MAX_DEV]; memset(D, 0, sizeof D);
 
     /* ---- the input, cut into jobs (before the device threads start: they index S.jobs) */
@@ -404,7 +472,9 @@ int main(int argc, char **argv) {
         job *J = wait_done(&S, k);
         if (!J) { fprintf(stderr, "cbc: %s\n", IA.err[0] ? IA.err : "ingest failed"); status = 1; break; }
         if (J->rc) { fprintf(stderr, "cbc: %s\n", J->err); status = 1; break; }
-        if (with_cigar && mode == 'd') {                         /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
+        if (sam && k == 0 && write_sam_header(fo, J, &fa)) { fprintf(stderr, "cbc: cannot write the SAM header of %s\n", files[0]); status = 1; break; }
+        if (sam && k > 0 && sam_table_differs(S.jobs[0], J)) { fprintf(stderr, "cbc: batch %llu names other chromosomes than batch 0: one SAM header cannot describe both\n", (unsigned long long)k); status = 1; break; }
+        if (with_cigar && mode == 'd' && !sam) {                         /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
             const uint8_t *c = J->cig, *ce = J->cig + J->cig_len, *q = J->out, *qe = J->out + J->out_len;
             while (c < ce && q < qe) {
                 const uint8_t *cn = (const uint8_t *)memchr(c, '\n', (size_t)(ce - c)), *qn = (const uint8_t *)memchr(q, '\n', (size_t)(qe - q));

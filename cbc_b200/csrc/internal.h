@@ -153,3 +153,13 @@ uint64_t region_num_tiles(uint64_t n_reads);
 int launch_region_select(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr, const RegionIv *iv, uint32_t n_iv,
                          const uint64_t *runs, uint32_t n_runs, cbcg_read_rec *out_recs, uint32_t *out_chr, uint64_t *out_ids,
                          uint64_t *tile_desc, uint32_t *ticket, uint64_t *total, unsigned long long *err, cudaStream_t st);
+/* k6_sam.cu: SAM lines from records + K3's text (seq_text, SEQ + '\n' per read; fixed_len: every read that long). names: MAX_NAME
+   bytes per genome record, name_len their lengths. ids (optional): container ordinal per read, the index into cls (optional,
+   per container read: CIGAR class); exc_*: the class-4 reads' texts by ascending container ordinal. tile_desc: 2 x
+   sam_num_tiles(n_reads) words. *total_bytes receives the text's size. */
+uint64_t sam_num_tiles(uint64_t n_reads);
+int launch_sam(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr, const uint16_t *edits, const DevGenome &g,
+               const uint8_t *names, const uint32_t *name_len, const uint8_t *seq_text, uint32_t max_len, uint32_t fixed_len,
+               const uint64_t *ids, const uint8_t *cls, const uint64_t *exc_read, const uint64_t *exc_off, const uint8_t *exc_text,
+               uint64_t n_exc, uint8_t *out, uint64_t out_cap, uint64_t *tile_desc, uint32_t *ticket, uint64_t *total_bytes,
+               unsigned long long *err, cudaStream_t st);

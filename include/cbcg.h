@@ -236,6 +236,34 @@ int cbcg_decode_region(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int le
                        uint8_t *seq_out, uint64_t seq_cap, uint64_t *seq_len,
                        uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
 
+/* ---- SAM output (DESIGN.md, "SAM output"): the reads as alignment records, one line per read in container order:
+ *     *  FLAG  RNAME  POS  255  CIGAR  *  0  0  SEQ  *  NM:i:<n>  MD:Z:<md>
+ * (tab-separated). QNAME, MAPQ, RNEXT, PNEXT, TLEN and QUAL are not stored: they carry the SAM spec's "unavailable"
+ * values. RNAME is the chromosome's name; SEQ is what cbcg_decode returns. CIGAR: the read's text from the side section
+ * (byte for byte the input's, as cbcg_cigar_unpack); without a section the implied CIGAR (soft clips read as I).
+ * MD and NM are recomputed from the line's CIGAR, its SEQ and the loaded reference (upper-cased): M, = and X consume read
+ * and reference, I and S the read, D the reference, H and P neither; an aligned base is a mismatch when it differs from
+ * the reference base, so N against N is not one (samtools calmd counts it); MD is spelled [0-9]+(([A-Z]|\^[A-Z]+)[0-9]+)*
+ * with reference letters; NM = mismatches + I bases + D bases.
+ * The header: @HD VN:1.6 SO:coordinate, then @SQ SN:<name> per chromosome of the container's table (legacy stream: of the
+ * loaded reference). The container does not store record lengths: cbcg_sam_header writes no LN; cbcg_decode_sam writes
+ * LN:<len> from the loaded reference for every name it holds. */
+#define CBCG_SAM_HEADER 1u
+/* @HD + @SQ lines of a blocked container, from its header alone: no context, no device, no payload read. A malformed
+ * header -> CBCG_ERR_FORMAT; out_cap too small -> CBCG_ERR_CAPACITY with *out_len the size needed. */
+int cbcg_sam_header(const uint8_t *in, uint64_t in_len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+/* SAM records (flags & CBCG_SAM_HEADER: the header first). section / section_len: the CIGAR side section or NULL; its read
+ * count must be the container's (the header's n_reads; legacy: the stream's), else CBCG_ERR_FORMAT.
+ * regions / n_regions: NULL / 0 = every read; otherwise cbcg_decode_region's selection and overlap rule (n_regions == 0
+ * with regions != NULL -> CBCG_ERR_ARG). read_ids (optional): each line's read ordinal in the container.
+ * Errors, capacity (cbcg_fetch_decoded then returns the SAM text), statistics and state as cbcg_decode_region; K6's time
+ * is part of ms_reconstruct, ms_k3 is K3's alone. */
+int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                    const uint8_t *section, uint64_t section_len,
+                    const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
+                    uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                    uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
+
 /* ---- device-resident variants (inputs already in HBM when the timed region starts): upload once,
  * run many times. Results stay on the device until fetched. Used by bench.py for `value`. */
 int cbcg_batch_upload(cbcg_ctx *ctx, const cbcg_batch *batch);                 /* replaces the resident batch */
