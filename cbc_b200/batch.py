@@ -3,12 +3,13 @@
 A ``Batch`` is what the reference's ``load_sam_line`` (src/sam_file_allocation.c:437-529)
 yields per SAM record, laid out structure-of-arrays: POS, FLAG, SEQ length, chromosome
 ordinal and three byte pools (SEQ, CIGAR text, MD:Z payload) with n+1 offsets each.
+A batch without MD (``md_off`` and ``md`` None) has its MD derived on the GPU (include/cbcg.h).
 """
 from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, field
-from typing import List
+from typing import List, Optional
 
 import numpy as np
 
@@ -34,8 +35,8 @@ class Batch:
     seq: np.ndarray        # uint8
     cigar_off: np.ndarray  # uint64 [n+1]
     cigar: np.ndarray      # uint8
-    md_off: np.ndarray     # uint64 [n+1]
-    md: np.ndarray         # uint8
+    md_off: Optional[np.ndarray]   # uint64 [n+1]; None with md: no MD, the library derives it
+    md: Optional[np.ndarray]       # uint8
 
     @property
     def n_reads(self) -> int:
@@ -46,12 +47,17 @@ class Batch:
                          ("seq_off", np.uint64), ("seq", np.uint8), ("cigar_off", np.uint64),
                          ("cigar", np.uint8), ("md_off", np.uint64), ("md", np.uint8)):
             a = getattr(self, name)
-            assert a.dtype == dt and a.flags["C_CONTIGUOUS"], name
+            assert (a is None and name in ("md_off", "md")) or (a.dtype == dt and a.flags["C_CONTIGUOUS"]), name
         s = CBatch()
         s.n_reads = self.n_reads
         for name in ("pos", "flag", "seq_len", "chr", "seq_off", "seq", "cigar_off", "cigar", "md_off", "md"):
-            setattr(s, name, getattr(self, name).ctypes.data)
+            a = getattr(self, name)
+            setattr(s, name, a.ctypes.data if a is not None else None)
         return s
+
+    def without_md(self) -> "Batch":
+        """The same reads without MD (the arrays are shared): the library derives each read's MD on the GPU."""
+        return Batch(self.pos, self.flag, self.seq_len, self.chr, self.seq_off, self.seq, self.cigar_off, self.cigar, None, None)
 
     def slice(self, r0: int, r1: int) -> "Batch":
         """Reads [r0, r1) as an independent batch (pools re-based)."""
@@ -60,7 +66,7 @@ class Batch:
             return (off[r0:r1 + 1] - off[r0]).astype(np.uint64), np.ascontiguousarray(data[lo:hi])
         so, s = pool(self.seq_off, self.seq)
         co, c = pool(self.cigar_off, self.cigar)
-        mo, m = pool(self.md_off, self.md)
+        mo, m = pool(self.md_off, self.md) if self.md_off is not None else (None, None)
         return Batch(self.pos[r0:r1].copy(), self.flag[r0:r1].copy(), self.seq_len[r0:r1].copy(),
                      self.chr[r0:r1].copy(), so, s, co, c, mo, m)
 

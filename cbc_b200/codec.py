@@ -42,7 +42,7 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_reconstruct", "cbcg_batch_upload", "cbcg_encode_resident", "cbcg_decode_resident",
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
            "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
-           "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam"]
+           "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam", "cbcg_derive_md"]
 
 
 UINT64_MAX = (1 << 64) - 1
@@ -163,6 +163,7 @@ def load_library():
         lib.cbcg_decode_region.argtypes = [vp, vp, u64, C.c_int, P(Region), u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_sam_header.argtypes = [vp, u64, vp, u64, P(u64)]
         lib.cbcg_decode_sam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
+        lib.cbcg_derive_md.argtypes = [vp, P(CBatch), vp, u64, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -191,6 +192,8 @@ def pinned_empty(n: int, dtype) -> np.ndarray:
 def pin_batch(b: Batch) -> Batch:
     """Copy of a batch in page-locked memory (what a production ingest thread would fill directly)."""
     def pin(a):
+        if a is None:
+            return None
         out = pinned_empty(a.shape[0], a.dtype)
         out[:] = a
         return out
@@ -477,6 +480,21 @@ class Codec:
                 continue
             self._check(rc)
             return recs[:nr.value].copy(), chr_[:nr.value].copy(), edits[:ne.value].copy()
+
+    def derive_md(self, batch: Batch) -> bytes:
+        """Each read's MD as a batch without MD gets it on the GPU (include/cbcg.h, cbcg_derive_md): MD + '\\n' per read, in
+        read order. Any MD the batch carries is ignored. The batch becomes the resident batch, with the derived MD."""
+        cb = batch.c_struct()
+        cap = batch.total_bases() // 4 + 16 * batch.n_reads + 4096
+        while True:
+            out = np.empty(max(cap, 1), np.uint8)
+            n = C.c_uint64(0)
+            rc = self.lib.cbcg_derive_md(self.h, C.byref(cb), out.ctypes.data, out.nbytes, C.byref(n))
+            if rc == -5 and n.value > out.nbytes:
+                cap = n.value
+                continue
+            self._check(rc)
+            return out[:n.value].tobytes()
 
     # ---- K3
     def reconstruct(self, recs: np.ndarray, chr_: np.ndarray, edits: np.ndarray) -> bytes:

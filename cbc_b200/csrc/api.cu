@@ -42,6 +42,7 @@ struct Words {
     uint32_t pad;
     uint64_t chain[2];                        /* pipelined encode: edit entries so far, ping-pong between K1 launches */
     uint64_t n_selected;                      /* region decode: reads K5 kept */
+    uint64_t md_chain[2];                     /* MD derivation (K7): MD bytes of the batch ([0]), or so far, ping-pong between chunk launches */
 };
 
 struct cbcg_ctx {
@@ -71,6 +72,7 @@ struct cbcg_ctx {
     std::vector<ChrRun> runs;
     uint64_t total_bases = 0;
     bool have_batch = false;
+    bool batch_no_md = false;                 /* the resident batch came without MD: K7 derives it (DESIGN.md 5d) */
 
     /* compact batches (cbcg_batch_compact): staging for what is unpacked on the device */
     DevBuf c_seq2, c_cl, c_ml, c_tile, c_rfirst, c_rchr, c_er, c_eb, c_ec;
@@ -308,23 +310,30 @@ extern "C" int cbcg_set_reference(cbcg_ctx *ctx, uint32_t n_chr, const char *con
 static int check_batch(cbcg_ctx *ctx, const cbcg_batch *b) {
     if (!b) return fail(ctx, CBCG_ERR_ARG, "NULL batch");
     if (b->n_reads == 0) return 0;
-    if (!b->pos || !b->flag || !b->seq_len || !b->chr || !b->seq_off || !b->seq || !b->cigar_off || !b->cigar || !b->md_off || !b->md)
+    const bool no_md = !b->md_off && !b->md;               /* no MD: K7 derives it */
+    if (!b->pos || !b->flag || !b->seq_len || !b->chr || !b->seq_off || !b->seq || !b->cigar_off || !b->cigar || (!no_md && (!b->md_off || !b->md)))
         return fail(ctx, CBCG_ERR_ARG, "batch has NULL arrays");
     if (b->n_reads >= 0xfffffff0ull) return fail(ctx, CBCG_ERR_ARG, "more than 2^32 reads in one shard");
     const uint64_t n = b->n_reads;                          /* the copies are sized from the pool offsets' end points */
-    if (b->seq_off[n] < b->seq_off[0] || b->cigar_off[n] < b->cigar_off[0] || b->md_off[n] < b->md_off[0])
+    if (b->seq_off[n] < b->seq_off[0] || b->cigar_off[n] < b->cigar_off[0] || (!no_md && b->md_off[n] < b->md_off[0]))
         return fail(ctx, CBCG_ERR_INPUT, "batch pool offsets decrease");
     return 0;
 }
+
+/* MD pool of a batch without MD, before K7 has counted it: canonical MD is about a digit or two per run of matches and two
+ * or three bytes per edit, so an eighth of the bases plus 8 per read covers a batch with one edit in twenty bases several
+ * times over. A batch that needs more is derived again at the exact size (derive_md). */
+static uint64_t md_bytes_guess(uint64_t bases, uint64_t n) { return bases / 8 + 8 * n + 4096; }
 
 /* Device buffers for the batch and ctx->db pointing at them (no copies yet). */
 static int batch_prepare(cbcg_ctx *ctx, const cbcg_batch *b) {
     const uint64_t n = b->n_reads;
     ctx->have_batch = false; ctx->have_encoded = false;
+    ctx->batch_no_md = !b->md_off;
     ctx->runs.clear();
     ctx->stats = cbcg_stats();
     if (n) {
-        const uint64_t seq_b = b->seq_off[n], cig_b = b->cigar_off[n], md_b = b->md_off[n];
+        const uint64_t seq_b = b->seq_off[n], cig_b = b->cigar_off[n], md_b = b->md_off ? b->md_off[n] : md_bytes_guess(seq_b - b->seq_off[0], n);
         TRY(ensure(ctx, ctx->b_pos, n * 4));  TRY(ensure(ctx, ctx->b_flag, n * 2)); TRY(ensure(ctx, ctx->b_len, n * 2));
         TRY(ensure(ctx, ctx->b_chr, n * 4));
         TRY(ensure(ctx, ctx->b_soff, (n + 1) * 8)); TRY(ensure(ctx, ctx->b_coff, (n + 1) * 8)); TRY(ensure(ctx, ctx->b_moff, (n + 1) * 8));
@@ -343,13 +352,14 @@ static int batch_prepare(cbcg_ctx *ctx, const cbcg_batch *b) {
 static int batch_copy_range(cbcg_ctx *ctx, const cbcg_batch *b, uint64_t r0, uint64_t r1, cudaStream_t st, uint64_t *bytes) {
     if (r1 <= r0) return 0;
     const uint64_t m = r1 - r0;
-    const uint64_t s0 = b->seq_off[r0], s1 = b->seq_off[r1], c0 = b->cigar_off[r0], c1 = b->cigar_off[r1], m0 = b->md_off[r0], m1 = b->md_off[r1];
+    const bool md = b->md_off != nullptr;                   /* without MD there is none to copy: K7 writes md_off and the pool */
+    const uint64_t s0 = b->seq_off[r0], s1 = b->seq_off[r1], c0 = b->cigar_off[r0], c1 = b->cigar_off[r1], m0 = md ? b->md_off[r0] : 0, m1 = md ? b->md_off[r1] : 0;
     struct { void *d; const void *h; uint64_t bytes; } cp[] = {
         { ctx->b_pos.as<uint32_t>() + r0, b->pos + r0, m * 4 }, { ctx->b_flag.as<uint16_t>() + r0, b->flag + r0, m * 2 },
         { ctx->b_len.as<uint16_t>() + r0, b->seq_len + r0, m * 2 }, { ctx->b_chr.as<uint32_t>() + r0, b->chr + r0, m * 4 },
         { ctx->b_soff.as<uint64_t>() + r0, b->seq_off + r0, (m + 1) * 8 }, { ctx->b_coff.as<uint64_t>() + r0, b->cigar_off + r0, (m + 1) * 8 },
-        { ctx->b_moff.as<uint64_t>() + r0, b->md_off + r0, (m + 1) * 8 }, { ctx->b_seq.as<uint8_t>() + s0, b->seq + s0, s1 - s0 },
-        { ctx->b_cigar.as<uint8_t>() + c0, b->cigar + c0, c1 - c0 }, { ctx->b_md.as<uint8_t>() + m0, b->md + m0, m1 - m0 } };
+        { ctx->b_moff.as<uint64_t>() + r0, md ? b->md_off + r0 : nullptr, md ? (m + 1) * 8 : 0 }, { ctx->b_seq.as<uint8_t>() + s0, b->seq + s0, s1 - s0 },
+        { ctx->b_cigar.as<uint8_t>() + c0, b->cigar + c0, c1 - c0 }, { ctx->b_md.as<uint8_t>() + m0, md ? b->md + m0 : nullptr, m1 - m0 } };
     for (auto &c : cp) { if (c.bytes) CU(cudaMemcpyAsync(c.d, c.h, c.bytes, cudaMemcpyHostToDevice, st)); *bytes += c.bytes; }
     return 0;
 }
@@ -371,7 +381,7 @@ static int batch_scan(cbcg_ctx *ctx, const cbcg_batch *b) {
     uint64_t bad = 0;
     if (n) {
         const uint16_t *sl = b->seq_len;
-        const uint64_t *so = b->seq_off, *co = b->cigar_off, *mo = b->md_off;
+        const uint64_t *so = b->seq_off, *co = b->cigar_off, *mo = b->md_off ? b->md_off : b->cigar_off;   /* no MD: nothing more to check */
         for (uint64_t r = 0; r < n; r++) {
             const uint32_t l = sl[r]; max_len = l > max_len ? l : max_len; min_len = l < min_len ? l : min_len;
             /* SEQ pool entries are exactly the reads; CIGAR / MD offsets never decrease (kernels size their loops from them) */
@@ -399,12 +409,14 @@ static int batch_scan(cbcg_ctx *ctx, const cbcg_batch *b) {
 
 static int reset_words(cbcg_ctx *ctx);
 static int fetch_words(cbcg_ctx *ctx);
+static int derive_md(cbcg_ctx *ctx, uint64_t need);
 /* ---- compact batches: what crosses the link packed, rebuilt into the layout above on the device (k0_unpack.cu) */
 struct BatchSrc { const cbcg_batch *full; const cbcg_batch_compact *compact; uint64_t n; };
 static int check_compact(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
     if (!b) return fail(ctx, CBCG_ERR_ARG, "NULL batch");
     if (b->n_reads == 0) return 0;
-    if (!b->pos || !b->flag || !b->seq_len || !b->cigar_len || !b->md_len || !b->n_runs || !b->run_first || !b->run_chr || !b->seq2 || !b->cigar || !b->md ||
+    const bool no_md = !b->md_len && !b->md;               /* no MD: K7 derives it */
+    if (!b->pos || !b->flag || !b->seq_len || !b->cigar_len || (!no_md && (!b->md_len || !b->md)) || !b->n_runs || !b->run_first || !b->run_chr || !b->seq2 || !b->cigar ||
         !b->tile_base || (b->n_exc && (!b->exc_read || !b->exc_base || !b->exc_char)))
         return fail(ctx, CBCG_ERR_ARG, "compact batch has NULL arrays");
     if (b->n_reads >= 0xfffffff0ull) return fail(ctx, CBCG_ERR_ARG, "more than 2^32 reads in one shard");
@@ -415,6 +427,8 @@ static int check_compact(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
     for (int q = 0; q < 4; q++) if (b->tile_base[q] != 0) return fail(ctx, CBCG_ERR_INPUT, "compact batch: tile offsets must start at 0");
     if (b->tile_base[tiles * 4] > b->n_reads * (uint64_t)b->max_len || b->tile_base[tiles * 4 + 1] > b->tile_base[tiles * 4])
         return fail(ctx, CBCG_ERR_INPUT, "compact batch: totals inconsistent");
+    if (no_md)
+        for (uint64_t t = 0; t <= tiles; t++) if (b->tile_base[t * 4 + 3]) return fail(ctx, CBCG_ERR_INPUT, "compact batch without MD: its tile offsets count MD bytes");
     return 0;
 }
 /* Device buffers of a compact batch and ctx->db; chromosome runs and the exception list are checked here (both short),
@@ -422,6 +436,7 @@ static int check_compact(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
 static int compact_buffers(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
     const uint64_t n = b->n_reads, tiles = (n + 127u) / 128u;
     ctx->have_batch = false; ctx->have_encoded = false;
+    ctx->batch_no_md = !b->md_len;
     ctx->runs.clear();
     ctx->stats = cbcg_stats();
     uint64_t seq_b = 0;
@@ -438,7 +453,7 @@ static int compact_buffers(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
         for (uint64_t e = 0; e < b->n_exc; e++) if (b->exc_base[e] >= b->max_len) return fail(ctx, CBCG_ERR_INPUT, "compact batch: exception beyond the longest read");
         const uint64_t *tot = b->tile_base + tiles * 4;
         seq_b = tot[0];
-        const uint64_t s2_b = tot[1], cig_b = tot[2], md_b = tot[3];
+        const uint64_t s2_b = tot[1], cig_b = tot[2], md_b = b->md_len ? tot[3] : md_bytes_guess(seq_b, n);
         TRY(ensure(ctx, ctx->b_pos, n * 4));  TRY(ensure(ctx, ctx->b_flag, n * 2)); TRY(ensure(ctx, ctx->b_len, n * 2));
         TRY(ensure(ctx, ctx->b_chr, n * 4));
         TRY(ensure(ctx, ctx->b_soff, (n + 1) * 8)); TRY(ensure(ctx, ctx->b_coff, (n + 1) * 8)); TRY(ensure(ctx, ctx->b_moff, (n + 1) * 8));
@@ -465,6 +480,7 @@ static int compact_copy_head(cbcg_ctx *ctx, const cbcg_batch_compact *b, cudaStr
         { ctx->c_tile.p, b->tile_base, (tiles + 1) * 32 }, { ctx->c_rfirst.p, b->run_first, (uint64_t)b->n_runs * 8 }, { ctx->c_rchr.p, b->run_chr, (uint64_t)b->n_runs * 4 },
         { ctx->c_er.p, b->exc_read, b->n_exc * 4 }, { ctx->c_eb.p, b->exc_base, b->n_exc * 2 }, { ctx->c_ec.p, b->exc_char, b->n_exc } };
     for (auto &c : cp) { if (c.bytes) CU(cudaMemcpyAsync(c.d, c.h, c.bytes, cudaMemcpyHostToDevice, st)); *bytes += c.bytes; }
+    if (!b->md_len) CU(cudaMemsetAsync(ctx->c_ml.p, 0, b->n_reads * 2, st));   /* no MD: K0 lays out empty texts, K7 fills them in */
     return 0;
 }
 /* reads [r0, r1), both multiples of 128 (or the end of the batch) */
@@ -472,12 +488,12 @@ static int compact_copy_range(cbcg_ctx *ctx, const cbcg_batch_compact *b, uint64
     if (r1 <= r0) return 0;
     const uint64_t m = r1 - r0;
     const uint64_t *t0 = b->tile_base + (r0 >> 7) * 4, *t1 = b->tile_base + ((r1 + 127u) >> 7) * 4;
-    const uint64_t s0 = t0[1], s1 = t1[1], c0 = t0[2], c1 = t1[2], m0 = t0[3], m1 = t1[3];
+    const uint64_t s0 = t0[1], s1 = t1[1], c0 = t0[2], c1 = t1[2], m0 = t0[3], m1 = t1[3];   /* no MD: m0 = m1 = 0 (check_compact) */
     struct { void *d; const void *h; uint64_t bytes; } cp[] = {
         { ctx->b_pos.as<uint32_t>() + r0, b->pos + r0, m * 4 }, { ctx->b_flag.as<uint16_t>() + r0, b->flag + r0, m * 2 },
         { ctx->b_len.as<uint16_t>() + r0, b->seq_len + r0, m * 2 }, { ctx->c_cl.as<uint16_t>() + r0, b->cigar_len + r0, m * 2 },
-        { ctx->c_ml.as<uint16_t>() + r0, b->md_len + r0, m * 2 }, { ctx->c_seq2.as<uint8_t>() + s0, b->seq2 + s0, s1 - s0 },
-        { ctx->b_cigar.as<uint8_t>() + c0, b->cigar + c0, c1 - c0 }, { ctx->b_md.as<uint8_t>() + m0, b->md + m0, m1 - m0 } };
+        { ctx->c_ml.as<uint16_t>() + r0, b->md_len ? b->md_len + r0 : nullptr, b->md_len ? m * 2 : 0 }, { ctx->c_seq2.as<uint8_t>() + s0, b->seq2 + s0, s1 - s0 },
+        { ctx->b_cigar.as<uint8_t>() + c0, b->cigar + c0, c1 - c0 }, { ctx->b_md.as<uint8_t>() + m0, b->md ? b->md + m0 : nullptr, m1 - m0 } };
     for (auto &c : cp) { if (c.bytes) CU(cudaMemcpyAsync(c.d, c.h, c.bytes, cudaMemcpyHostToDevice, st)); *bytes += c.bytes; }
     return 0;
 }
@@ -510,6 +526,7 @@ static int src_copy_range(cbcg_ctx *ctx, const BatchSrc &s, uint64_t r0, uint64_
 extern "C" int cbcg_batch_upload_compact(cbcg_ctx *ctx, const cbcg_batch_compact *b) {
     if (!ctx) return CBCG_ERR_ARG;
     TRY(check_compact(ctx, b));
+    if (b->n_reads && !b->md_len && !ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "a batch without MD needs the reference: cbcg_set_reference has not been called");
     CU(cudaSetDevice(ctx->device));
     const uint64_t n = b->n_reads;
     TRY(compact_buffers(ctx, b));
@@ -520,6 +537,10 @@ extern "C" int cbcg_batch_upload_compact(cbcg_ctx *ctx, const cbcg_batch_compact
         TRY(compact_copy_head(ctx, b, ctx->st, &h2d));
         TRY(compact_copy_range(ctx, b, 0, n, ctx->st, &h2d));
         TRY(compact_unpack_range(ctx, b, 0, n, ctx->st));
+        if (ctx->batch_no_md) {                             /* K7 walks what K0 laid out: only once K0 has found it consistent */
+            TRY(fetch_words(ctx)); TRY(device_error(ctx, "compact batch"));
+            TRY(derive_md(ctx, 0));
+        }
     }
     CU(cudaEventRecord(ctx->ev[1], ctx->st));
     if (n) { TRY(fetch_words(ctx)); TRY(device_error(ctx, "compact batch")); }
@@ -533,6 +554,7 @@ extern "C" int cbcg_batch_upload_compact(cbcg_ctx *ctx, const cbcg_batch_compact
 extern "C" int cbcg_batch_upload(cbcg_ctx *ctx, const cbcg_batch *b) {
     if (!ctx) return CBCG_ERR_ARG;
     TRY(check_batch(ctx, b));
+    if (b->n_reads && !b->md_off && !ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "a batch without MD needs the reference: cbcg_set_reference has not been called");
     CU(cudaSetDevice(ctx->device));
     const uint64_t n = b->n_reads;
     TRY(batch_prepare(ctx, b));
@@ -540,9 +562,11 @@ extern "C" int cbcg_batch_upload(cbcg_ctx *ctx, const cbcg_batch *b) {
     uint64_t h2d = 0;
     TRY(batch_copy_range(ctx, b, 0, n, ctx->st, &h2d));
     const int scan_rc = batch_scan(ctx, b);               /* while the copies fly */
+    const int md_rc = !scan_rc && n && ctx->batch_no_md ? derive_md(ctx, 0) : 0;   /* K7 on a checked batch; its time is part of ms_h2d */
     CU(cudaEventRecord(ctx->ev[1], ctx->st));
     CU(cudaStreamSynchronize(ctx->st));
     if (scan_rc) return scan_rc;                          /* nothing is left in flight that reads the caller's buffers */
+    if (md_rc) return md_rc;
     ctx->have_batch = true;
     float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]);
     ctx->stats.ms_h2d = ms; ctx->stats.h2d_bytes = h2d; ctx->stats.n_reads = n;
@@ -596,6 +620,54 @@ static int run_extract(cbcg_ctx *ctx) {
         return device_error(ctx, "edit extraction");
     }
     return fail(ctx, CBCG_ERR_INTERNAL, "edit extraction: capacity retry failed");
+}
+
+/* K7 over the whole resident batch, one that came without MD: its MD pool and md_off. need: the pool's exact size when it
+ * is known (the pipelined encode counted it), else 0. A pool too small for what K7 counts is grown to the exact size and
+ * the batch derived once more, as run_extract does for edit entries. */
+static int derive_md(cbcg_ctx *ctx, uint64_t need) {
+    const uint64_t n = ctx->db.n_reads;
+    TRY(ensure(ctx, ctx->tile_desc, (md_num_tiles(n) + 1) * 8));
+    if (need + POOL_PAD > ctx->b_md.cap) TRY(ensure(ctx, ctx->b_md, need + POOL_PAD));
+    for (int attempt = 0; attempt < 2; attempt++) {
+        ctx->db.md = ctx->b_md.as<uint8_t>();
+        TRY(reset_words(ctx));
+        if (launch_md(ctx->db, ctx->dg, ctx->b_moff.as<uint64_t>(), ctx->b_md.as<uint8_t>(), ctx->b_md.cap - POOL_PAD, ctx->tile_desc.as<uint64_t>(),
+                      wptr<uint32_t>(ctx, W_OFF(ticket)), wptr<uint64_t>(ctx, W_OFF(md_chain)), wptr<unsigned long long>(ctx, W_OFF(err)),
+                      ctx->st, 0, n, nullptr))
+            return fail(ctx, CBCG_ERR_CUDA, "K7 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        ctx->stats.kernel_launches++;
+        TRY(fetch_words(ctx));
+        const unsigned long long v = ctx->hw->err;
+        if (v && -(int)(v >> 40) == CBCG_ERR_CAPACITY && attempt == 0) {   /* MD pool too small: the count is exact */
+            TRY(ensure(ctx, ctx->b_md, ctx->hw->md_chain[0] + POOL_PAD));
+            continue;
+        }
+        return device_error(ctx, "MD derivation");
+    }
+    return fail(ctx, CBCG_ERR_INTERNAL, "MD derivation: capacity retry failed");
+}
+
+extern "C" int cbcg_derive_md(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!ctx || !batch || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_derive_md: bad argument");
+    *out_len = 0;
+    cbcg_batch b = *batch;
+    b.md_off = nullptr; b.md = nullptr;                   /* any MD the batch carries is ignored */
+    TRY(cbcg_batch_upload(ctx, &b));
+    const uint64_t n = ctx->db.n_reads;
+    if (!n) return CBCG_OK;
+    std::vector<uint64_t> off(n + 1);
+    CU(cudaMemcpyAsync(off.data(), ctx->b_moff.p, (n + 1) * 8, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    *out_len = off[n] + n;
+    if (!out || off[n] + n > out_cap) return fail(ctx, CBCG_ERR_CAPACITY, "derived MD is %llu bytes, room for %llu", (unsigned long long)(off[n] + n), (unsigned long long)out_cap);
+    if (off[n]) CU(cudaMemcpyAsync(out, ctx->b_md.p, off[n], cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    for (uint64_t r = n; r-- > 0;) {                      /* in place, from the back: read r moves r bytes up, then its '\n' */
+        memmove(out + off[r] + r, out + off[r], off[r + 1] - off[r]);
+        out[off[r + 1] + r] = '\n';
+    }
+    return CBCG_OK;
 }
 
 extern "C" int cbcg_extract(cbcg_ctx *ctx, const cbcg_batch *batch, cbcg_read_rec *recs,
@@ -1201,6 +1273,14 @@ static int encode_pipelined(cbcg_ctx *ctx, const BatchSrc &src, const cbcg_encod
     for (uint32_t c = 0; c <= PIPE_CHUNKS; c++) {
         CU(cudaStreamWaitEvent(ctx->st, ctx->cev[c], 0));
         if (src.compact) TRY(compact_unpack_range(ctx, src.compact, cut[c], cut[c + 1], ctx->st));   /* 2-bit SEQ, lengths, runs -> the SoA batch */
+        if (ctx->batch_no_md) {                              /* K7: the chunk's MD, continuing the previous chunk's */
+            uint64_t *mdc = wptr<uint64_t>(ctx, W_OFF(md_chain));
+            if (launch_md(ctx->db, ctx->dg, ctx->b_moff.as<uint64_t>(), ctx->b_md.as<uint8_t>(), ctx->b_md.cap - POOL_PAD,
+                          ctx->tile_desc.as<uint64_t>() + tile_off, wptr<uint32_t>(ctx, W_OFF(ticket)), &mdc[(c + 1u) & 1u],
+                          wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st, cut[c], cut[c + 1], c ? &mdc[c & 1u] : nullptr))
+                return fail(ctx, CBCG_ERR_CUDA, "K7 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+            S.kernel_launches++;
+        }
         /* K1 on the chunk; its edit entries continue the previous chunk's */
         if (launch_extract(ctx->db, ctx->dg, ctx->recs.as<cbcg_read_rec>(), ctx->edits.as<uint16_t>(), edits_cap,
                            ctx->tile_desc.as<uint64_t>() + tile_off, wptr<uint32_t>(ctx, W_OFF(ticket)), &chain[(c + 1u) & 1u],
@@ -1252,7 +1332,8 @@ static int encode_pipelined(cbcg_ctx *ctx, const BatchSrc &src, const cbcg_encod
     if (launch_copy16(ctx->hblocks, ctx->blocks.p, nb * sizeof(BlockDesc), ctx->st) ||
         launch_copy_words(&ctx->hw->total_bytes, ctx->out_off.as<uint64_t>() + nb, 1, ctx->st) ||
         launch_copy_words(&ctx->hw->total_edits, &chain[(PIPE_CHUNKS + 1u) & 1u], 1, ctx->st) ||
-        launch_copy_words(&ctx->hw->err, wptr<unsigned long long>(ctx, W_OFF(err)), 1, ctx->st))
+        launch_copy_words(&ctx->hw->err, wptr<unsigned long long>(ctx, W_OFF(err)), 1, ctx->st) ||
+        (ctx->batch_no_md && launch_copy_words(&ctx->hw->md_chain[0], wptr<uint64_t>(ctx, W_OFF(md_chain)) + ((PIPE_CHUNKS + 1u) & 1u), 1, ctx->st)))
         return fail(ctx, CBCG_ERR_CUDA, "result copy launch failed");
     CU(cudaStreamSynchronize(ctx->st));
     ctx->have_batch = true;
@@ -1289,6 +1370,8 @@ static int encode_from(cbcg_ctx *ctx, const BatchSrc &src, const cbcg_encode_opt
         if (rc < 0) { pipe_drain(ctx); return rc; }          /* copies from the caller's batch may still be queued */
         if (rc == CBCG_OK) return cbcg_fetch_container(ctx, out, out_cap, out_len);
         if (ctx->have_batch) {                              /* fallback with the batch already resident */
+            /* without MD: a pool that overflowed holds empty MD for the reads past its end; derive it whole at the size counted */
+            if (ctx->batch_no_md) TRY(derive_md(ctx, ctx->hw->md_chain[0]));
             TRY(cbcg_encode_resident(ctx, opts));
             return cbcg_fetch_container(ctx, out, out_cap, out_len);
         }

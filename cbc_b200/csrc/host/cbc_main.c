@@ -8,6 +8,10 @@
  *          -l       variable-length reads: header read length = longest SEQ (src/main.c -l)
  *          -g LIST  CUDA devices, e.g. `-g 0,1,2,3`: batches (region shards of the sorted input) are dealt out to them
  *          -B MB    SAM text per batch (default 2048): memory is bounded by three batches whatever the file size
+ *          -M       -c only: the input's MD:Z tags are not read (records need none); every read's MD is derived on the GPU from its
+ *                   CIGAR, SEQ and the reference (cbcg.h, "a batch without MD"), so an aligner's output without --MD codes as it
+ *                   would after `samtools calmd`. The container is the one the derived MD gives, and nothing in it records -M.
+ *                   A read whose CIGAR's query length is not its SEQ length is refused. Without -M a record without MD:Z is an error.
  *          -C       CIGAR recovery (SURVEY.md 8f row 4; cbcg_cigar_pack / cbcg_cigar_unpack): -c also writes <out>.cig, the side
  *                   sections of the batches (u64 length + section each); -d reads <in>.cig and writes "CIGAR<TAB>SEQ" lines
  *          -r NAME[:START[-END]]   -d only, repeatable: write only the reads that overlap one of the regions (1-based, inclusive;
@@ -47,7 +51,7 @@ static uint32_t rd_u32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return 
 static double now(void) { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t); return (double)t.tv_sec + 1e-9 * (double)t.tv_nsec; }
 
 static int usage(void) {
-    fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
+    fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-M] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
                     "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n");
@@ -78,7 +82,7 @@ typedef struct shared {
     uint64_t next_take;                         /* next job a device thread takes */
     int producer_failed;
     /* run parameters */
-    int mode, single, var_length, with_cigar, sam; uint32_t block_reads;
+    int mode, single, var_length, with_cigar, sam, derive_md; uint32_t block_reads;
     const cbch_fasta *fa; int fa_ready;
     const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
     double t_gpu_ready;
@@ -232,7 +236,8 @@ static void *ingest_main(void *arg) {
         pthread_mutex_unlock(&S->mu);
         job *J = S->jobs[k];
         const double t0 = now();
-        int rc = cbch_ingest_range(A->cut[k], A->cut[k + 1], S->fa, S->var_length, cbch_default_threads(), header_len, &J->hb, A->err, sizeof A->err);
+        int rc = cbch_ingest_range_ex(A->cut[k], A->cut[k + 1], S->fa, S->var_length, cbch_default_threads(), header_len,
+                                      S->derive_md ? CBCH_DERIVE_MD : 0u, &J->hb, A->err, sizeof A->err);
         if (!rc) {
             cbcg_batch v; cbch_batch_view(&J->hb, &v);
             cbcg_encode_opts o = { J->hb.read_len_header ? J->hb.read_len_header : 1u, S->single ? 0u : S->block_reads, S->single ? 0u : 1u, 0u };
@@ -329,7 +334,7 @@ static int parse_devices(const char *s, int *dev) {
 }
 
 int main(int argc, char **argv) {
-    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
+    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, derive_md = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
     uint32_t block_reads = CBCG_BLOCK_AUTO;
     uint64_t batch_mb = 2048;
     const char *files[4]; int nfiles = 0;
@@ -342,6 +347,7 @@ int main(int argc, char **argv) {
         else if (!strcmp(a, "-l")) var_length = 1;
         else if (!strcmp(a, "-C")) with_cigar = 1;
         else if (!strcmp(a, "-S")) sam = 1;
+        else if (!strcmp(a, "-M")) derive_md = 1;
         else if (!strcmp(a, "-b") && i + 1 < argc) block_reads = (uint32_t)strtoul(argv[++i], NULL, 10);
         else if (!strcmp(a, "-B") && i + 1 < argc) batch_mb = strtoull(argv[++i], NULL, 10);
         else if (!strcmp(a, "-r") && i + 1 < argc) {
@@ -365,6 +371,7 @@ int main(int argc, char **argv) {
     if (!mode || nfiles != 3) { fprintf(stderr, "Missing required filenames\n"); return usage(); }
     if (n_regions && mode != 'd') { fprintf(stderr, "cbc: -r selects reads to decode: it goes with -d\n"); return usage(); }
     if (sam && mode != 'd') { fprintf(stderr, "cbc: -S writes SAM: it goes with -d\n"); return usage(); }
+    if (derive_md && mode != 'c') { fprintf(stderr, "cbc: -M derives MD for encoding: it goes with -c\n"); return usage(); }
     if (n_regions && with_cigar && !sam) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
     if (!single && block_reads == 0) block_reads = CBCG_BLOCK_AUTO;
     if (batch_mb < 1) batch_mb = 1;
@@ -373,7 +380,7 @@ int main(int argc, char **argv) {
     shared S; memset(&S, 0, sizeof S);
     pthread_mutex_init(&S.mu, NULL); pthread_cond_init(&S.cv, NULL);
     S.mode = mode; S.single = single; S.var_length = var_length; S.block_reads = block_reads; S.with_cigar = with_cigar;
-    S.regions = regions; S.n_regions = n_regions; S.sam = sam;
+    S.regions = regions; S.n_regions = n_regions; S.sam = sam; S.derive_md = derive_md;
     devthread D[MAX_DEV]; memset(D, 0, sizeof D);
 
     /* ---- the input, cut into jobs (before the device threads start: they index S.jobs) */

@@ -108,12 +108,13 @@ static int grow(void **p, uint64_t *cap, uint64_t need, size_t elem) {
     *p = q; *cap = c;
     return 0;
 }
-static int reserve_reads(cbch_batch *b, uint64_t n) {
+static int reserve_reads(cbch_batch *b, uint64_t n, int with_md) {
     if (n <= b->cap) return 0;
     uint64_t c = b->cap ? b->cap : 4096;
     while (c < n) c += c / 2;
 #define RS(field, extra) do { void *q = realloc(b->field, (size_t)((c + extra) * sizeof *b->field)); if (!q) return -1; b->field = q; } while (0)
-    RS(pos, 0); RS(flag, 0); RS(seq_len, 0); RS(chr, 0); RS(seq_off, 1); RS(cigar_off, 1); RS(md_off, 1);
+    RS(pos, 0); RS(flag, 0); RS(seq_len, 0); RS(chr, 0); RS(seq_off, 1); RS(cigar_off, 1);
+    if (with_md) RS(md_off, 1);
 #undef RS
     b->cap = c;
     return 0;
@@ -132,6 +133,7 @@ static int parse_u32(const uint8_t *s, const uint8_t *e, uint32_t *v) {
 typedef struct {
     const uint8_t *begin, *end;
     const cbch_fasta *fa;
+    uint32_t flags;                      /* CBCH_DERIVE_MD: MD tags are not looked for, the part has no MD arrays */
     cbch_batch part;
     uint64_t records; uint32_t len1, len2;
     int rc; uint64_t err_line; char err[200];
@@ -154,8 +156,9 @@ static void parse_range(ingest_part *w) {
     /* sized from the range once (a record is at least 22 bytes of text, its SEQ / CIGAR / MD are substrings of it): no
        reallocation while parsing; untouched pages cost nothing */
     const uint64_t range = (uint64_t)(end - p);
-    if (reserve_reads(b, range / 22u + 16u) || grow((void **)&b->seq, &b->seq_cap, range + 64, 1) ||
-        grow((void **)&b->cigar, &b->cigar_cap, range / 2u + 64, 1) || grow((void **)&b->md, &b->md_cap, range / 2u + 64, 1)) rc = part_fail(w, CBCH_ERR_NOMEM, "out of memory");
+    const int with_md = !(w->flags & CBCH_DERIVE_MD);
+    if (reserve_reads(b, range / 22u + 16u, with_md) || grow((void **)&b->seq, &b->seq_cap, range + 64, 1) ||
+        grow((void **)&b->cigar, &b->cigar_cap, range / 2u + 64, 1) || (with_md && grow((void **)&b->md, &b->md_cap, range / 2u + 64, 1))) rc = part_fail(w, CBCH_ERR_NOMEM, "out of memory");
     uint64_t so = 0, co = 0, mo = 0;
     while (!rc && p < end) {
         const uint8_t *nl = memchr(p, '\n', (size_t)(end - p));
@@ -194,26 +197,26 @@ static void parse_range(ingest_part *w) {
             if (c == fa->n) { rc = part_fail(w, CBCH_ERR_RNAME, "RNAME %.*s is not in the reference", (int)rl, rn); break; }
             chr = c; last_chr = c; last_name = rn; last_name_len = rl;
         }
-        /* MD:Z among the optional fields */
+        /* MD:Z among the optional fields (CBCH_DERIVE_MD: not looked for) */
         const uint8_t *md = NULL; size_t mdl = 0;
-        for (const uint8_t *o = f[11]; o < le;) {
+        for (const uint8_t *o = f[11]; with_md && o < le;) {
             const uint8_t *t = memchr(o, '\t', (size_t)(le - o));
             const uint8_t *oe = t ? t : le;
             if (oe - o >= 5 && o[0] == 'M' && o[1] == 'D' && o[2] == ':' && o[3] == 'Z' && o[4] == ':') { md = o + 5; mdl = (size_t)(oe - md); break; }
             o = oe + 1;
         }
-        if (!md) { rc = part_fail(w, CBCH_ERR_NO_MD, "no MD:Z tag (README.md:25-29 requires it)"); break; }
+        if (with_md && !md) { rc = part_fail(w, CBCH_ERR_NO_MD, "no MD:Z tag (README.md:25-29 requires it; -M derives it on the GPU)"); break; }
         const size_t cgl = (size_t)(FEND(5) - f[5]);
-        if (reserve_reads(b, b->n_reads + 1) || grow((void **)&b->seq, &b->seq_cap, so + seqlen + 64, 1) ||
-            grow((void **)&b->cigar, &b->cigar_cap, co + cgl + 64, 1) || grow((void **)&b->md, &b->md_cap, mo + mdl + 64, 1)) { rc = part_fail(w, CBCH_ERR_NOMEM, "out of memory"); break; }
+        if (reserve_reads(b, b->n_reads + 1, with_md) || grow((void **)&b->seq, &b->seq_cap, so + seqlen + 64, 1) ||
+            grow((void **)&b->cigar, &b->cigar_cap, co + cgl + 64, 1) || (with_md && grow((void **)&b->md, &b->md_cap, mo + mdl + 64, 1))) { rc = part_fail(w, CBCH_ERR_NOMEM, "out of memory"); break; }
         const uint64_t r = b->n_reads++;
         b->pos[r] = pos; b->flag[r] = (uint16_t)flag; b->seq_len[r] = (uint16_t)seqlen; b->chr[r] = chr;
         b->seq_off[r] = so; memcpy(b->seq + so, f[9], seqlen); so += seqlen;
         b->cigar_off[r] = co; memcpy(b->cigar + co, f[5], cgl); co += cgl;
-        b->md_off[r] = mo; memcpy(b->md + mo, md, mdl); mo += mdl;
+        if (with_md) { b->md_off[r] = mo; memcpy(b->md + mo, md, mdl); mo += mdl; }
         if (seqlen > b->max_len) b->max_len = seqlen;
     }
-    if (!rc) { b->seq_off[b->n_reads] = so; b->cigar_off[b->n_reads] = co; b->md_off[b->n_reads] = mo; }
+    if (!rc) { b->seq_off[b->n_reads] = so; b->cigar_off[b->n_reads] = co; if (with_md) b->md_off[b->n_reads] = mo; }
 }
 
 /* second phase of the threaded ingest: every worker copies its part to its place in the merged batch */
@@ -224,8 +227,12 @@ static void merge_part(merge_job *j) {
     if (!n) return;
     memcpy(d->pos + j->r0, s->pos, n * sizeof *d->pos); memcpy(d->flag + j->r0, s->flag, n * sizeof *d->flag);
     memcpy(d->seq_len + j->r0, s->seq_len, n * sizeof *d->seq_len); memcpy(d->chr + j->r0, s->chr, n * sizeof *d->chr);
-    for (uint64_t r = 0; r < n; r++) { d->seq_off[j->r0 + r] = s->seq_off[r] + j->s0; d->cigar_off[j->r0 + r] = s->cigar_off[r] + j->c0; d->md_off[j->r0 + r] = s->md_off[r] + j->m0; }
-    memcpy(d->seq + j->s0, s->seq, s->seq_off[n]); memcpy(d->cigar + j->c0, s->cigar, s->cigar_off[n]); memcpy(d->md + j->m0, s->md, s->md_off[n]);
+    for (uint64_t r = 0; r < n; r++) { d->seq_off[j->r0 + r] = s->seq_off[r] + j->s0; d->cigar_off[j->r0 + r] = s->cigar_off[r] + j->c0; }
+    memcpy(d->seq + j->s0, s->seq, s->seq_off[n]); memcpy(d->cigar + j->c0, s->cigar, s->cigar_off[n]);
+    if (d->md_off) {                                              /* NULL: a batch without MD (CBCH_DERIVE_MD) */
+        for (uint64_t r = 0; r < n; r++) d->md_off[j->r0 + r] = s->md_off[r] + j->m0;
+        memcpy(d->md + j->m0, s->md, s->md_off[n]);
+    }
     cbch_free_batch(&j->w->part);                                 /* every worker returns its own part (unmapping them one after the other on the caller's thread was a sixth of the ingest) */
 }
 static double now_s(void) { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t); return (double)t.tv_sec + (double)t.tv_nsec * 1e-9; }
@@ -241,7 +248,7 @@ int cbch_default_threads(void) {
 }
 
 int cbch_read_sam(const char *path, const cbch_fasta *fa, int var_length, cbch_batch *b, char *err, size_t errlen) {
-    return cbch_read_sam_mt(path, fa, var_length, cbch_default_threads(), b, err, errlen);
+    return cbch_read_sam_ex(path, fa, var_length, cbch_default_threads(), 0u, b, err, errlen);
 }
 
 /* The file is cut at line starts into n_threads ranges of about equal bytes; every worker parses its range into its own
@@ -268,10 +275,13 @@ const uint8_t *cbch_next_line(const uint8_t *p, const uint8_t *end) {
 }
 
 int cbch_read_sam_mt(const char *path, const cbch_fasta *fa, int var_length, int n_threads, cbch_batch *b, char *err, size_t errlen) {
+    return cbch_read_sam_ex(path, fa, var_length, n_threads, 0u, b, err, errlen);
+}
+int cbch_read_sam_ex(const char *path, const cbch_fasta *fa, int var_length, int n_threads, uint32_t flags, cbch_batch *b, char *err, size_t errlen) {
     memset(b, 0, sizeof *b);
     mapped m;
     if (map_file(path, &m)) return fail(err, errlen, CBCH_ERR_IO, "cannot open %s", path);
-    const int rc = cbch_ingest_range(m.p, m.p + m.n, fa, var_length, n_threads, 0, b, err, errlen);
+    const int rc = cbch_ingest_range_ex(m.p, m.p + m.n, fa, var_length, n_threads, 0, flags, b, err, errlen);
     unmap_file(&m);
     return rc;
 }
@@ -280,7 +290,12 @@ int cbch_read_sam_mt(const char *path, const cbch_fasta *fa, int var_length, int
  * (a later batch of a file takes the first batch's: get_read_length looks at the file's second record). */
 int cbch_ingest_range(const uint8_t *begin, const uint8_t *range_end, const cbch_fasta *fa, int var_length, int n_threads, uint32_t header_len,
                       cbch_batch *b, char *err, size_t errlen) {
+    return cbch_ingest_range_ex(begin, range_end, fa, var_length, n_threads, header_len, 0u, b, err, errlen);
+}
+int cbch_ingest_range_ex(const uint8_t *begin, const uint8_t *range_end, const cbch_fasta *fa, int var_length, int n_threads, uint32_t header_len,
+                         uint32_t flags, cbch_batch *b, char *err, size_t errlen) {
     memset(b, 0, sizeof *b);
+    const int with_md = !(flags & CBCH_DERIVE_MD);
     const char *path = "the SAM input";
     struct { const uint8_t *p; size_t n; } m = { begin, (size_t)(range_end - begin) };
     if (n_threads < 1) n_threads = 1;
@@ -299,7 +314,7 @@ int cbch_ingest_range(const uint8_t *begin, const uint8_t *range_end, const cbch
             const uint8_t *nl = guess < end ? memchr(guess, '\n', (size_t)(end - guess)) : NULL;
             stop = nl ? nl + 1 : end;
         }
-        w[t].begin = cur; w[t].end = stop; w[t].fa = fa;
+        w[t].begin = cur; w[t].end = stop; w[t].fa = fa; w[t].flags = flags;
         cur = stop;
     }
     const int trace = getenv("CBCH_TRACE") != NULL;
@@ -325,12 +340,12 @@ int cbch_ingest_range(const uint8_t *begin, const uint8_t *range_end, const cbch
         records += w[t].records;
         jobs[t].w = &w[t]; jobs[t].dst = b; jobs[t].r0 = n; jobs[t].s0 = so; jobs[t].c0 = co; jobs[t].m0 = mo;
         n += w[t].part.n_reads; lines += w[t].part.n_lines; b->n_unmapped += w[t].part.n_unmapped;
-        if (w[t].part.n_reads) { so += w[t].part.seq_off[w[t].part.n_reads]; co += w[t].part.cigar_off[w[t].part.n_reads]; mo += w[t].part.md_off[w[t].part.n_reads]; }
+        if (w[t].part.n_reads) { so += w[t].part.seq_off[w[t].part.n_reads]; co += w[t].part.cigar_off[w[t].part.n_reads]; if (with_md) mo += w[t].part.md_off[w[t].part.n_reads]; }
         if (w[t].part.max_len > b->max_len) b->max_len = w[t].part.max_len;
     }
     if (!rc) {
-        if (reserve_reads(b, n + 1) || grow((void **)&b->seq, &b->seq_cap, so + 64, 1) || grow((void **)&b->cigar, &b->cigar_cap, co + 64, 1) ||
-            grow((void **)&b->md, &b->md_cap, mo + 64, 1)) rc = fail(err, errlen, CBCH_ERR_NOMEM, "out of memory reading %s", path);
+        if (reserve_reads(b, n + 1, with_md) || grow((void **)&b->seq, &b->seq_cap, so + 64, 1) || grow((void **)&b->cigar, &b->cigar_cap, co + 64, 1) ||
+            (with_md && grow((void **)&b->md, &b->md_cap, mo + 64, 1))) rc = fail(err, errlen, CBCH_ERR_NOMEM, "out of memory reading %s", path);
     }
     if (!rc) {
         b->n_reads = n; b->n_lines = lines;
@@ -339,7 +354,7 @@ int cbch_ingest_range(const uint8_t *begin, const uint8_t *range_end, const cbch
         for (int t = started + 1; t < n_threads; t++) merge_part(&jobs[t]);
         merge_part(&jobs[0]);
         for (int t = 1; t <= started; t++) pthread_join(th[t], NULL);
-        b->seq_off[n] = so; b->cigar_off[n] = co; b->md_off[n] = mo;
+        b->seq_off[n] = so; b->cigar_off[n] = co; if (with_md) b->md_off[n] = mo;
         /* get_read_length (:47-53): fixed-length mode takes the SECOND record's SEQ length; -l takes the maximum */
         b->read_len_header = var_length ? b->max_len : header_len ? header_len : (records >= 2 ? lens[1] : lens[0]);
     }
@@ -394,10 +409,10 @@ static inline int pack8(const uint8_t *s, uint8_t *d2) {
 static void pack_part(pack_job *j) {
     const cbcg_batch *b = j->b;
     if (j->r1 > j->r0) {
-        const uint64_t m = j->r1 - j->r0, c0 = b->cigar_off[0], m0 = b->md_off[0];
+        const uint64_t m = j->r1 - j->r0, c0 = b->cigar_off[0];
         memcpy(j->pos + j->r0, b->pos + j->r0, m * 4); memcpy(j->flag + j->r0, b->flag + j->r0, m * 2); memcpy(j->sl + j->r0, b->seq_len + j->r0, m * 2);
         memcpy(j->cig + (b->cigar_off[j->r0] - c0), b->cigar + b->cigar_off[j->r0], b->cigar_off[j->r1] - b->cigar_off[j->r0]);
-        memcpy(j->md + (b->md_off[j->r0] - m0), b->md + b->md_off[j->r0], b->md_off[j->r1] - b->md_off[j->r0]);
+        if (b->md_off) memcpy(j->md + (b->md_off[j->r0] - b->md_off[0]), b->md + b->md_off[j->r0], b->md_off[j->r1] - b->md_off[j->r0]);
     }
     for (uint64_t r = j->r0; r < j->r1; r++) {
         const uint8_t *s = b->seq + b->seq_off[r];
@@ -423,7 +438,7 @@ static void pack_part(pack_job *j) {
             d[i >> 2] = (uint8_t)byte;
         }
         j->cl[r] = (uint16_t)(b->cigar_off[r + 1] - b->cigar_off[r]);
-        j->ml[r] = (uint16_t)(b->md_off[r + 1] - b->md_off[r]);
+        if (b->md_off) j->ml[r] = (uint16_t)(b->md_off[r + 1] - b->md_off[r]);
     }
 }
 static void *pack_thread(void *arg) { pack_part((pack_job *)arg); return NULL; }
@@ -463,20 +478,21 @@ int cbch_pack_batch(const cbcg_batch *b, int n_threads, void *(*alloc)(size_t), 
         if (r == 0 || b->chr[r] != b->chr[r - 1]) n_runs++;
     }
     so[n] = o;
-    const uint64_t s0 = b->seq_off[0], c0 = b->cigar_off[0], m0 = b->md_off[0], co_n = b->cigar_off[n] - c0, mo_n = b->md_off[n] - m0;
+    const int with_md = b->md_off != NULL;                    /* without MD: md_len = md = NULL and a zero MD column */
+    const uint64_t s0 = b->seq_off[0], c0 = b->cigar_off[0], m0 = with_md ? b->md_off[0] : 0, co_n = b->cigar_off[n] - c0, mo_n = with_md ? b->md_off[n] - m0 : 0;
     {   /* one entry per tile of 128 reads, and the totals */
         const uint64_t tiles = (n + 127u) / 128u;
         uint64_t *tb = alloc((tiles + 1) * 32);
         v->tile_base = tb;
         if (!tb) { free(so); return CBCH_ERR_NOMEM; }
-        for (uint64_t t = 0; t <= tiles; t++) { const uint64_t r = t * 128u < n ? t * 128u : n; tb[4 * t] = b->seq_off[r] - s0; tb[4 * t + 1] = so[r]; tb[4 * t + 2] = b->cigar_off[r] - c0; tb[4 * t + 3] = b->md_off[r] - m0; }
+        for (uint64_t t = 0; t <= tiles; t++) { const uint64_t r = t * 128u < n ? t * 128u : n; tb[4 * t] = b->seq_off[r] - s0; tb[4 * t + 1] = so[r]; tb[4 * t + 2] = b->cigar_off[r] - c0; tb[4 * t + 3] = with_md ? b->md_off[r] - m0 : 0; }
         v->max_len = mx; v->min_len = mn;
     }
-    uint32_t *pos = alloc(n * 4); uint16_t *flag = alloc(n * 2), *sl = alloc(n * 2), *cl = alloc(n * 2), *ml = alloc(n * 2);
+    uint32_t *pos = alloc(n * 4); uint16_t *flag = alloc(n * 2), *sl = alloc(n * 2), *cl = alloc(n * 2), *ml = with_md ? alloc(n * 2) : NULL;
     uint64_t *rf = alloc(n_runs * 8); uint32_t *rc = alloc(n_runs * 4);
-    uint8_t *seq2 = alloc(o + 64), *cig = alloc(co_n + 64), *md = alloc(mo_n + 64);
+    uint8_t *seq2 = alloc(o + 64), *cig = alloc(co_n + 64), *md = with_md ? alloc(mo_n + 64) : NULL;
     v->pos = pos; v->flag = flag; v->seq_len = sl; v->cigar_len = cl; v->md_len = ml; v->run_first = rf; v->run_chr = rc; v->seq2 = seq2; v->cigar = cig; v->md = md;
-    if (!pos || !flag || !sl || !cl || !ml || !rf || !rc || !seq2 || !cig || !md) { free(so); cbch_free_compact(out); return CBCH_ERR_NOMEM; }
+    if (!pos || !flag || !sl || !cl || (with_md && (!ml || !md)) || !rf || !rc || !seq2 || !cig) { free(so); cbch_free_compact(out); return CBCH_ERR_NOMEM; }
     { uint64_t k = 0; for (uint64_t r = 0; r < n; r++) if (r == 0 || b->chr[r] != b->chr[r - 1]) { rf[k] = r; rc[k] = b->chr[r]; k++; } v->n_runs = (uint32_t)n_runs; }
     const double t_head = now_s();
     pack_job *jobs = calloc((size_t)n_threads, sizeof *jobs);
@@ -504,7 +520,7 @@ int cbch_pack_batch(const cbcg_batch *b, int n_threads, void *(*alloc)(size_t), 
     v->n_exc = oom ? 0 : n_exc;
     for (int t = 0; t < n_threads; t++) { free(jobs[t].er); free(jobs[t].eb); free(jobs[t].ec); }
     free(jobs); free(th);
-    out->bytes = n * (4 + 2 + 2 + 2 + 2) + o + co_n + mo_n + n_runs * 12 + n_exc * 7 + ((n + 127u) / 128u + 1) * 32;
+    out->bytes = n * (4 + 2 + 2 + 2 + (with_md ? 2 : 0)) + o + co_n + mo_n + n_runs * 12 + n_exc * 7 + ((n + 127u) / 128u + 1) * 32;
     free(so);
     if (oom) { cbch_free_compact(out); return CBCH_ERR_NOMEM; }
     return CBCH_OK;

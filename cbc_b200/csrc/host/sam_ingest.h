@@ -34,6 +34,9 @@ typedef struct cbch_batch {
 } cbch_batch;
 
 enum { CBCH_OK = 0, CBCH_ERR_IO = -1, CBCH_ERR_NOMEM = -2, CBCH_ERR_PARSE = -3, CBCH_ERR_RNAME = -4, CBCH_ERR_NO_MD = -5 };
+/* Ingest flags. CBCH_DERIVE_MD: MD:Z tags are not looked for (a record without one is accepted, one that has one is read as
+ * if it had none); the batch's md_off and md stay NULL, a batch without MD that the library derives MD for (cbcg.h). */
+#define CBCH_DERIVE_MD 1u
 
 int  cbch_read_fasta(const char *path, cbch_fasta *out, char *err, size_t errlen);
 void cbch_free_fasta(cbch_fasta *fa);
@@ -42,6 +45,8 @@ int  cbch_read_sam(const char *path, const cbch_fasta *fa, int var_length, cbch_
 /* The same with an explicit worker count (cbch_read_sam uses CBCH_THREADS or the online cores, at most 64): the file is
  * cut at line starts, the ranges are parsed in parallel and merged; the result does not depend on the count. */
 int  cbch_read_sam_mt(const char *path, const cbch_fasta *fa, int var_length, int n_threads, cbch_batch *out, char *err, size_t errlen);
+/* The same with ingest flags (CBCH_DERIVE_MD); cbch_read_sam and cbch_read_sam_mt are this with flags 0. */
+int  cbch_read_sam_ex(const char *path, const cbch_fasta *fa, int var_length, int n_threads, uint32_t flags, cbch_batch *out, char *err, size_t errlen);
 int  cbch_default_threads(void);
 /* Streaming: the file mapped once (populate: fault it all in now, for files that fit in memory), cut at line starts with
  * cbch_next_line, ingested range by range. header_len != 0 overrides the fixed-length header value (later batches of a
@@ -52,10 +57,14 @@ void cbch_unmap(cbch_mapped *m);
 const uint8_t *cbch_next_line(const uint8_t *p, const uint8_t *end);
 int  cbch_ingest_range(const uint8_t *begin, const uint8_t *end, const cbch_fasta *fa, int var_length, int n_threads, uint32_t header_len,
                        cbch_batch *out, char *err, size_t errlen);
+/* The same with ingest flags (CBCH_DERIVE_MD); cbch_ingest_range is this with flags 0. */
+int  cbch_ingest_range_ex(const uint8_t *begin, const uint8_t *end, const cbch_fasta *fa, int var_length, int n_threads, uint32_t header_len,
+                          uint32_t flags, cbch_batch *out, char *err, size_t errlen);
 void cbch_free_batch(cbch_batch *b);
 void cbch_batch_view(const cbch_batch *b, cbcg_batch *view);
 
-/* The compact form of a batch (cbcg_batch_compact, include/cbcg.h): what crosses the host-device link. All arrays are
+/* The compact form of a batch (cbcg_batch_compact, include/cbcg.h): what crosses the host-device link (a batch without MD:
+ * md_len = md = NULL and a zero MD column in tile_base). All arrays are
  * allocated with `alloc` (NULL: malloc; pass cbcg_host_alloc for page-locked memory) and released with cbch_free_compact
  * through `release`. n_threads <= 0: the default worker count. */
 typedef struct cbch_compact {

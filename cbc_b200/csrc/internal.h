@@ -163,3 +163,11 @@ int launch_sam(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr,
                const uint64_t *ids, const uint8_t *cls, const uint64_t *exc_read, const uint64_t *exc_off, const uint8_t *exc_text,
                uint64_t n_exc, uint8_t *out, uint64_t out_cap, uint64_t *tile_desc, uint32_t *ticket, uint64_t *total_bytes,
                unsigned long long *err, cudaStream_t st);
+/* k7_md.cu: the MD of reads [r_begin, r_end) of a batch that carries none, into md / md_off (md_cap bytes of pool; a read
+   whose MD does not fit gets an empty one at md_cap and CBCG_ERR_CAPACITY). md_base (optional): MD bytes of the reads
+   before r_begin. *total_md receives md_base + the range's MD bytes, exact even when they do not fit. tile_desc:
+   md_num_tiles(r_end - r_begin) words. */
+uint64_t md_num_tiles(uint64_t n_reads);
+int launch_md(const DevBatch &b, const DevGenome &g, uint64_t *md_off, uint8_t *md, uint64_t md_cap, uint64_t *tile_desc,
+              uint32_t *ticket, uint64_t *total_md, unsigned long long *err, cudaStream_t st, uint64_t r_begin, uint64_t r_end,
+              const uint64_t *md_base);

@@ -57,8 +57,19 @@ typedef struct cbcg_batch {
     const uint32_t *chr;        /* chromosome ordinal into the table given to cbcg_set_reference */
     const uint64_t *seq_off;    const uint8_t *seq;     /* SEQ */
     const uint64_t *cigar_off;  const uint8_t *cigar;   /* CIGAR text */
-    const uint64_t *md_off;     const uint8_t *md;      /* MD:Z payload (read_line_t.edits) */
+    const uint64_t *md_off;     const uint8_t *md;      /* MD:Z payload (read_line_t.edits); both NULL: no MD, see below */
 } cbcg_batch;
+
+/* A batch without MD (cbcg_batch: md_off == md == NULL; cbcg_batch_compact: md_len == md == NULL, and then the MD column of
+ * tile_base must be all zero, else CBCG_ERR_INPUT; one of a pair NULL is CBCG_ERR_ARG). Each read's MD is derived on the
+ * device (K7, DESIGN.md 5d) while the batch is made resident -- by cbcg_batch_upload, cbcg_batch_upload_compact, and chunk
+ * by chunk in a pipelined cbcg_encode / cbcg_encode_compact -- from its CIGAR, its SEQ and the loaded reference, by the
+ * rule of the SAM output below (the MD cbcg_decode_sam prints). Every call that takes a batch then runs as on the same batch
+ * carrying that MD, byte for byte: containers, extraction, symbol lists, CIGAR sections. The container does not record it.
+ *   needs the reference: without cbcg_set_reference the upload is CBCG_ERR_NO_REFERENCE.
+ *   refused (CBCG_ERR_INPUT): what the batch with that MD would refuse, and also a read whose CIGAR's query length
+ *     (M + I + S + = + X) is not its SEQ length (with MD such a read is coded as before).
+ *   statistics: K7's time is part of ms_h2d. */
 
 /* The same batch in the form that crosses the host-device link (about 60 bytes per 150-base read instead of 196): SEQ at
  * 2 bits per base, every read starting on a byte (ceil(len / 4) bytes; base i in bits 2 (i & 3) of byte i >> 2;
@@ -263,6 +274,12 @@ int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legac
                     const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
                     uint8_t *out, uint64_t out_cap, uint64_t *out_len,
                     uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
+
+/* Each read's MD as the batch without MD would get it: MD + '\n' per read, in read order (samtools calmd on the device,
+ * under the rule above: N against N is not a mismatch). Any MD the batch carries is ignored. out_cap too small ->
+ * CBCG_ERR_CAPACITY with *out_len the size needed. State: the batch is uploaded (it becomes the resident batch, with the
+ * derived MD), as cbcg_batch_upload. */
+int cbcg_derive_md(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 
 /* ---- device-resident variants (inputs already in HBM when the timed region starts): upload once,
  * run many times. Results stay on the device until fetched. Used by bench.py for `value`. */
