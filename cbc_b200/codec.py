@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Optional, Tuple
+from typing import List, Optional, Tuple
 
 import numpy as np
 
@@ -42,10 +42,13 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_reconstruct", "cbcg_batch_upload", "cbcg_encode_resident", "cbcg_decode_resident",
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
            "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
-           "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam", "cbcg_derive_md"]
+           "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam", "cbcg_derive_md",
+           "cbcg_pileup"]
 
 
 UINT64_MAX = (1 << 64) - 1
+PILEUP_COLUMNS = ("A", "C", "G", "T", "N", "DEL", "INS", "REF")      # CBCG_PU_A .. CBCG_PU_REF
+PILEUP_FLAG_EXCLUDE = 0x704                                          # UNMAP | SECONDARY | QCFAIL | DUP
 
 
 class Region(C.Structure):
@@ -164,6 +167,7 @@ def load_library():
         lib.cbcg_sam_header.argtypes = [vp, u64, vp, u64, P(u64)]
         lib.cbcg_decode_sam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_derive_md.argtypes = [vp, P(CBatch), vp, u64, P(u64)]
+        lib.cbcg_pileup.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -261,6 +265,7 @@ class Codec:
             raise CbcgError(rc, self.lib.cbcg_strerror(rc).decode())
         self.h = h
         self._genome_keep = None
+        self.last_pileup_reads = 0                   # reads the last ``pileup`` counted
 
     def close(self):
         if getattr(self, "h", None):
@@ -412,6 +417,28 @@ class Codec:
                 continue
             self._check(rc)
             return out[:n.value].tobytes(), ids[:nr.value].copy()
+
+    def pileup(self, data: bytes, regions, cigar_section: Optional[bytes] = None, flag_exclude: int = PILEUP_FLAG_EXCLUDE,
+               legacy: bool = False) -> List[np.ndarray]:
+        """Per-position counts over regions (include/cbcg.h, cbcg_pileup): one [rows, 8] uint32 array per region, in the
+        order given, columns A C G T N DEL INS REF (PILEUP_COLUMNS), one row per position start .. min(end, LN). The reads
+        are ``decompress_sam``'s for the same regions without those whose FLAG & flag_exclude; cigar_section: as there.
+        The arrays are views into one buffer, sized by the library's capacity answer before anything is decoded."""
+        src = np.frombuffer(data, np.uint8)
+        sec = np.frombuffer(cigar_section, np.uint8) if cigar_section is not None else None
+        arr, n_regions = _region_array(regions)                              # an empty list is CBCG_ERR_ARG
+        per = np.zeros(max(n_regions, 1), np.uint64)
+        n, nr = C.c_uint64(0), C.c_uint64(0)
+        args = (self.h, src.ctypes.data, src.nbytes, int(legacy), sec.ctypes.data if sec is not None else None,
+                sec.nbytes if sec is not None else 0, arr, n_regions, int(flag_exclude))
+        rc = self.lib.cbcg_pileup(*args, None, 0, C.byref(n), per.ctypes.data, None)
+        if rc != -5:
+            self._check(rc)
+        rows = np.empty((max(n.value, 1), len(PILEUP_COLUMNS)), np.uint32)
+        self._check(self.lib.cbcg_pileup(*args, rows.ctypes.data, n.value, C.byref(n), per.ctypes.data, C.byref(nr)))
+        self.last_pileup_reads = nr.value
+        ends = np.cumsum(per[:n_regions].astype(np.int64))
+        return [rows[e - int(k):e] for e, k in zip(ends.tolist(), per[:n_regions].tolist())]
 
     def cigar_pack(self, batch: Batch) -> bytes:
         """The CIGAR side section of a batch (SURVEY.md 8f row 4, cbcg.h): reads whose CIGAR is not the one their indels

@@ -43,6 +43,7 @@ struct Words {
     uint64_t chain[2];                        /* pipelined encode: edit entries so far, ping-pong between K1 launches */
     uint64_t n_selected;                      /* region decode: reads K5 kept */
     uint64_t md_chain[2];                     /* MD derivation (K7): MD bytes of the batch ([0]), or so far, ping-pong between chunk launches */
+    uint64_t pu_reads;                        /* pileup (K8): reads counted */
 };
 
 struct cbcg_ctx {
@@ -84,6 +85,7 @@ struct cbcg_ctx {
     DevBuf tri;                                /* two-kernel encode: the symbols' intervals between the model and the interval kernel */
     DevBuf reg, sel_recs, sel_chr, sel_ids;    /* region decode (k5_region.cu): intervals + ordinal runs, and the kept reads */
     DevBuf sam_aux, sam_out;                   /* SAM output (k6_sam.cu): name lengths, CIGAR classes and texts; the text */
+    DevBuf pu_aux, pu_acc, pu_rows;            /* pileup (k8_pileup.cu): intervals, regions, CIGAR classes and texts; accumulators; rows */
     DevBuf snap_a, snap_b, fin;                /* generation snapshots and per-block final states (gen_mode 1) */
     std::vector<std::pair<uint32_t, uint32_t>> gens;   /* (first block, block count) per generation of the last cut */
     uint32_t layout = 1;                       /* the call in progress: 1 = one stream per block, 4 = four substreams, 0 = four in the narrow early generations */
@@ -212,7 +214,8 @@ extern "C" void cbcg_destroy(cbcg_ctx *ctx) {
     if (ctx->hblocks) cudaFreeHost(ctx->hblocks);
     if (ctx->h_tile) cudaFreeHost(ctx->h_tile);
     for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec,
-                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out }) free_buf(*d);
+                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out,
+                       &ctx->pu_aux, &ctx->pu_acc, &ctx->pu_rows }) free_buf(*d);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->mark) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->kev) if (e) cudaEventDestroy(e);
@@ -2403,6 +2406,113 @@ extern "C" int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len
     cudaEventElapsedTime(&S.ms_d2h, ctx->ev[4], ctx->ev[5]);
     cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[5]);
     S.d2h_bytes = bytes + (read_ids && d_ids ? n_sel * 8 : 0);
+    return CBCG_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------ pileup
+ * cbcg_pileup (DESIGN.md, "Pileup"; the counts: k8_pileup.cu). The reads are cbcg_decode_sam's for the same regions: the
+ * region decode's steps give them, the CIGAR section is parsed as for K6, and K3 runs only when the section lists class-4
+ * reads (the only ones whose bases K8 reads). The regions are mapped to the loaded reference, clipped to its lengths and
+ * merged into the accumulators' intervals. The row count follows from the regions and the reference alone, so capacity
+ * is answered before anything is decoded. */
+extern "C" int cbcg_pileup(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const uint8_t *section, uint64_t section_len,
+                           const cbcg_region *regions, uint32_t n_regions, uint32_t flag_exclude, uint32_t *rows, uint64_t rows_cap,
+                           uint64_t *n_rows, uint64_t *region_rows, uint64_t *n_reads) {
+    if (!ctx || !n_rows || (section && !section_len)) return fail(ctx, CBCG_ERR_ARG, "cbcg_pileup: bad argument");
+    *n_rows = 0; if (n_reads) *n_reads = 0;
+    TRY(check_regions(ctx, regions, n_regions));
+    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
+    /* rows per region, from the loaded reference's lengths */
+    std::vector<PileupReg> reg;                              /* the regions that have rows, in request order */
+    std::vector<RegionIv> iv;                                /* their intervals, then merged */
+    uint64_t total = 0;
+    for (uint32_t k = 0; k < n_regions; k++) {
+        const size_t nl = strlen(regions[k].name);
+        size_t g = 0;
+        while (g < ctx->names.size() && !(ctx->names[g].size() == nl && !memcmp(ctx->names[g].data(), regions[k].name, nl))) g++;
+        if (g == ctx->names.size()) return fail(ctx, CBCG_ERR_NO_REFERENCE, "region %u: '%s' is not in the loaded reference", k, regions[k].name);
+        const uint64_t s = regions[k].start, e = std::min<uint64_t>(regions[k].end, ctx->h_len[g]);
+        const uint64_t n = s > e ? 0 : e - s + 1;
+        if (region_rows) region_rows[k] = n;
+        if (n) { reg.push_back({ total, s, 0, (uint32_t)g, 0u }); iv.push_back({ (uint32_t)g, 0u, s, e }); }
+        total += n;
+    }
+    *n_rows = total;
+    if (!rows || total > rows_cap)
+        return fail(ctx, CBCG_ERR_CAPACITY, "%llu rows, room for %llu", (unsigned long long)total, (unsigned long long)(rows ? rows_cap : 0));
+    merge_intervals(iv);
+    std::vector<uint64_t> iv_slot(iv.size());
+    uint64_t n_slots = 0;
+    for (size_t j = 0; j < iv.size(); j++) { iv_slot[j] = n_slots; n_slots += iv[j].end - iv[j].start + 2; }   /* + the slot after it */
+    if (n_slots > (1ull << 36)) return fail(ctx, CBCG_ERR_NOMEM, "%llu positions", (unsigned long long)n_slots);
+    const uint64_t n_pad = (n_slots + K8_SCAN_TILE - 1) / K8_SCAN_TILE * K8_SCAN_TILE;
+    for (PileupReg &R : reg) {                               /* the merged interval that holds the region */
+        const auto it = std::upper_bound(iv.begin(), iv.end(), R, [](const PileupReg &a, const RegionIv &v) {
+            return a.chr < v.chr || (a.chr == v.chr && a.start < v.start); }) - 1;
+        R.slot0 = iv_slot[it - iv.begin()] + (R.start - it->start);
+    }
+    /* the CIGAR section, by container ordinal (a legacy stream: by read, after the decode) */
+    std::vector<uint8_t> cls;
+    std::vector<uint64_t> exc_read, exc_off(1, 0);
+    std::vector<uint8_t> exc_text;
+    if (section && !legacy) {
+        Container c;
+        if (parse_container(in, in_len, nullptr, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
+        TRY(parse_cigar_section(ctx, section, section_len, c.n_reads, cls, exc_read, exc_off, exc_text));
+    }
+    uint64_t nr = 0, ne = 0, n_sel = 0; uint32_t max_len = 1, fixed_len = 0;
+    TRY(region_records(ctx, in, in_len, legacy, regions, n_regions, &nr, &ne, &n_sel, &max_len, &fixed_len));
+    if (section && legacy) TRY(parse_cigar_section(ctx, section, section_len, nr, cls, exc_read, exc_off, exc_text));
+    cbcg_stats &S = ctx->stats;
+    const uint64_t n_exc = exc_read.size();
+    const uint8_t *seq = nullptr;
+    if (n_sel && n_exc) {
+        TRY(run_reconstruct(ctx, n_sel, max_len, fixed_len, ctx->sel_chr.as<uint32_t>(), 0u, ctx->sel_recs.as<cbcg_read_rec>()));
+        seq = ctx->seq_out.as<uint8_t>();
+    } else CU(cudaMemsetAsync(wptr<unsigned long long>(ctx, W_OFF(err)), 0, 8, ctx->st));
+    /* device copies: intervals, their slots, the regions, then the section's texts and classes */
+    const uint64_t b_iv = iv.size() * sizeof(RegionIv), b_slot = iv.size() * 8, b_reg = reg.size() * sizeof(PileupReg);
+    const uint64_t b_exc = n_exc * 8, b_off = (n_exc + 1) * 8;
+    TRY(ensure(ctx, ctx->pu_aux, b_iv + b_slot + b_reg + b_exc + b_off + cls.size() + exc_text.size() + 256));
+    uint8_t *a = ctx->pu_aux.as<uint8_t>();
+    RegionIv *d_iv = reinterpret_cast<RegionIv *>(a);
+    uint64_t *d_slot = reinterpret_cast<uint64_t *>(a + b_iv);
+    PileupReg *d_reg = reinterpret_cast<PileupReg *>(a + b_iv + b_slot);
+    uint64_t *d_read = reinterpret_cast<uint64_t *>(a + b_iv + b_slot + b_reg), *d_off = d_read + n_exc;
+    uint8_t *d_cls = reinterpret_cast<uint8_t *>(d_off + n_exc + 1), *d_text = d_cls + cls.size();
+    if (b_iv) CU(cudaMemcpyAsync(d_iv, iv.data(), b_iv, cudaMemcpyHostToDevice, ctx->st));
+    if (b_slot) CU(cudaMemcpyAsync(d_slot, iv_slot.data(), b_slot, cudaMemcpyHostToDevice, ctx->st));
+    if (b_reg) CU(cudaMemcpyAsync(d_reg, reg.data(), b_reg, cudaMemcpyHostToDevice, ctx->st));
+    if (n_exc) CU(cudaMemcpyAsync(d_read, exc_read.data(), b_exc, cudaMemcpyHostToDevice, ctx->st));
+    CU(cudaMemcpyAsync(d_off, exc_off.data(), b_off, cudaMemcpyHostToDevice, ctx->st));
+    if (!cls.empty()) CU(cudaMemcpyAsync(d_cls, cls.data(), cls.size(), cudaMemcpyHostToDevice, ctx->st));
+    if (!exc_text.empty()) CU(cudaMemcpyAsync(d_text, exc_text.data(), exc_text.size(), cudaMemcpyHostToDevice, ctx->st));
+    TRY(ensure(ctx, ctx->pu_acc, n_pad * CBCG_PU_COLS * 4 + 64));
+    TRY(ensure(ctx, ctx->pu_rows, total * CBCG_PU_COLS * 4 + 64));
+    TRY(ensure(ctx, ctx->tile_desc, (std::max(pileup_num_tiles(n_sel), 2 * n_pad / K8_SCAN_TILE) + 1) * 8));
+    if (n_pad) CU(cudaMemsetAsync(ctx->pu_acc.p, 0, n_pad * CBCG_PU_COLS * 4, ctx->st));   /* zeroed on every call */
+    if (launch_pileup(n_sel, ctx->sel_recs.as<cbcg_read_rec>(), ctx->sel_chr.as<uint32_t>(), ctx->edits.as<uint16_t>(), ctx->dg, d_iv, d_slot,
+                      (uint32_t)iv.size(), flag_exclude, ctx->sel_ids.as<uint64_t>(), section ? d_cls : nullptr, d_read, d_off, d_text, n_exc,
+                      seq, max_len, fixed_len, ctx->pu_acc.as<uint32_t>(), n_pad, n_slots, d_reg, (uint32_t)reg.size(),
+                      ctx->pu_rows.as<uint32_t>(), total, ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)),
+                      wptr<uint64_t>(ctx, W_OFF(pu_reads)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "K8 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    ctx->stats.kernel_launches += (n_sel ? 1 : 0) + (n_pad ? 1 : 0) + (total ? 1 : 0);
+    CU(cudaEventRecord(ctx->ev[3], ctx->st));
+    TRY(fetch_words(ctx));                                   /* synchronises: the host vectors above may go */
+    TRY(device_error(ctx, "pileup"));
+    if (seq) cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
+    if (n_reads) *n_reads = ctx->hw->pu_reads;
+    CU(cudaEventRecord(ctx->ev[4], ctx->st));
+    if (total) CU(cudaMemcpyAsync(rows, ctx->pu_rows.p, total * CBCG_PU_COLS * 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaEventRecord(ctx->ev[5], ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    cudaEventElapsedTime(&S.ms_h2d, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&S.ms_code, ctx->ev[1], ctx->ev[2]);
+    cudaEventElapsedTime(&S.ms_reconstruct, ctx->ev[2], ctx->ev[3]);
+    cudaEventElapsedTime(&S.ms_d2h, ctx->ev[4], ctx->ev[5]);
+    cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[5]);
+    S.d2h_bytes = total * CBCG_PU_COLS * 4;
     return CBCG_OK;
 }
 

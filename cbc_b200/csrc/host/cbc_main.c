@@ -24,6 +24,14 @@
  *                   later batch whose table differs is an error), for a single-block stream from the reference; LN comes
  *                   from the reference. With -C the CIGARs are the input's (<in>.cig), else the ones the indels imply.
  *                   With -r only the region's records.
+ *          -P       -d only, with at least one -r, not with -S: pileup (cbcg_pileup): `#chrom pos ref A C G T N del ins`, then one
+ *                   tab-separated line per reference position of each region (start .. min(end, LN)), region by region in
+ *                   the order given. A C G T N count the reads that align a base there, by base; del the reads whose deletion
+ *                   covers it; ins the reads with an insertion after it that has aligned bases on both sides. A position's
+ *                   reads can sit in two batches of a "CBCS" file, so the rows of every batch are summed; a batch that no
+ *                   region touches makes no device call. With -C the CIGARs are the input's (<in>.cig), else the implied ones.
+ *          -F MASK  -P only: reads with FLAG & MASK are not counted (decimal or 0x hex; default 0x704: unmapped, secondary,
+ *                   QC fail, duplicate).
  *
  * Host C only: SAM/FASTA ingest (sam_ingest.c) and file I/O; the coding runs on the GPU through include/cbcg.h.
  * Where the reference's compress() (src/compression.c:112-170) reads a line, codes it and moves on, this driver
@@ -54,7 +62,8 @@ static int usage(void) {
     fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-M] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
                     "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n"
-                    "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n");
+                    "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n"
+                    "       cbc -d -P -r NAME[:START[-END]] [-r ...] [-C] [-F flag_mask] [-g devices] <in> <out.tsv> <ref.fa>\n");
     return 2;
 }
 
@@ -82,7 +91,7 @@ typedef struct shared {
     uint64_t next_take;                         /* next job a device thread takes */
     int producer_failed;
     /* run parameters */
-    int mode, single, var_length, with_cigar, sam, derive_md; uint32_t block_reads;
+    int mode, single, var_length, with_cigar, sam, derive_md, pileup; uint32_t block_reads, flag_exclude;
     const cbch_fasta *fa; int fa_ready;
     const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
     double t_gpu_ready;
@@ -140,6 +149,24 @@ static void *device_main(void *arg) {
                 }
             }
             if (J->have_compact) cbch_free_compact(&J->cb);
+        } else if (S->pileup) {                                   /* rows of CBCG_PU_COLS u32; the writer sums the batches */
+            uint64_t nb = 0, n_reads = 0, pb = 0, cap = 0, n = 0;
+            rc = cbcg_region_plan(J->in, J->in_len, J->legacy, S->regions, S->n_regions, &nb, &n_reads, &pb, &cap);
+            if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "region plan: %s", cbcg_strerror(rc)); }
+            else if (nb) {                                        /* a batch that no region touches costs no device call */
+                tq = now();
+                const uint8_t *sec = S->with_cigar ? J->cig_in : NULL; const uint64_t sec_len = S->with_cigar ? J->cig_in_len : 0;
+                rc = cbcg_pileup(ctx, J->in, J->in_len, J->legacy, sec, sec_len, S->regions, S->n_regions, S->flag_exclude, NULL, 0, &n, NULL, NULL);
+                if (rc == CBCG_ERR_CAPACITY) {                    /* the row count, answered before any decode */
+                    J->out = (uint8_t *)malloc(n ? n * CBCG_PU_COLS * 4 : 1);
+                    rc = J->out ? cbcg_pileup(ctx, J->in, J->in_len, J->legacy, sec, sec_len, S->regions, S->n_regions, S->flag_exclude,
+                                              (uint32_t *)J->out, n, &n, NULL, &n_reads) : CBCG_ERR_NOMEM;
+                }
+                if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "%s", ctx ? cbcg_last_error(ctx) : "no context"); }
+                J->out_len = n * CBCG_PU_COLS * 4; J->n_reads = n_reads;
+                D->call_s += now() - tq;
+                cbcg_stats st; cbcg_get_stats(ctx, &st); J->device_ms = st.ms_total;
+            }
         } else if (S->sam) {                                      /* SAM records; the writer adds the header */
             uint64_t nb = 1, n_reads = 0, pb = 0, cap = 0, n = 0;
             if (S->n_regions) {
@@ -321,6 +348,55 @@ static int parse_region(const char *a, cbcg_region *r) {
     return 0;
 }
 
+/* -P: the rows of every region by the FASTA (a name it lacks is an error), REF filled in, counts zero */
+static uint32_t *pileup_rows(const cbch_fasta *fa, const cbcg_region *reg, uint32_t n_reg, uint32_t *chr_of, uint64_t *n_rows) {
+    uint64_t total = 0;
+    for (uint32_t k = 0; k < n_reg; k++) {
+        uint32_t g = 0;
+        while (g < fa->n && strcmp(fa->names[g], reg[k].name)) g++;
+        if (g == fa->n) { fprintf(stderr, "cbc: region '%s' names no record of the reference\n", reg[k].name); return NULL; }
+        chr_of[k] = g;
+        const uint64_t e = reg[k].end < fa->len[g] ? reg[k].end : fa->len[g];
+        if (reg[k].start <= e) total += e - reg[k].start + 1;
+    }
+    uint32_t *rows = (uint32_t *)calloc(total ? total * CBCG_PU_COLS : 1, 4);
+    if (!rows) { fprintf(stderr, "cbc: out of memory\n"); return NULL; }
+    uint64_t t = 0;
+    for (uint32_t k = 0; k < n_reg; k++) {
+        const uint32_t g = chr_of[k];
+        const uint64_t e = reg[k].end < fa->len[g] ? reg[k].end : fa->len[g];
+        for (uint64_t p = reg[k].start; p <= e; p++, t++) {
+            const uint8_t c = fa->bases[g][p - 1];
+            rows[t * CBCG_PU_COLS + CBCG_PU_REF] = (c >= 'a' && c <= 'z') ? (uint32_t)(c - 32) : c;
+        }
+    }
+    *n_rows = total;
+    return rows;
+}
+/* -P: one batch's rows added to the sums; REF must agree */
+static int pileup_add(uint32_t *sum, const uint32_t *rows, uint64_t n_rows) {
+    for (uint64_t t = 0; t < n_rows; t++) {
+        uint32_t *o = sum + t * CBCG_PU_COLS; const uint32_t *r = rows + t * CBCG_PU_COLS;
+        if (o[CBCG_PU_REF] != r[CBCG_PU_REF]) return 1;
+        for (int c = 0; c < CBCG_PU_REF; c++) o[c] += r[c];
+    }
+    return 0;
+}
+static int pileup_write(FILE *fo, const uint32_t *rows, const cbch_fasta *fa, const cbcg_region *reg, uint32_t n_reg, const uint32_t *chr_of) {
+    if (fputs("#chrom\tpos\tref\tA\tC\tG\tT\tN\tdel\tins\n", fo) == EOF) return 1;
+    uint64_t t = 0;
+    for (uint32_t k = 0; k < n_reg; k++) {
+        const uint32_t g = chr_of[k];
+        const uint64_t e = reg[k].end < fa->len[g] ? reg[k].end : fa->len[g];
+        for (uint64_t p = reg[k].start; p <= e; p++, t++) {
+            const uint32_t *r = rows + t * CBCG_PU_COLS;
+            if (fprintf(fo, "%s\t%llu\t%c\t%u\t%u\t%u\t%u\t%u\t%u\t%u\n", fa->names[g], (unsigned long long)p, (char)r[CBCG_PU_REF],
+                        r[CBCG_PU_A], r[CBCG_PU_C], r[CBCG_PU_G], r[CBCG_PU_T], r[CBCG_PU_N], r[CBCG_PU_DEL], r[CBCG_PU_INS]) < 0) return 1;
+        }
+    }
+    return 0;
+}
+
 static int parse_devices(const char *s, int *dev) {
     int n = 0;
     while (*s && n < MAX_DEV) {
@@ -334,7 +410,8 @@ static int parse_devices(const char *s, int *dev) {
 }
 
 int main(int argc, char **argv) {
-    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, derive_md = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
+    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, derive_md = 0, pileup = 0, have_mask = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
+    uint32_t flag_exclude = CBCG_PILEUP_FLAG_EXCLUDE;
     uint32_t block_reads = CBCG_BLOCK_AUTO;
     uint64_t batch_mb = 2048;
     const char *files[4]; int nfiles = 0;
@@ -348,6 +425,14 @@ int main(int argc, char **argv) {
         else if (!strcmp(a, "-C")) with_cigar = 1;
         else if (!strcmp(a, "-S")) sam = 1;
         else if (!strcmp(a, "-M")) derive_md = 1;
+        else if (!strcmp(a, "-P")) pileup = 1;
+        else if (!strcmp(a, "-F") && i + 1 < argc) {
+            const char *m = argv[++i]; char *e;
+            const int hex = m[0] == '0' && (m[1] == 'x' || m[1] == 'X');
+            const unsigned long v = strtoul(hex ? m + 2 : m, &e, hex ? 16 : 10);
+            if (!*m || *e || e == (hex ? m + 2 : m) || v > 0xffffu) { fprintf(stderr, "cbc: bad flag mask '%s' (decimal or 0x hex)\n", m); return 2; }
+            flag_exclude = (uint32_t)v; have_mask = 1;
+        }
         else if (!strcmp(a, "-b") && i + 1 < argc) block_reads = (uint32_t)strtoul(argv[++i], NULL, 10);
         else if (!strcmp(a, "-B") && i + 1 < argc) batch_mb = strtoull(argv[++i], NULL, 10);
         else if (!strcmp(a, "-r") && i + 1 < argc) {
@@ -372,7 +457,11 @@ int main(int argc, char **argv) {
     if (n_regions && mode != 'd') { fprintf(stderr, "cbc: -r selects reads to decode: it goes with -d\n"); return usage(); }
     if (sam && mode != 'd') { fprintf(stderr, "cbc: -S writes SAM: it goes with -d\n"); return usage(); }
     if (derive_md && mode != 'c') { fprintf(stderr, "cbc: -M derives MD for encoding: it goes with -c\n"); return usage(); }
-    if (n_regions && with_cigar && !sam) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
+    if (pileup && mode != 'd') { fprintf(stderr, "cbc: -P writes a pileup of a container: it goes with -d\n"); return usage(); }
+    if (pileup && sam) { fprintf(stderr, "cbc: -P and -S are two outputs: choose one\n"); return usage(); }
+    if (pileup && !n_regions) { fprintf(stderr, "cbc: -P needs at least one -r region\n"); return usage(); }
+    if (have_mask && !pileup) { fprintf(stderr, "cbc: -F selects the reads a pileup counts: it goes with -P\n"); return usage(); }
+    if (n_regions && with_cigar && !sam && !pileup) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
     if (!single && block_reads == 0) block_reads = CBCG_BLOCK_AUTO;
     if (batch_mb < 1) batch_mb = 1;
 
@@ -380,7 +469,7 @@ int main(int argc, char **argv) {
     shared S; memset(&S, 0, sizeof S);
     pthread_mutex_init(&S.mu, NULL); pthread_cond_init(&S.cv, NULL);
     S.mode = mode; S.single = single; S.var_length = var_length; S.block_reads = block_reads; S.with_cigar = with_cigar;
-    S.regions = regions; S.n_regions = n_regions; S.sam = sam; S.derive_md = derive_md;
+    S.regions = regions; S.n_regions = n_regions; S.sam = sam; S.derive_md = derive_md; S.pileup = pileup; S.flag_exclude = flag_exclude;
     devthread D[MAX_DEV]; memset(D, 0, sizeof D);
 
     /* ---- the input, cut into jobs (before the device threads start: they index S.jobs) */
@@ -475,13 +564,22 @@ int main(int argc, char **argv) {
         filepos = 16 + 16 * S.n_jobs;
         if (fseek(fo, (long)filepos, SEEK_SET)) status = 1;
     }
+    uint32_t *pu_sum = NULL, *pu_chr = NULL; uint64_t pu_rows = 0;
+    if (pileup && !status) {
+        pu_chr = (uint32_t *)calloc(n_regions, 4);
+        if (!pu_chr || !(pu_sum = pileup_rows(&fa, regions, n_regions, pu_chr, &pu_rows))) status = 1;
+    }
     for (uint64_t k = 0; k < S.n_jobs && !status; k++) {
         job *J = wait_done(&S, k);
         if (!J) { fprintf(stderr, "cbc: %s\n", IA.err[0] ? IA.err : "ingest failed"); status = 1; break; }
         if (J->rc) { fprintf(stderr, "cbc: %s\n", J->err); status = 1; break; }
         if (sam && k == 0 && write_sam_header(fo, J, &fa)) { fprintf(stderr, "cbc: cannot write the SAM header of %s\n", files[0]); status = 1; break; }
         if (sam && k > 0 && sam_table_differs(S.jobs[0], J)) { fprintf(stderr, "cbc: batch %llu names other chromosomes than batch 0: one SAM header cannot describe both\n", (unsigned long long)k); status = 1; break; }
-        if (with_cigar && mode == 'd' && !sam) {                         /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
+        if (pileup) {
+            if (J->out_len && (J->out_len != pu_rows * CBCG_PU_COLS * 4 || pileup_add(pu_sum, (const uint32_t *)J->out, pu_rows))) {
+                fprintf(stderr, "cbc: batch %llu: pileup rows disagree with the reference\n", (unsigned long long)k); status = 1; break;
+            }
+        } else if (with_cigar && mode == 'd' && !sam) {                         /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
             const uint8_t *c = J->cig, *ce = J->cig + J->cig_len, *q = J->out, *qe = J->out + J->out_len;
             while (c < ce && q < qe) {
                 const uint8_t *cn = (const uint8_t *)memchr(c, '\n', (size_t)(ce - c)), *qn = (const uint8_t *)memchr(q, '\n', (size_t)(qe - q));
@@ -504,6 +602,8 @@ int main(int argc, char **argv) {
         pthread_cond_broadcast(&S.cv);
         pthread_mutex_unlock(&S.mu);
     }
+    if (pileup && !status && pileup_write(fo, pu_sum, &fa, regions, n_regions, pu_chr)) { fprintf(stderr, "cbc: cannot write %s\n", files[1]); status = 1; }
+    free(pu_sum); free(pu_chr);
     if (status) { pthread_mutex_lock(&S.mu); S.producer_failed = 1; S.next_take = S.n_jobs; pthread_cond_broadcast(&S.cv); pthread_mutex_unlock(&S.mu); }
     if (sharded && !status) {
         uint32_t h[4] = { CBCS_MAGIC, 1u, (uint32_t)S.n_jobs, 0u };

@@ -171,3 +171,18 @@ uint64_t md_num_tiles(uint64_t n_reads);
 int launch_md(const DevBatch &b, const DevGenome &g, uint64_t *md_off, uint8_t *md, uint64_t md_cap, uint64_t *tile_desc,
               uint32_t *ticket, uint64_t *total_md, unsigned long long *err, cudaStream_t st, uint64_t r_begin, uint64_t r_end,
               const uint64_t *md_base);
+/* k8_pileup.cu: per-position counts over regions. iv: the merged request intervals (genome ordinals, clipped to the record
+   lengths), iv_slot: the accumulator slot of each one's first position (each takes end - start + 2 slots); acc: 8 columns of
+   n_pad u32 (n_pad a multiple of K8_SCAN_TILE, zeroed by the caller). reg: per requested region with rows, its first output
+   row, chromosome, first position and first slot, ascending by row. cls / exc_*: as launch_sam; seq_text: K3's text of the
+   reads (needed only when cls lists class-4 reads, else NULL). rows: n_rows x CBCG_PU_COLS u32. tile_desc: max(
+   pileup_num_tiles(n_reads), 2 n_pad / K8_SCAN_TILE) words. *n_counted receives the reads counted. */
+#define K8_SCAN_TILE 1024u
+struct PileupReg { uint64_t row0, start, slot0; uint32_t chr, pad; };
+uint64_t pileup_num_tiles(uint64_t n_reads);
+int launch_pileup(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr, const uint16_t *edits, const DevGenome &g,
+                  const RegionIv *iv, const uint64_t *iv_slot, uint32_t n_iv, uint32_t flag_exclude, const uint64_t *ids, const uint8_t *cls,
+                  const uint64_t *exc_read, const uint64_t *exc_off, const uint8_t *exc_text, uint64_t n_exc, const uint8_t *seq_text,
+                  uint32_t max_len, uint32_t fixed_len, uint32_t *acc, uint64_t n_pad, uint64_t n_slots, const PileupReg *reg, uint32_t n_reg,
+                  uint32_t *rows, uint64_t n_rows, uint64_t *tile_desc, uint32_t *ticket, uint64_t *n_counted, unsigned long long *err,
+                  cudaStream_t st);

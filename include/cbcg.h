@@ -275,6 +275,34 @@ int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legac
                     uint8_t *out, uint64_t out_cap, uint64_t *out_len,
                     uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
 
+/* ---- pileup (DESIGN.md, "Pileup"): per reference position of each region, u32[CBCG_PU_COLS] = A C G T N DEL INS REF.
+ *   reads: the ones cbcg_decode_sam(section, regions) returns (the same selection, overlap rule and decode), minus those
+ *     with FLAG & flag_exclude. Each is aligned by the CIGAR of its SAM line: the section's verbatim text for class 4, else
+ *     the implied CIGAR (end I written as S per class; without a section every read is class 0).
+ *   A C G T N: the reads whose M, = or X aligns a base to the position, by that base (anything but A C G T counts as N);
+ *     their sum is the depth. DEL: the reads whose D covers it. INS: the reads with at least one inserted base between
+ *     it and the next position and an aligned base (M, = or X) before and after the insertion, so leading and trailing
+ *     insertions and soft clips never count; the position is the last reference base the CIGAR consumed (M, =, X or D)
+ *     before the inserted base. REF: the reference byte (upper-cased, as uploaded).
+ *   rows: region by region in the order given, start .. min(end, LN) each (LN: the name's length in the loaded
+ *     reference; end UINT64_MAX: to the end of the record; start > LN: no rows); overlapping or repeated regions each get
+ *     their own. region_rows (optional, n_regions entries) receives each region's row count, *n_rows their sum and
+ *     *n_reads (optional) the reads counted.
+ *   capacity: the row count depends on the regions and the loaded reference alone, so it is answered first: rows == NULL
+ *     (with rows to write) or rows_cap (in rows) too small -> CBCG_ERR_CAPACITY with *n_rows and region_rows set and
+ *     nothing decoded.
+ *   errors: as cbcg_decode_sam, and a region whose name is not in the loaded reference -> CBCG_ERR_NO_REFERENCE (its rows
+ *     need the bases and the length). A name in the reference but not in the container gets rows of zero counts.
+ *   statistics and state as cbcg_decode_sam: ms_reconstruct holds K3 (run only when the section lists class-4 reads) and
+ *     the pileup kernels, ms_k3 K3's alone. */
+enum { CBCG_PU_A, CBCG_PU_C, CBCG_PU_G, CBCG_PU_T, CBCG_PU_N, CBCG_PU_DEL, CBCG_PU_INS, CBCG_PU_REF, CBCG_PU_COLS };
+#define CBCG_PILEUP_FLAG_EXCLUDE 0x704u   /* default: UNMAP | SECONDARY | QCFAIL | DUP */
+int cbcg_pileup(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                const uint8_t *section, uint64_t section_len,
+                const cbcg_region *regions, uint32_t n_regions, uint32_t flag_exclude,
+                uint32_t *rows, uint64_t rows_cap, uint64_t *n_rows,
+                uint64_t *region_rows, uint64_t *n_reads);
+
 /* Each read's MD as the batch without MD would get it: MD + '\n' per read, in read order (samtools calmd on the device,
  * under the rule above: N against N is not a mismatch). Any MD the batch carries is ignored. out_cap too small ->
  * CBCG_ERR_CAPACITY with *out_len the size needed. State: the batch is uploaded (it becomes the resident batch, with the
