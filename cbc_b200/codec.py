@@ -43,12 +43,13 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
            "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
            "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam", "cbcg_derive_md",
-           "cbcg_pileup"]
+           "cbcg_pileup", "cbcg_bam_header", "cbcg_decode_bam"]
 
 
 UINT64_MAX = (1 << 64) - 1
 PILEUP_COLUMNS = ("A", "C", "G", "T", "N", "DEL", "INS", "REF")      # CBCG_PU_A .. CBCG_PU_REF
 PILEUP_FLAG_EXCLUDE = 0x704                                          # UNMAP | SECONDARY | QCFAIL | DUP
+BAM_HEADER, BAM_EOF = 1, 2                                           # CBCG_BAM_HEADER, CBCG_BAM_EOF
 
 
 class Region(C.Structure):
@@ -168,6 +169,8 @@ def load_library():
         lib.cbcg_decode_sam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_derive_md.argtypes = [vp, P(CBatch), vp, u64, P(u64)]
         lib.cbcg_pileup.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, P(u64)]
+        lib.cbcg_bam_header.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(u64)]
+        lib.cbcg_decode_bam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -417,6 +420,51 @@ class Codec:
                 continue
             self._check(rc)
             return out[:n.value].tobytes(), ids[:nr.value].copy()
+
+    def decompress_bam(self, data: bytes, cigar_section: Optional[bytes] = None, regions=None, header: bool = True,
+                       eof: bool = True, legacy: bool = False) -> Tuple[bytes, np.ndarray]:
+        """BAM of a container (include/cbcg.h, cbcg_decode_bam): ``decompress_sam``'s reads as BAM records in BGZF blocks,
+        after the header blocks (header=True) and before the end-of-file block (eof=True); and each record's read ordinal in
+        the container as uint64. cigar_section and regions: as ``decompress_sam``. The output of several calls without
+        header and EOF concatenates into one file between ``bam_header`` and the EOF block."""
+        src = np.frombuffer(data, np.uint8)
+        sec = np.frombuffer(cigar_section, np.uint8) if cigar_section is not None else None
+        if regions is not None:
+            arr, n_regions = _region_array(regions)                          # an empty list is CBCG_ERR_ARG
+        else:
+            arr, n_regions = None, 0
+        flags = (BAM_HEADER if header else 0) | (BAM_EOF if eof else 0)
+        n_ids = 1 << 16
+        size = max(len(data) * 8, 1 << 20)
+        if not legacy:
+            n_reads, cap = C.c_uint64(0), C.c_uint64(0)
+            if self.lib.cbcg_decoded_size(src.ctypes.data, src.nbytes, C.byref(n_reads), C.byref(cap)) == 0:
+                size, n_ids = max(size, 2 * cap.value + 1024), max(n_reads.value, 1)
+        while True:
+            out = np.empty(size, np.uint8)
+            ids = np.empty(n_ids, np.uint64)
+            n, nr = C.c_uint64(0), C.c_uint64(0)
+            rc = self.lib.cbcg_decode_bam(self.h, src.ctypes.data, src.nbytes, int(legacy),
+                                          sec.ctypes.data if sec is not None else None, sec.nbytes if sec is not None else 0,
+                                          arr, n_regions, flags, out.ctypes.data, out.nbytes, C.byref(n),
+                                          ids.ctypes.data, ids.size, C.byref(nr))
+            if rc == -5 and (n.value > out.nbytes or nr.value > ids.size):
+                size, n_ids = max(size, n.value), max(n_ids, nr.value)
+                continue
+            self._check(rc)
+            return out[:n.value].tobytes(), ids[:nr.value].copy()
+
+    def bam_header(self, data: bytes, legacy: bool = False) -> bytes:
+        """The BAM header of a container in BGZF blocks (include/cbcg.h, cbcg_bam_header): its table's names with the loaded
+        reference's lengths (legacy: the loaded reference's names). Host only; needs ``set_reference``."""
+        src = np.frombuffer(data, np.uint8)
+        n = C.c_uint64(0)
+        rc = self.lib.cbcg_bam_header(self.h, src.ctypes.data, src.nbytes, int(legacy), None, 0, C.byref(n))
+        if rc != -5:
+            self._check(rc)
+        out = np.empty(max(n.value, 1), np.uint8)
+        self._check(self.lib.cbcg_bam_header(self.h, src.ctypes.data, src.nbytes, int(legacy), out.ctypes.data, out.nbytes, C.byref(n)))
+        return out[:n.value].tobytes()
 
     def pileup(self, data: bytes, regions, cigar_section: Optional[bytes] = None, flag_exclude: int = PILEUP_FLAG_EXCLUDE,
                legacy: bool = False) -> List[np.ndarray]:

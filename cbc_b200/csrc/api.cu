@@ -85,6 +85,7 @@ struct cbcg_ctx {
     DevBuf tri;                                /* two-kernel encode: the symbols' intervals between the model and the interval kernel */
     DevBuf reg, sel_recs, sel_chr, sel_ids;    /* region decode (k5_region.cu): intervals + ordinal runs, and the kept reads */
     DevBuf sam_aux, sam_out;                   /* SAM output (k6_sam.cu): name lengths, CIGAR classes and texts; the text */
+    DevBuf bam_rec, bam_idx;                   /* BAM output (k9_bam.cu): the uncompressed record stream; record offsets and block starts */
     DevBuf pu_aux, pu_acc, pu_rows;            /* pileup (k8_pileup.cu): intervals, regions, CIGAR classes and texts; accumulators; rows */
     DevBuf snap_a, snap_b, fin;                /* generation snapshots and per-block final states (gen_mode 1) */
     std::vector<std::pair<uint32_t, uint32_t>> gens;   /* (first block, block count) per generation of the last cut */
@@ -214,7 +215,7 @@ extern "C" void cbcg_destroy(cbcg_ctx *ctx) {
     if (ctx->hblocks) cudaFreeHost(ctx->hblocks);
     if (ctx->h_tile) cudaFreeHost(ctx->h_tile);
     for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec,
-                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out,
+                       &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out, &ctx->bam_rec, &ctx->bam_idx,
                        &ctx->pu_aux, &ctx->pu_acc, &ctx->pu_rows }) free_buf(*d);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->mark) if (e) cudaEventDestroy(e);
@@ -2299,99 +2300,17 @@ extern "C" int cbcg_sam_header(const uint8_t *in, uint64_t in_len, uint8_t *out,
     return CBCG_OK;
 }
 
-extern "C" int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
-                               const uint8_t *section, uint64_t section_len,
-                               const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
-                               uint8_t *out, uint64_t out_cap, uint64_t *out_len,
-                               uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
-    if (!ctx || !out_len || (flags & ~CBCG_SAM_HEADER) || (!regions && n_regions) || (section && !section_len))
-        return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_sam: bad argument");
-    *out_len = 0; if (n_reads) *n_reads = 0;
-    if (regions) TRY(check_regions(ctx, regions, n_regions));
-    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
-    /* the chromosome table (legacy: the loaded reference) and the read count the section must match */
-    std::vector<std::string> table = ctx->names;
-    uint64_t cont_reads = 0;
-    if (!legacy) {
-        Container c;
-        if (parse_container(in, in_len, nullptr, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
-        table = container_names(in, c);
-        cont_reads = c.n_reads;
-    }
-    std::vector<uint8_t> cls;
-    std::vector<uint64_t> exc_read, exc_off(1, 0);
-    std::vector<uint8_t> exc_text;
-    if (section && !legacy) TRY(parse_cigar_section(ctx, section, section_len, cont_reads, cls, exc_read, exc_off, exc_text));
-    /* records: every read, or the region's (with their container ordinals) */
-    uint64_t nr = 0, ne = 0, n_sel = 0; uint32_t max_len = 1, fixed_len = 0;
-    const cbcg_read_rec *d_recs = ctx->recs.as<cbcg_read_rec>();
-    const uint32_t *d_chr = nullptr; const uint64_t *d_ids = nullptr;
-    uint32_t ref_hint = 0;
-    if (!regions) {
-        TRY(decode_to_records(ctx, in, in_len, legacy, &nr, &ne, &max_len, &fixed_len));
-        if (legacy) max_len = CBCG_MAX_READ_LEN;            /* per-read lengths are coded mod 256 (src/read_compression.c:29-33) */
-        else ref_hint = ref_window_from_blocks(ctx, max_len);
-        n_sel = nr;
-        d_recs = ctx->recs.as<cbcg_read_rec>(); d_chr = ctx->chr_out.as<uint32_t>();
-    } else {
-        TRY(region_records(ctx, in, in_len, legacy, regions, n_regions, &nr, &ne, &n_sel, &max_len, &fixed_len));
-        d_recs = ctx->sel_recs.as<cbcg_read_rec>(); d_chr = ctx->sel_chr.as<uint32_t>(); d_ids = ctx->sel_ids.as<uint64_t>();
-    }
-    if (section && legacy) TRY(parse_cigar_section(ctx, section, section_len, nr, cls, exc_read, exc_off, exc_text));   /* a legacy stream is decoded whole */
+/* The end of cbcg_decode_sam / cbcg_decode_bam: the output in ctx->sam_out (bytes of it) becomes "the decoded text" that
+ * cbcg_fetch_decoded returns, then capacity, the copies out and the statistics. */
+static int finish_sam_like(cbcg_ctx *ctx, uint64_t bytes, uint64_t n_sel, const uint64_t *d_ids, uint8_t *out, uint64_t out_cap,
+                           uint64_t *out_len, uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads, const char *what) {
     cbcg_stats &S = ctx->stats;
-    std::vector<uint64_t> lengths(table.size(), UINT64_MAX);
-    for (size_t k = 0; k < table.size(); k++)
-        for (size_t g = 0; g < ctx->names.size(); g++)
-            if (ctx->names[g] == table[k]) { lengths[k] = ctx->h_len[g]; break; }
-    const std::string head = (flags & CBCG_SAM_HEADER) ? sam_header_text(table, &lengths) : std::string();
-    uint64_t rec_bytes = 0;
-    if (n_sel) {
-        TRY(run_reconstruct(ctx, n_sel, max_len, fixed_len, d_chr, ref_hint, d_recs));
-        /* an upper bound on the lines (k6_sam.cu): per read 64 bytes of fields, the name, SEQ, 16 per edit (implied CIGAR +
-           MD), and per verbatim CIGAR its text, 4 per base and 5 per deleted base (<= 255) of MD */
-        size_t max_name = 0;
-        std::vector<uint32_t> name_len(ctx->names.size());
-        for (size_t g = 0; g < ctx->names.size(); g++) { name_len[g] = (uint32_t)ctx->names[g].size(); max_name = std::max(max_name, ctx->names[g].size()); }
-        const uint64_t bound = n_sel * (64u + max_name + max_len) + 16u * ne + exc_text.size() + exc_read.size() * (4u * max_len + 5u * 255u + 8u) + 64u;
-        const uint64_t n_exc = exc_read.size();
-        const uint64_t aux = name_len.size() * 4 + cls.size() + (2 * n_exc + 1) * 8 + exc_text.size() + 256;
-        TRY(ensure(ctx, ctx->sam_aux, aux));
-        TRY(ensure(ctx, ctx->sam_out, head.size() + bound + 64));
-        TRY(ensure(ctx, ctx->tile_desc, (2 * sam_num_tiles(n_sel) + 1) * 8));
-        uint8_t *a = ctx->sam_aux.as<uint8_t>();
-        uint64_t *d_read = reinterpret_cast<uint64_t *>(a), *d_off = d_read + n_exc;
-        uint32_t *d_nl = reinterpret_cast<uint32_t *>(d_off + n_exc + 1);
-        uint8_t *d_cls = reinterpret_cast<uint8_t *>(d_nl + name_len.size()), *d_text = d_cls + cls.size();
-        if (n_exc) CU(cudaMemcpyAsync(d_read, exc_read.data(), n_exc * 8, cudaMemcpyHostToDevice, ctx->st));
-        CU(cudaMemcpyAsync(d_off, exc_off.data(), (n_exc + 1) * 8, cudaMemcpyHostToDevice, ctx->st));
-        CU(cudaMemcpyAsync(d_nl, name_len.data(), name_len.size() * 4, cudaMemcpyHostToDevice, ctx->st));
-        if (!cls.empty()) CU(cudaMemcpyAsync(d_cls, cls.data(), cls.size(), cudaMemcpyHostToDevice, ctx->st));
-        if (!exc_text.empty()) CU(cudaMemcpyAsync(d_text, exc_text.data(), exc_text.size(), cudaMemcpyHostToDevice, ctx->st));
-        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
-        if (launch_sam(n_sel, d_recs, d_chr, ctx->edits.as<uint16_t>(), ctx->dg, ctx->g_names.as<uint8_t>(), d_nl, ctx->seq_out.as<uint8_t>(),
-                       max_len, fixed_len, d_ids, section ? d_cls : nullptr, d_read, d_off, d_text, n_exc,
-                       ctx->sam_out.as<uint8_t>() + head.size(), bound, ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)),
-                       wptr<uint64_t>(ctx, W_OFF(total_bytes)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
-            return fail(ctx, CBCG_ERR_CUDA, "K6 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-        ctx->stats.kernel_launches++;
-        CU(cudaEventRecord(ctx->ev[3], ctx->st));
-        TRY(fetch_words(ctx));                               /* synchronises: the host vectors above may go */
-        TRY(device_error(ctx, "SAM output"));
-        cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
-        rec_bytes = ctx->hw->total_bytes;
-    } else {
-        TRY(ensure(ctx, ctx->sam_out, head.size() + 64));
-        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
-        CU(cudaEventRecord(ctx->ev[3], ctx->st));
-    }
-    /* the SAM text becomes "the decoded text" that cbcg_fetch_decoded returns */
     std::swap(ctx->seq_out, ctx->sam_out);
-    const uint64_t bytes = head.size() + rec_bytes;
     *out_len = bytes; if (n_reads) *n_reads = n_sel;
     ctx->dec_bytes = bytes; ctx->dec_n_reads = n_sel; ctx->have_decoded = true;
     if (bytes > out_cap || (!out && bytes) || (read_ids && n_sel > ids_cap))
-        return fail(ctx, CBCG_ERR_CAPACITY, "%llu reads / %llu bytes of SAM, room for %llu / %llu", (unsigned long long)n_sel,
-                    (unsigned long long)bytes, (unsigned long long)ids_cap, (unsigned long long)out_cap);
+        return fail(ctx, CBCG_ERR_CAPACITY, "%llu reads / %llu bytes of %s, room for %llu / %llu", (unsigned long long)n_sel,
+                    (unsigned long long)bytes, what, (unsigned long long)ids_cap, (unsigned long long)out_cap);
     CU(cudaEventRecord(ctx->ev[4], ctx->st));
     if (bytes) CU(cudaMemcpyAsync(out, ctx->seq_out.p, bytes, cudaMemcpyDeviceToHost, ctx->st));
     if (read_ids && n_sel) {
@@ -2407,6 +2326,253 @@ extern "C" int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len
     cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[5]);
     S.d2h_bytes = bytes + (read_ids && d_ids ? n_sel * 8 : 0);
     return CBCG_OK;
+}
+
+/* What cbcg_decode_sam and cbcg_decode_bam share. sam_table: the chromosome table (legacy: the loaded reference) and the
+ * read count the section must match. sam_records: the section, then the records -- every read, or the regions' (with their
+ * container ordinals). upload_sam_section: the section's classes and class-4 texts on the device, with `extra` bytes after
+ * them for the caller. */
+struct SamRecords {
+    std::vector<std::string> table;
+    uint64_t cont_reads = 0;
+    std::vector<uint8_t> cls;
+    std::vector<uint64_t> exc_read, exc_off{ 0 };
+    std::vector<uint8_t> exc_text;
+    uint64_t nr = 0, ne = 0, n_sel = 0;
+    uint32_t max_len = 1, fixed_len = 0, ref_hint = 0;
+    const cbcg_read_rec *d_recs = nullptr; const uint32_t *d_chr = nullptr; const uint64_t *d_ids = nullptr;
+};
+struct SamAux { const uint64_t *read, *off; const uint8_t *cls, *text; uint8_t *extra; };
+static int sam_table(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const cbcg_region *regions, uint32_t n_regions, SamRecords &R) {
+    if (regions) TRY(check_regions(ctx, regions, n_regions));
+    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_set_reference has not been called");
+    R.table = ctx->names;
+    if (!legacy) {
+        Container c;
+        if (parse_container(in, in_len, nullptr, c)) return fail(ctx, CBCG_ERR_FORMAT, "malformed container header");
+        R.table = container_names(in, c);
+        R.cont_reads = c.n_reads;
+    }
+    return 0;
+}
+static int sam_records(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, const uint8_t *section, uint64_t section_len,
+                       const cbcg_region *regions, uint32_t n_regions, SamRecords &R) {
+    if (section && !legacy) TRY(parse_cigar_section(ctx, section, section_len, R.cont_reads, R.cls, R.exc_read, R.exc_off, R.exc_text));
+    if (!regions) {
+        TRY(decode_to_records(ctx, in, in_len, legacy, &R.nr, &R.ne, &R.max_len, &R.fixed_len));
+        if (legacy) R.max_len = CBCG_MAX_READ_LEN;          /* per-read lengths are coded mod 256 (src/read_compression.c:29-33) */
+        else R.ref_hint = ref_window_from_blocks(ctx, R.max_len);
+        R.n_sel = R.nr;
+        R.d_recs = ctx->recs.as<cbcg_read_rec>(); R.d_chr = ctx->chr_out.as<uint32_t>();
+    } else {
+        TRY(region_records(ctx, in, in_len, legacy, regions, n_regions, &R.nr, &R.ne, &R.n_sel, &R.max_len, &R.fixed_len));
+        R.d_recs = ctx->sel_recs.as<cbcg_read_rec>(); R.d_chr = ctx->sel_chr.as<uint32_t>(); R.d_ids = ctx->sel_ids.as<uint64_t>();
+    }
+    if (section && legacy) TRY(parse_cigar_section(ctx, section, section_len, R.nr, R.cls, R.exc_read, R.exc_off, R.exc_text));   /* a legacy stream is decoded whole */
+    return 0;
+}
+static int upload_sam_section(cbcg_ctx *ctx, const SamRecords &R, const void *extra, uint64_t extra_bytes, SamAux &A) {
+    const uint64_t n_exc = R.exc_read.size();
+    TRY(ensure(ctx, ctx->sam_aux, (2 * n_exc + 1) * 8 + extra_bytes + R.cls.size() + R.exc_text.size() + 256));
+    uint64_t *d_read = ctx->sam_aux.as<uint64_t>(), *d_off = d_read + n_exc;
+    uint8_t *d_extra = reinterpret_cast<uint8_t *>(d_off + n_exc + 1);
+    uint8_t *d_cls = d_extra + extra_bytes, *d_text = d_cls + R.cls.size();
+    if (n_exc) CU(cudaMemcpyAsync(d_read, R.exc_read.data(), n_exc * 8, cudaMemcpyHostToDevice, ctx->st));
+    CU(cudaMemcpyAsync(d_off, R.exc_off.data(), (n_exc + 1) * 8, cudaMemcpyHostToDevice, ctx->st));
+    if (extra_bytes) CU(cudaMemcpyAsync(d_extra, extra, extra_bytes, cudaMemcpyHostToDevice, ctx->st));
+    if (!R.cls.empty()) CU(cudaMemcpyAsync(d_cls, R.cls.data(), R.cls.size(), cudaMemcpyHostToDevice, ctx->st));
+    if (!R.exc_text.empty()) CU(cudaMemcpyAsync(d_text, R.exc_text.data(), R.exc_text.size(), cudaMemcpyHostToDevice, ctx->st));
+    A = { d_read, d_off, d_cls, d_text, d_extra };
+    return 0;
+}
+
+extern "C" int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                               const uint8_t *section, uint64_t section_len,
+                               const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
+                               uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                               uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
+    if (!ctx || !out_len || (flags & ~CBCG_SAM_HEADER) || (!regions && n_regions) || (section && !section_len))
+        return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_sam: bad argument");
+    *out_len = 0; if (n_reads) *n_reads = 0;
+    SamRecords R;
+    TRY(sam_table(ctx, in, in_len, legacy, regions, n_regions, R));
+    TRY(sam_records(ctx, in, in_len, legacy, section, section_len, regions, n_regions, R));
+    const std::vector<std::string> &table = R.table;
+    const uint64_t n_sel = R.n_sel, ne = R.ne;
+    const uint32_t max_len = R.max_len;
+    const uint64_t *d_ids = R.d_ids;
+    cbcg_stats &S = ctx->stats;
+    std::vector<uint64_t> lengths(table.size(), UINT64_MAX);
+    for (size_t k = 0; k < table.size(); k++)
+        for (size_t g = 0; g < ctx->names.size(); g++)
+            if (ctx->names[g] == table[k]) { lengths[k] = ctx->h_len[g]; break; }
+    const std::string head = (flags & CBCG_SAM_HEADER) ? sam_header_text(table, &lengths) : std::string();
+    uint64_t rec_bytes = 0;
+    if (n_sel) {
+        TRY(run_reconstruct(ctx, n_sel, max_len, R.fixed_len, R.d_chr, R.ref_hint, R.d_recs));
+        /* an upper bound on the lines (k6_sam.cu): per read 64 bytes of fields, the name, SEQ, 16 per edit (implied CIGAR +
+           MD), and per verbatim CIGAR its text, 4 per base and 5 per deleted base (<= 255) of MD */
+        size_t max_name = 0;
+        std::vector<uint32_t> name_len(ctx->names.size());
+        for (size_t g = 0; g < ctx->names.size(); g++) { name_len[g] = (uint32_t)ctx->names[g].size(); max_name = std::max(max_name, ctx->names[g].size()); }
+        const uint64_t bound = n_sel * (64u + max_name + max_len) + 16u * ne + R.exc_text.size() + R.exc_read.size() * (4u * max_len + 5u * 255u + 8u) + 64u;
+        SamAux A;
+        TRY(upload_sam_section(ctx, R, name_len.data(), name_len.size() * 4, A));
+        TRY(ensure(ctx, ctx->sam_out, head.size() + bound + 64));
+        TRY(ensure(ctx, ctx->tile_desc, (2 * sam_num_tiles(n_sel) + 1) * 8));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        if (launch_sam(n_sel, R.d_recs, R.d_chr, ctx->edits.as<uint16_t>(), ctx->dg, ctx->g_names.as<uint8_t>(), reinterpret_cast<const uint32_t *>(A.extra),
+                       ctx->seq_out.as<uint8_t>(), max_len, R.fixed_len, d_ids, section ? A.cls : nullptr, A.read, A.off, A.text, R.exc_read.size(),
+                       ctx->sam_out.as<uint8_t>() + head.size(), bound, ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)),
+                       wptr<uint64_t>(ctx, W_OFF(total_bytes)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+            return fail(ctx, CBCG_ERR_CUDA, "K6 launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        ctx->stats.kernel_launches++;
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+        TRY(fetch_words(ctx));                               /* synchronises: the host vectors above may go */
+        TRY(device_error(ctx, "SAM output"));
+        cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
+        rec_bytes = ctx->hw->total_bytes;
+    } else {
+        TRY(ensure(ctx, ctx->sam_out, head.size() + 64));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+    }
+    return finish_sam_like(ctx, head.size() + rec_bytes, n_sel, d_ids, out, out_cap, out_len, read_ids, ids_cap, n_reads, "SAM");
+}
+
+/* ------------------------------------------------------------------------------------------------ BAM output
+ * cbcg_bam_header / cbcg_decode_bam (DESIGN.md 5f; the records and the BGZF blocks: k9_bam.cu). The reads, their CIGARs
+ * and MD / NM are cbcg_decode_sam's: the same records, section and K3, then K9 instead of K6. The header is built here
+ * in BGZF blocks of stored deflate blocks. */
+static const uint8_t BGZF_EOF[28] = { 0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0 };
+#define BAM_STORED_BLOCK 65280u                               /* header bytes per BGZF block */
+
+static uint32_t host_crc32(const uint8_t *p, size_t n) {
+    static uint32_t tab[256];
+    if (!tab[1]) for (uint32_t k = 0; k < 256; k++) { uint32_t c = k; for (int j = 0; j < 8; j++) c = (c & 1u) ? (c >> 1) ^ 0xedb88320u : c >> 1; tab[k] = c; }
+    uint32_t c = 0xffffffffu;
+    for (size_t i = 0; i < n; i++) c = tab[(c ^ p[i]) & 0xffu] ^ (c >> 8);
+    return c ^ 0xffffffffu;
+}
+static void put_le32(std::vector<uint8_t> &v, uint32_t x) { for (int i = 0; i < 4; i++) v.push_back((uint8_t)(x >> (8 * i))); }
+
+/* The BAM header of a name table: "BAM\1", l_text, cbcg_decode_sam's header text, n_ref, then (l_name, name\0, l_ref) per
+ * name, in BGZF blocks of one stored deflate block each. Every name needs its length from the loaded reference. */
+static int bam_header_blocks(cbcg_ctx *ctx, const std::vector<std::string> &table, std::vector<uint8_t> &out) {
+    std::vector<uint64_t> lengths(table.size(), UINT64_MAX);
+    for (size_t k = 0; k < table.size(); k++) {
+        for (size_t g = 0; g < ctx->names.size(); g++)
+            if (ctx->names[g] == table[k]) { lengths[k] = ctx->h_len[g]; break; }
+        if (lengths[k] == UINT64_MAX) return fail(ctx, CBCG_ERR_NO_REFERENCE, "'%s' is not in the loaded reference: a BAM header needs its length", table[k].c_str());
+        if (lengths[k] > 0x7fffffffull) return fail(ctx, CBCG_ERR_INPUT, "'%s' is %llu bases long: BAM lengths stop at 2^31 - 1", table[k].c_str(), (unsigned long long)lengths[k]);
+    }
+    const std::string text = sam_header_text(table, &lengths);
+    std::vector<uint8_t> raw = { 'B', 'A', 'M', 1 };
+    put_le32(raw, (uint32_t)text.size());
+    raw.insert(raw.end(), text.begin(), text.end());
+    put_le32(raw, (uint32_t)table.size());
+    for (size_t k = 0; k < table.size(); k++) {
+        put_le32(raw, (uint32_t)table[k].size() + 1u);
+        raw.insert(raw.end(), table[k].begin(), table[k].end());
+        raw.push_back(0);
+        put_le32(raw, (uint32_t)lengths[k]);
+    }
+    out.clear();
+    for (size_t a = 0; a < raw.size(); a += BAM_STORED_BLOCK) {
+        const uint32_t n = (uint32_t)std::min<size_t>(BAM_STORED_BLOCK, raw.size() - a);
+        const uint32_t bsize = 18u + 5u + n + 8u - 1u;
+        const uint8_t h[18] = { 0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, (uint8_t)bsize, (uint8_t)(bsize >> 8) };
+        out.insert(out.end(), h, h + 18);
+        out.push_back(1);                                    /* BFINAL 1, BTYPE 00: stored */
+        out.push_back((uint8_t)n); out.push_back((uint8_t)(n >> 8));
+        out.push_back((uint8_t)~n); out.push_back((uint8_t)(~n >> 8));
+        out.insert(out.end(), raw.begin() + a, raw.begin() + a + n);
+        put_le32(out, host_crc32(raw.data() + a, n));
+        put_le32(out, n);
+    }
+    return 0;
+}
+
+extern "C" int cbcg_bam_header(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!ctx || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_bam_header: bad argument");
+    *out_len = 0;
+    SamRecords R;
+    TRY(sam_table(ctx, in, in_len, legacy, nullptr, 0, R));
+    std::vector<uint8_t> h;
+    TRY(bam_header_blocks(ctx, R.table, h));
+    *out_len = h.size();
+    if (!out || h.size() > out_cap) return fail(ctx, CBCG_ERR_CAPACITY, "BAM header is %llu bytes, room for %llu", (unsigned long long)h.size(), (unsigned long long)out_cap);
+    memcpy(out, h.data(), h.size());
+    return CBCG_OK;
+}
+
+extern "C" int cbcg_decode_bam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                               const uint8_t *section, uint64_t section_len,
+                               const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
+                               uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                               uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads) {
+    if (!ctx || !out_len || (flags & ~(CBCG_BAM_HEADER | CBCG_BAM_EOF)) || (!regions && n_regions) || (section && !section_len))
+        return fail(ctx, CBCG_ERR_ARG, "cbcg_decode_bam: bad argument");
+    *out_len = 0; if (n_reads) *n_reads = 0;
+    SamRecords R;
+    TRY(sam_table(ctx, in, in_len, legacy, regions, n_regions, R));
+    std::vector<uint8_t> head;
+    if (flags & CBCG_BAM_HEADER) TRY(bam_header_blocks(ctx, R.table, head));   /* before anything is decoded */
+    TRY(sam_records(ctx, in, in_len, legacy, section, section_len, regions, n_regions, R));
+    const uint64_t n_sel = R.n_sel;
+    const uint32_t max_len = R.max_len;
+    cbcg_stats &S = ctx->stats;
+    const uint64_t eof = (flags & CBCG_BAM_EOF) ? sizeof BGZF_EOF : 0;
+    uint64_t blk_bytes = 0;
+    if (n_sel) {
+        TRY(run_reconstruct(ctx, n_sel, max_len, R.fixed_len, R.d_chr, R.ref_hint, R.d_recs));
+        /* refID: a genome record's index in the table (first match), -1 for a record the table does not name */
+        std::vector<int32_t> ref_id(ctx->names.size(), -1);
+        for (size_t g = 0; g < ctx->names.size(); g++)
+            for (size_t k = 0; k < R.table.size(); k++)
+                if (R.table[k] == ctx->names[g]) { ref_id[g] = (int32_t)k; break; }
+        /* an upper bound on the records (k9_bam.cu): per read 64 bytes of fixed fields, tags and the MD's last number, SEQ
+           and QUAL (3 / 2 per base), 20 per edit (<= 3 CIGAR operations and <= 5 bytes of MD), and per verbatim CIGAR 2 per
+           byte of text (an operation takes >= 2 characters and 4 bytes), 4 per base and 5 per deleted base (<= 255) of MD */
+        const uint64_t bound = n_sel * (64u + (3u * max_len + 1u) / 2u) + 20u * R.ne + 2u * R.exc_text.size() +
+                               R.exc_read.size() * (4u * max_len + 5u * 255u + 8u) + 64u;
+        const uint64_t max_blocks = bound / K9_BLOCK_CUT + 2u;
+        SamAux A;
+        TRY(upload_sam_section(ctx, R, ref_id.data(), ref_id.size() * 4, A));
+        TRY(ensure(ctx, ctx->bam_rec, bound + 64));
+        TRY(ensure(ctx, ctx->bam_idx, (n_sel + 1) * 8 + (max_blocks + 1) * 4 + 64));
+        TRY(ensure(ctx, ctx->tile_desc, (std::max<uint64_t>(2 * bam_num_tiles(n_sel), max_blocks) + 1) * 8));
+        uint64_t *d_rec_off = ctx->bam_idx.as<uint64_t>();
+        uint32_t *d_first = reinterpret_cast<uint32_t *>(d_rec_off + n_sel + 1);
+        uint64_t *totals = wptr<uint64_t>(ctx, W_OFF(totals));
+        if (launch_bam_records(n_sel, R.d_recs, R.d_chr, ctx->edits.as<uint16_t>(), ctx->dg, reinterpret_cast<const int32_t *>(A.extra),
+                               ctx->seq_out.as<uint8_t>(), max_len, R.fixed_len, R.d_ids, section ? A.cls : nullptr, A.read, A.off, A.text,
+                               R.exc_read.size(), ctx->bam_rec.as<uint8_t>(), bound, d_rec_off, d_first, ctx->tile_desc.as<uint64_t>(),
+                               wptr<uint32_t>(ctx, W_OFF(ticket)), totals, wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+            return fail(ctx, CBCG_ERR_CUDA, "K9 record launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        TRY(fetch_words(ctx));                               /* synchronises: the block count sizes the BGZF launch */
+        TRY(device_error(ctx, "BAM records"));
+        const uint64_t rec_bytes = ctx->hw->totals[0], n_blocks = ctx->hw->totals[1];
+        /* a fixed-Huffman block costs at most 9 bits per byte, and 26 bytes of framing + 2 of bit padding */
+        TRY(ensure(ctx, ctx->sam_out, head.size() + rec_bytes + rec_bytes / 8 + 28 * n_blocks + eof + 64));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        if (launch_bgzf(ctx->bam_rec.as<uint8_t>(), d_rec_off, d_first, (uint32_t)n_blocks, ctx->sam_out.as<uint8_t>() + head.size(),
+                        ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)), wptr<uint64_t>(ctx, W_OFF(total_bytes)),
+                        wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+            return fail(ctx, CBCG_ERR_CUDA, "K9 BGZF launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        ctx->stats.kernel_launches += 2;
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+        TRY(fetch_words(ctx));
+        TRY(device_error(ctx, "BGZF blocks"));
+        cudaEventElapsedTime(&S.ms_k3, ctx->kev[2], ctx->kev[3]);
+        blk_bytes = ctx->hw->total_bytes;
+    } else {
+        TRY(ensure(ctx, ctx->sam_out, head.size() + eof + 64));
+        if (!head.empty()) CU(cudaMemcpyAsync(ctx->sam_out.p, head.data(), head.size(), cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaEventRecord(ctx->ev[3], ctx->st));
+    }
+    if (eof) CU(cudaMemcpyAsync(ctx->sam_out.as<uint8_t>() + head.size() + blk_bytes, BGZF_EOF, eof, cudaMemcpyHostToDevice, ctx->st));
+    return finish_sam_like(ctx, head.size() + blk_bytes + eof, n_sel, R.d_ids, out, out_cap, out_len, read_ids, ids_cap, n_reads, "BAM");
 }
 
 /* ------------------------------------------------------------------------------------------------ pileup

@@ -24,6 +24,12 @@
  *                   later batch whose table differs is an error), for a single-block stream from the reference; LN comes
  *                   from the reference. With -C the CIGARs are the input's (<in>.cig), else the ones the indels imply.
  *                   With -r only the region's records.
+ *          -Z       -d only, not with -S or -P: write BAM (cbcg_decode_bam): the records -S writes, as BAM records in BGZF blocks
+ *                   (SEQ through the 4-bit code). The header blocks come from batch 0 (cbcg_bam_header: its chromosome table,
+ *                   every name's length from the reference; a later batch whose table differs is an error), then each
+ *                   batch's record blocks, then the BGZF end-of-file block. With -C the CIGARs are the input's (<in>.cig),
+ *                   else the ones the indels imply. With -r only the region's records; a batch that no region touches makes
+ *                   no device call.
  *          -P       -d only, with at least one -r, not with -S: pileup (cbcg_pileup): `#chrom pos ref A C G T N del ins`, then one
  *                   tab-separated line per reference position of each region (start .. min(end, LN)), region by region in
  *                   the order given. A C G T N count the reads that align a base there, by base; del the reads whose deletion
@@ -63,6 +69,7 @@ static int usage(void) {
                     "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n"
+                    "       cbc -d -Z [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.bam> <ref.fa>\n"
                     "       cbc -d -P -r NAME[:START[-END]] [-r ...] [-C] [-F flag_mask] [-g devices] <in> <out.tsv> <ref.fa>\n");
     return 2;
 }
@@ -82,6 +89,7 @@ typedef struct job {
     int rc; char err[256];
     int done, written;
     uint64_t bound, seq_bases; uint32_t header_len;
+    uint8_t *bam_head; uint64_t bam_head_len;   /* -Z, batch 0: the BAM header blocks */
 } job;
 
 typedef struct shared {
@@ -91,7 +99,7 @@ typedef struct shared {
     uint64_t next_take;                         /* next job a device thread takes */
     int producer_failed;
     /* run parameters */
-    int mode, single, var_length, with_cigar, sam, derive_md, pileup; uint32_t block_reads, flag_exclude;
+    int mode, single, var_length, with_cigar, sam, bam, derive_md, pileup; uint32_t block_reads, flag_exclude;
     const cbch_fasta *fa; int fa_ready;
     const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
     double t_gpu_ready;
@@ -167,19 +175,28 @@ static void *device_main(void *arg) {
                 D->call_s += now() - tq;
                 cbcg_stats st; cbcg_get_stats(ctx, &st); J->device_ms = st.ms_total;
             }
-        } else if (S->sam) {                                      /* SAM records; the writer adds the header */
+        } else if (S->sam || S->bam) {                            /* SAM / BAM records; the writer adds the header (and BAM's EOF) */
             uint64_t nb = 1, n_reads = 0, pb = 0, cap = 0, n = 0;
-            if (S->n_regions) {
+            if (S->bam && J->index == 0) {                        /* host only: the header needs the reference's lengths */
+                rc = cbcg_bam_header(ctx, J->in, J->in_len, J->legacy, NULL, 0, &n);
+                if (rc == CBCG_ERR_CAPACITY) rc = (J->bam_head = (uint8_t *)malloc(n)) ? cbcg_bam_header(ctx, J->in, J->in_len, J->legacy, J->bam_head, n, &n) : CBCG_ERR_NOMEM;
+                if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "BAM header: %s", ctx ? cbcg_last_error(ctx) : "no context"); nb = 0; }
+                J->bam_head_len = n; n = 0;
+            }
+            if (S->n_regions && !J->rc) {
                 rc = cbcg_region_plan(J->in, J->in_len, J->legacy, S->regions, S->n_regions, &nb, &n_reads, &pb, &cap);
                 if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "region plan: %s", cbcg_strerror(rc)); nb = 0; }
             }
-            if (nb) {                                             /* a batch that no region touches costs no device call */
+            if (nb && !J->rc) {                                   /* a batch that no region touches costs no device call */
                 if (J->legacy || cbcg_decoded_size(J->in, J->in_len, &n_reads, &cap) != CBCG_OK) cap = 1u << 20;
-                cap = 2 * cap + (1u << 16);                       /* SAM lines: about SEQ + 60 bytes */
+                cap = 2 * cap + (1u << 16);                       /* SAM lines: about SEQ + 60 bytes; BAM records fewer */
                 tq = now();
                 J->out = (uint8_t *)malloc(cap);
-                rc = J->out ? cbcg_decode_sam(ctx, J->in, J->in_len, J->legacy, S->with_cigar ? J->cig_in : NULL, S->with_cigar ? J->cig_in_len : 0,
-                                              S->n_regions ? S->regions : NULL, S->n_regions, 0u, J->out, cap, &n, NULL, 0, &n_reads) : CBCG_ERR_NOMEM;
+                const uint8_t *sec = S->with_cigar ? J->cig_in : NULL; const uint64_t sec_len = S->with_cigar ? J->cig_in_len : 0;
+                const cbcg_region *reg = S->n_regions ? S->regions : NULL;
+                rc = !J->out ? CBCG_ERR_NOMEM
+                   : S->bam ? cbcg_decode_bam(ctx, J->in, J->in_len, J->legacy, sec, sec_len, reg, S->n_regions, 0u, J->out, cap, &n, NULL, 0, &n_reads)
+                            : cbcg_decode_sam(ctx, J->in, J->in_len, J->legacy, sec, sec_len, reg, S->n_regions, 0u, J->out, cap, &n, NULL, 0, &n_reads);
                 if (rc == CBCG_ERR_CAPACITY && n > cap) { free(J->out); J->out = (uint8_t *)malloc(n); rc = J->out ? cbcg_fetch_decoded(ctx, J->out, n, &n) : CBCG_ERR_NOMEM; }
                 if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "%s", ctx ? cbcg_last_error(ctx) : "no context"); }
                 J->out_len = n; J->n_reads = n_reads;
@@ -410,7 +427,7 @@ static int parse_devices(const char *s, int *dev) {
 }
 
 int main(int argc, char **argv) {
-    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, derive_md = 0, pileup = 0, have_mask = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
+    int mode = 0, single = 0, var_length = 0, with_cigar = 0, sam = 0, bam = 0, derive_md = 0, pileup = 0, have_mask = 0, n_dev = 1, dev[MAX_DEV] = { 0 };
     uint32_t flag_exclude = CBCG_PILEUP_FLAG_EXCLUDE;
     uint32_t block_reads = CBCG_BLOCK_AUTO;
     uint64_t batch_mb = 2048;
@@ -424,6 +441,7 @@ int main(int argc, char **argv) {
         else if (!strcmp(a, "-l")) var_length = 1;
         else if (!strcmp(a, "-C")) with_cigar = 1;
         else if (!strcmp(a, "-S")) sam = 1;
+        else if (!strcmp(a, "-Z")) bam = 1;
         else if (!strcmp(a, "-M")) derive_md = 1;
         else if (!strcmp(a, "-P")) pileup = 1;
         else if (!strcmp(a, "-F") && i + 1 < argc) {
@@ -456,12 +474,14 @@ int main(int argc, char **argv) {
     if (!mode || nfiles != 3) { fprintf(stderr, "Missing required filenames\n"); return usage(); }
     if (n_regions && mode != 'd') { fprintf(stderr, "cbc: -r selects reads to decode: it goes with -d\n"); return usage(); }
     if (sam && mode != 'd') { fprintf(stderr, "cbc: -S writes SAM: it goes with -d\n"); return usage(); }
+    if (bam && mode != 'd') { fprintf(stderr, "cbc: -Z writes BAM: it goes with -d\n"); return usage(); }
+    if (bam && (sam || pileup)) { fprintf(stderr, "cbc: -Z writes BAM; -S and -P are other outputs: choose one\n"); return usage(); }
     if (derive_md && mode != 'c') { fprintf(stderr, "cbc: -M derives MD for encoding: it goes with -c\n"); return usage(); }
     if (pileup && mode != 'd') { fprintf(stderr, "cbc: -P writes a pileup of a container: it goes with -d\n"); return usage(); }
     if (pileup && sam) { fprintf(stderr, "cbc: -P and -S are two outputs: choose one\n"); return usage(); }
     if (pileup && !n_regions) { fprintf(stderr, "cbc: -P needs at least one -r region\n"); return usage(); }
     if (have_mask && !pileup) { fprintf(stderr, "cbc: -F selects the reads a pileup counts: it goes with -P\n"); return usage(); }
-    if (n_regions && with_cigar && !sam && !pileup) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
+    if (n_regions && with_cigar && !sam && !bam && !pileup) { fprintf(stderr, "cbc: -r cannot be combined with -C: CIGAR recovery rebuilds every read of a batch\n"); return 2; }
     if (!single && block_reads == 0) block_reads = CBCG_BLOCK_AUTO;
     if (batch_mb < 1) batch_mb = 1;
 
@@ -469,7 +489,7 @@ int main(int argc, char **argv) {
     shared S; memset(&S, 0, sizeof S);
     pthread_mutex_init(&S.mu, NULL); pthread_cond_init(&S.cv, NULL);
     S.mode = mode; S.single = single; S.var_length = var_length; S.block_reads = block_reads; S.with_cigar = with_cigar;
-    S.regions = regions; S.n_regions = n_regions; S.sam = sam; S.derive_md = derive_md; S.pileup = pileup; S.flag_exclude = flag_exclude;
+    S.regions = regions; S.n_regions = n_regions; S.sam = sam; S.bam = bam; S.derive_md = derive_md; S.pileup = pileup; S.flag_exclude = flag_exclude;
     devthread D[MAX_DEV]; memset(D, 0, sizeof D);
 
     /* ---- the input, cut into jobs (before the device threads start: they index S.jobs) */
@@ -574,12 +594,14 @@ int main(int argc, char **argv) {
         if (!J) { fprintf(stderr, "cbc: %s\n", IA.err[0] ? IA.err : "ingest failed"); status = 1; break; }
         if (J->rc) { fprintf(stderr, "cbc: %s\n", J->err); status = 1; break; }
         if (sam && k == 0 && write_sam_header(fo, J, &fa)) { fprintf(stderr, "cbc: cannot write the SAM header of %s\n", files[0]); status = 1; break; }
+        if (bam && k == 0 && fwrite(J->bam_head, 1, J->bam_head_len, fo) != J->bam_head_len) { fprintf(stderr, "cbc: cannot write %s\n", files[1]); status = 1; break; }
+        if (bam && k > 0 && sam_table_differs(S.jobs[0], J)) { fprintf(stderr, "cbc: batch %llu names other chromosomes than batch 0: one BAM header cannot describe both\n", (unsigned long long)k); status = 1; break; }
         if (sam && k > 0 && sam_table_differs(S.jobs[0], J)) { fprintf(stderr, "cbc: batch %llu names other chromosomes than batch 0: one SAM header cannot describe both\n", (unsigned long long)k); status = 1; break; }
         if (pileup) {
             if (J->out_len && (J->out_len != pu_rows * CBCG_PU_COLS * 4 || pileup_add(pu_sum, (const uint32_t *)J->out, pu_rows))) {
                 fprintf(stderr, "cbc: batch %llu: pileup rows disagree with the reference\n", (unsigned long long)k); status = 1; break;
             }
-        } else if (with_cigar && mode == 'd' && !sam) {                         /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
+        } else if (with_cigar && mode == 'd' && !sam && !bam) {                 /* "CIGAR<TAB>SEQ" per read: the two texts hold one line per read each */
             const uint8_t *c = J->cig, *ce = J->cig + J->cig_len, *q = J->out, *qe = J->out + J->out_len;
             while (c < ce && q < qe) {
                 const uint8_t *cn = (const uint8_t *)memchr(c, '\n', (size_t)(ce - c)), *qn = (const uint8_t *)memchr(q, '\n', (size_t)(qe - q));
@@ -602,6 +624,8 @@ int main(int argc, char **argv) {
         pthread_cond_broadcast(&S.cv);
         pthread_mutex_unlock(&S.mu);
     }
+    static const uint8_t bgzf_eof[28] = { 0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0 };
+    if (bam && !status && fwrite(bgzf_eof, 1, sizeof bgzf_eof, fo) != sizeof bgzf_eof) { fprintf(stderr, "cbc: cannot write %s\n", files[1]); status = 1; }
     if (pileup && !status && pileup_write(fo, pu_sum, &fa, regions, n_regions, pu_chr)) { fprintf(stderr, "cbc: cannot write %s\n", files[1]); status = 1; }
     free(pu_sum); free(pu_chr);
     if (status) { pthread_mutex_lock(&S.mu); S.producer_failed = 1; S.next_take = S.n_jobs; pthread_cond_broadcast(&S.cv); pthread_mutex_unlock(&S.mu); }
@@ -632,7 +656,7 @@ int main(int argc, char **argv) {
     }
     if (getenv("CBC_TRACE")) for (int d = 0; d < n_dev; d++)
         fprintf(stderr, "[cbc] device %d: context %.3f s, reference upload %.3f s, coding calls %.3f s; writer done at %.3f s\n", dev[d], D[d].create_s, D[d].setref_s, D[d].call_s, t2 - t0);
-    for (uint64_t k = 0; k < S.n_jobs; k++) { free(S.jobs[k]->out); free(S.jobs[k]->cig); free(S.jobs[k]); }
+    for (uint64_t k = 0; k < S.n_jobs; k++) { free(S.jobs[k]->out); free(S.jobs[k]->cig); free(S.jobs[k]->bam_head); free(S.jobs[k]); }
     free(S.jobs); free(cut); free(cig_file); free(shard_off); free(shard_len);
     for (uint32_t k = 0; k < n_regions; k++) free((void *)regions[k].name);
     free(regions);

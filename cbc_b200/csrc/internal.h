@@ -186,3 +186,18 @@ int launch_pileup(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *c
                   uint32_t max_len, uint32_t fixed_len, uint32_t *acc, uint64_t n_pad, uint64_t n_slots, const PileupReg *reg, uint32_t n_reg,
                   uint32_t *rows, uint64_t n_rows, uint64_t *tile_desc, uint32_t *ticket, uint64_t *n_counted, unsigned long long *err,
                   cudaStream_t st);
+/* k9_bam.cu: BAM records in BGZF blocks. launch_bam_records: K6's inputs (ref_id: per genome ordinal, its index in the
+   header's name list, -1 for none) -> the uncompressed record stream (stream_cap bytes), rec_off (n_reads + 1 offsets: each
+   record's, then the stream's size) and block_first (the first record of each BGZF block, then n_reads; <= stream_cap /
+   K9_BLOCK_CUT + 2 entries); totals[0] receives the stream's size and totals[1] the block count. tile_desc: 2 x
+   bam_num_tiles(n_reads) words. launch_bgzf: those blocks -> out, back to back; *total_bytes receives their size.
+   tile_desc: n_blocks words. */
+#define K9_BLOCK_CUT 49152u
+uint64_t bam_num_tiles(uint64_t n_reads);
+int launch_bam_records(uint64_t n_reads, const cbcg_read_rec *recs, const uint32_t *chr, const uint16_t *edits, const DevGenome &g,
+                       const int32_t *ref_id, const uint8_t *seq_text, uint32_t max_len, uint32_t fixed_len, const uint64_t *ids,
+                       const uint8_t *cls, const uint64_t *exc_read, const uint64_t *exc_off, const uint8_t *exc_text, uint64_t n_exc,
+                       uint8_t *stream, uint64_t stream_cap, uint64_t *rec_off, uint32_t *block_first, uint64_t *tile_desc, uint32_t *ticket,
+                       uint64_t *totals, unsigned long long *err, cudaStream_t st);
+int launch_bgzf(const uint8_t *stream, const uint64_t *rec_off, const uint32_t *block_first, uint32_t n_blocks, uint8_t *out,
+                uint64_t *tile_desc, uint32_t *ticket, uint64_t *total_bytes, unsigned long long *err, cudaStream_t st);

@@ -19,6 +19,7 @@ template <bool W> struct K6Out {
         n += d;
     }
     __device__ __forceinline__ void str(const char *s) { for (; *s; s++) put((uint8_t)*s); }
+    __device__ __forceinline__ void cig(uint32_t cnt, uint32_t op) { num(cnt); put(op); }   /* one CIGAR operation as text */
 };
 
 /* Verbatim CIGAR: true when its read length is len, it deletes at most K6_MAX_DEL bases (what the host's size bound and the

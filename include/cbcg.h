@@ -275,6 +275,34 @@ int cbcg_decode_sam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legac
                     uint8_t *out, uint64_t out_cap, uint64_t *out_len,
                     uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
 
+/* ---- BAM output (DESIGN.md 5f): cbcg_decode_sam's reads, in the same order and with the same ordinals (the same selection,
+ * overlap rule, decode, CIGAR and MD / NM rule), as BAM records (SAMv1 4.2) in BGZF blocks (SAMv1 4.1). Read back by any
+ * BAM reader they give cbcg_decode_sam's lines, SEQ through the 4-bit code.
+ *   header (CBCG_BAM_HEADER): "BAM\1", l_text, cbcg_decode_sam's header text (@HD, @SQ SN LN per name), n_ref, then
+ *     (l_name, name\0, l_ref) per name of the container's table (legacy stream: of the loaded reference), in BGZF blocks of
+ *     stored deflate blocks of 65 280 bytes (the last one shorter). Every length comes from the loaded reference: a table
+ *     name it lacks is CBCG_ERR_NO_REFERENCE (SAM omits LN instead), a length above 2^31 - 1 CBCG_ERR_INPUT.
+ *   record: refID the read's index in that name list, pos POS - 1, read name "*", MAPQ 255, bin reg2bin(pos, pos + the
+ *     CIGAR's M D N = X span, or pos + 1), FLAG, the CIGAR as u32 len << 4 | op (MIDNSHP=X), SEQ in the 4-bit code
+ *     =ACMGRSVTWYHKDBN (any other byte: 15, N), QUAL l_seq x 0xff, no mate (-1, -1, 0), then NM (type C, S above 255)
+ *     and MD (type Z). A record above 8 192 bytes (only a pathological verbatim CIGAR) is CBCG_ERR_FORMAT.
+ *   blocks: whole records; record i > 0 of the call opens a block when floor(U_i / 49152) != floor(U_{i-1} / 49152), U_i
+ *     the record bytes before it. Each block is one fixed-Huffman deflate block: every byte a literal except QUAL, which is
+ *     one literal 0xff, then one match (length l_seq - 1, distance 1) when l_seq - 1 >= 3. The bytes are deterministic.
+ *   EOF (CBCG_BAM_EOF): the spec's 28-byte empty block. A call's blocks stand alone, so the output of several calls
+ *     concatenates into one file: the header once, the record blocks of every call, the EOF once.
+ * Errors, capacity (cbcg_fetch_decoded then returns the BAM bytes), read ids, statistics and state as cbcg_decode_sam; K9's
+ * time is part of ms_reconstruct, ms_k3 is K3's alone. cbcg_bam_header: the header blocks alone, on the host (no device
+ * work); it needs the loaded reference's lengths. */
+#define CBCG_BAM_HEADER 1u
+#define CBCG_BAM_EOF    2u
+int cbcg_bam_header(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+int cbcg_decode_bam(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
+                    const uint8_t *section, uint64_t section_len,
+                    const cbcg_region *regions, uint32_t n_regions, uint32_t flags,
+                    uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                    uint64_t *read_ids, uint64_t ids_cap, uint64_t *n_reads);
+
 /* ---- pileup (DESIGN.md, "Pileup"): per reference position of each region, u32[CBCG_PU_COLS] = A C G T N DEL INS REF.
  *   reads: the ones cbcg_decode_sam(section, regions) returns (the same selection, overlap rule and decode), minus those
  *     with FLAG & flag_exclude. Each is aligned by the CIGAR of its SAM line: the section's verbatim text for class 4, else
