@@ -43,13 +43,26 @@ EXPORTS = ["cbcg_create", "cbcg_destroy", "cbcg_strerror", "cbcg_last_error", "c
            "cbcg_fetch_container", "cbcg_fetch_decoded", "cbcg_fetch_index", "cbcg_mark", "cbcg_elapsed_ms",
            "cbcg_encode_compact", "cbcg_batch_upload_compact", "cbcg_cigar_bound", "cbcg_cigar_pack", "cbcg_cigar_unpack",
            "cbcg_region_plan", "cbcg_decode_region", "cbcg_sam_header", "cbcg_decode_sam", "cbcg_derive_md",
-           "cbcg_pileup", "cbcg_bam_header", "cbcg_decode_bam"]
+           "cbcg_pileup", "cbcg_bam_header", "cbcg_decode_bam", "cbcg_bgzf_inflate", "cbcg_bam_open", "cbcg_batch_upload_bam",
+           "cbcg_cigar_pack_resident"]
 
 
 UINT64_MAX = (1 << 64) - 1
 PILEUP_COLUMNS = ("A", "C", "G", "T", "N", "DEL", "INS", "REF")      # CBCG_PU_A .. CBCG_PU_REF
 PILEUP_FLAG_EXCLUDE = 0x704                                          # UNMAP | SECONDARY | QCFAIL | DUP
 BAM_HEADER, BAM_EOF = 1, 2                                           # CBCG_BAM_HEADER, CBCG_BAM_EOF
+BAM_DERIVE_MD, BAM_LAST = 1, 2                                       # CBCG_BAM_DERIVE_MD, CBCG_BAM_LAST
+BLOCK_AUTO = 0xFFFFFFFF                                              # CBCG_BLOCK_AUTO
+
+
+class BamInfo(C.Structure):
+    """Mirror of ``cbcg_bam_info`` (include/cbcg.h)."""
+    _fields_ = [("n_records", C.c_uint64), ("n_unmapped", C.c_uint64), ("n_reads", C.c_uint64), ("len_first", C.c_uint32),
+                ("len_second", C.c_uint32), ("max_len", C.c_uint32), ("min_len", C.c_uint32), ("inflated_bytes", C.c_uint64),
+                ("tail_len", C.c_uint64)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
 
 
 class Region(C.Structure):
@@ -171,6 +184,10 @@ def load_library():
         lib.cbcg_pileup.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, P(u64)]
         lib.cbcg_bam_header.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(u64)]
         lib.cbcg_decode_bam.argtypes = [vp, vp, u64, C.c_int, vp, u64, P(Region), u32, u32, vp, u64, P(u64), vp, u64, P(u64)]
+        lib.cbcg_bgzf_inflate.argtypes = [vp, vp, u64, vp, u64, P(u64)]
+        lib.cbcg_bam_open.argtypes = [vp, vp, u64, P(u64), vp, u64, P(u64)]
+        lib.cbcg_batch_upload_bam.argtypes = [vp, vp, u64, vp, u64, u32, P(BamInfo), vp, u64]
+        lib.cbcg_cigar_pack_resident.argtypes = [vp, vp, u64, P(u64)]
         lib.cbcg_mark.argtypes = [vp, C.c_int]
         lib.cbcg_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, P(C.c_float)]
         _LIB = lib
@@ -497,6 +514,68 @@ class Codec:
         n = C.c_uint64(0)
         self._check(self.lib.cbcg_cigar_pack(self.h, C.byref(cb), out.ctypes.data, out.nbytes, C.byref(n)))
         return out[:n.value].tobytes()
+
+    def cigar_pack_resident(self) -> bytes:
+        """``cigar_pack`` of the resident batch, without an upload (the batch of ``upload_bam`` exists only on the device)."""
+        n = C.c_uint64(0)
+        rc = self.lib.cbcg_cigar_pack_resident(self.h, None, 0, C.byref(n))
+        if rc != -5:
+            self._check(rc)
+        out = np.empty(max(n.value, 24), np.uint8)
+        self._check(self.lib.cbcg_cigar_pack_resident(self.h, out.ctypes.data, out.nbytes, C.byref(n)))
+        return out[:n.value].tobytes()
+
+    # ---- BAM input (include/cbcg.h, DESIGN.md 5g)
+    def bgzf_inflate(self, data: bytes) -> bytes:
+        """Whole BGZF members -> their inflated concatenation, inflated on the GPU."""
+        src = np.frombuffer(data, np.uint8)
+        n = C.c_uint64(0)
+        rc = self.lib.cbcg_bgzf_inflate(self.h, src.ctypes.data, src.nbytes, None, 0, C.byref(n))
+        if rc != -5:
+            self._check(rc)
+        out = np.empty(max(n.value, 1), np.uint8)
+        self._check(self.lib.cbcg_bgzf_inflate(self.h, src.ctypes.data, src.nbytes, out.ctypes.data, out.nbytes, C.byref(n)))
+        return out[:n.value].tobytes()
+
+    def bam_open(self, data: bytes) -> Tuple[int, bytes]:
+        """Reads the BAM header from the start of ``data`` (the whole file will do): (bytes of the members it consumed, the
+        record bytes after the header in the last of them). Needs ``set_reference``."""
+        src = np.frombuffer(data, np.uint8)
+        used, n = C.c_uint64(0), C.c_uint64(0)
+        tail = np.empty(1 << 17, np.uint8)
+        self._check(self.lib.cbcg_bam_open(self.h, src.ctypes.data, src.nbytes, C.byref(used), tail.ctypes.data, tail.nbytes, C.byref(n)))
+        return used.value, tail[:n.value].tobytes()
+
+    def upload_bam(self, data: bytes, carry: bytes = b"", derive_md: bool = False, last: bool = True) -> Tuple[dict, bytes]:
+        """Whole BGZF members after ``carry`` -> the resident batch: (cbcg_bam_info as a dict, the bytes after the last whole
+        record, the next call's carry)."""
+        src = np.frombuffer(data, np.uint8)
+        car = np.frombuffer(carry, np.uint8)
+        info = BamInfo()
+        flags = (BAM_DERIVE_MD if derive_md else 0) | (BAM_LAST if last else 0)
+        cap = 1 << 17
+        while True:
+            tail = np.empty(cap, np.uint8)
+            rc = self.lib.cbcg_batch_upload_bam(self.h, car.ctypes.data if car.size else None, car.size,
+                                                src.ctypes.data if src.size else None, src.size, flags, C.byref(info),
+                                                tail.ctypes.data, tail.nbytes)
+            if rc == -5 and info.tail_len > cap:
+                cap = int(info.tail_len)
+                continue
+            self._check(rc)
+            return info.as_dict(), tail[:info.tail_len].tobytes()
+
+    def compress_bam(self, data: bytes, read_len_header: Optional[int] = None, block_reads: int = BLOCK_AUTO, gen_mode: int = 1,
+                     substreams: int = 1, derive_md: bool = False, var_length: bool = False) -> Tuple[bytes, dict]:
+        """A whole BAM file -> (container, cbcg_bam_info dict): ``bam_open``, one ``upload_bam``, ``encode_resident``,
+        ``fetch_container``. read_len_header None: get_read_length's answer, the second record's l_seq (var_length: the
+        longest read)."""
+        used, tail = self.bam_open(data)
+        info, _ = self.upload_bam(data[used:], carry=tail, derive_md=derive_md, last=True)
+        if read_len_header is None:
+            read_len_header = info["max_len"] if var_length else (info["len_second"] if info["n_records"] >= 2 else info["len_first"])
+        self.encode_resident(read_len_header, block_reads, gen_mode, substreams)
+        return self.fetch_container().tobytes(), info
 
     def cigar_unpack(self, data: bytes, section: Optional[bytes], legacy: bool = False) -> Tuple[bytes, int]:
         """(CIGAR + '\\n' per read in read order, read count) of a container and its side section (None: the implied CIGARs)."""

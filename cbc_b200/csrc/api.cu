@@ -44,6 +44,8 @@ struct Words {
     uint64_t n_selected;                      /* region decode: reads K5 kept */
     uint64_t md_chain[2];                     /* MD derivation (K7): MD bytes of the batch ([0]), or so far, ping-pong between chunk launches */
     uint64_t pu_reads;                        /* pileup (K8): reads counted */
+    uint64_t bam[9];                          /* BAM input (K10): records, tail start, repairs, reads, SEQ / CIGAR / MD bytes, run starts / ends */
+    uint32_t bam_len[4];                      /*   l_seq of records 0 and 1, 0xffffffff - shortest, longest read */
 };
 
 struct cbcg_ctx {
@@ -87,6 +89,9 @@ struct cbcg_ctx {
     DevBuf sam_aux, sam_out;                   /* SAM output (k6_sam.cu): name lengths, CIGAR classes and texts; the text */
     DevBuf bam_rec, bam_idx;                   /* BAM output (k9_bam.cu): the uncompressed record stream; record offsets and block starts */
     DevBuf pu_aux, pu_acc, pu_rows;            /* pileup (k8_pileup.cu): intervals, regions, CIGAR classes and texts; accumulators; rows */
+    DevBuf bi_in, bi_mem, bi_stream, bi_seg, bi_work, bi_rec, bi_map, bi_src, bi_runs;   /* BAM input (k10_bam_in.cu): compressed bytes, members,
+                                                  inflated stream, segments and their chain words, record starts, refID map, each read's
+                                                  record and MD, chromosome runs */
     DevBuf snap_a, snap_b, fin;                /* generation snapshots and per-block final states (gen_mode 1) */
     std::vector<std::pair<uint32_t, uint32_t>> gens;   /* (first block, block count) per generation of the last cut */
     uint32_t layout = 1;                       /* the call in progress: 1 = one stream per block, 4 = four substreams, 0 = four in the narrow early generations */
@@ -102,6 +107,10 @@ struct cbcg_ctx {
     bool batch_indel_heavy = false;           /* CIGAR text per read well beyond "<len>M": most reads carry indels / clips (picks the model kernel's edit walk) */
     uint64_t enc_n_reads = 0, enc_n_edits = 0, enc_n_blocks = 0, enc_payload_bytes = 0;
     std::vector<uint8_t> enc_head;             /* container header + index */
+
+    /* BAM input: the refID -> genome ordinal map of the header cbcg_bam_open read (-1: a name the reference lacks) */
+    bool bam_opened = false;
+    std::vector<int32_t> bam_map;
 
     /* result of the last decode */
     bool have_decoded = false;
@@ -216,7 +225,8 @@ extern "C" void cbcg_destroy(cbcg_ctx *ctx) {
     if (ctx->h_tile) cudaFreeHost(ctx->h_tile);
     for (DevBuf *d : { &ctx->c_seq2, &ctx->c_cl, &ctx->c_ml, &ctx->c_tile, &ctx->c_rfirst, &ctx->c_rchr, &ctx->c_er, &ctx->c_eb, &ctx->c_ec,
                        &ctx->reg, &ctx->sel_recs, &ctx->sel_chr, &ctx->sel_ids, &ctx->sam_aux, &ctx->sam_out, &ctx->bam_rec, &ctx->bam_idx,
-                       &ctx->pu_aux, &ctx->pu_acc, &ctx->pu_rows }) free_buf(*d);
+                       &ctx->pu_aux, &ctx->pu_acc, &ctx->pu_rows, &ctx->bi_in, &ctx->bi_mem, &ctx->bi_stream, &ctx->bi_seg, &ctx->bi_work,
+                       &ctx->bi_rec, &ctx->bi_map, &ctx->bi_src, &ctx->bi_runs }) free_buf(*d);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->mark) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->kev) if (e) cudaEventDestroy(e);
@@ -275,6 +285,7 @@ extern "C" int cbcg_set_reference(cbcg_ctx *ctx, uint32_t n_chr, const char *con
     if (!ctx || !n_chr || !bases || !len || n_chr > MAX_CHR) return fail(ctx, CBCG_ERR_ARG, "cbcg_set_reference: bad argument");
     CU(cudaSetDevice(ctx->device));
     ctx->names.clear(); ctx->h_off.clear(); ctx->h_len.clear();
+    ctx->bam_opened = false; ctx->bam_map.clear();          /* the map names this reference's ordinals: cbcg_bam_open again */
     uint64_t total = 0;
     for (uint32_t c = 0; c < n_chr; c++) {
         if (!bases[c]) return fail(ctx, CBCG_ERR_ARG, "cbcg_set_reference: NULL record %u", c);
@@ -369,13 +380,16 @@ static int batch_copy_range(cbcg_ctx *ctx, const cbcg_batch *b, uint64_t r0, uin
 }
 /* K1's reference window (DevBatch.ref_cap): bytes of reference that 128 position-adjacent reads span at this batch's
  * coverage, twice over, plus a read. From the first and last POS of every chromosome run. */
+static uint32_t ref_window_from_span(uint64_t span, uint64_t n, uint32_t max_len) {
+    const double per_read = (double)span / (double)n;
+    const double want = per_read * 128.0 * 2.0 + max_len + 64.0;
+    return want > 1e9 ? 0u : (uint32_t)want;
+}
 static uint32_t ref_window_estimate(const cbcg_ctx *ctx, const uint32_t *pos, uint64_t n, uint32_t max_len) {
     if (!n || !pos) return 0u;
     uint64_t span = 0;
     for (const ChrRun &r : ctx->runs) if (r.n) { const uint32_t a = pos[r.first], z = pos[r.first + r.n - 1]; if (z > a) span += z - a; }
-    const double per_read = (double)span / (double)n;
-    const double want = per_read * 128.0 * 2.0 + max_len + 64.0;
-    return want > 1e9 ? 0u : (uint32_t)want;
+    return ref_window_from_span(span, n, max_len);
 }
 /* Host scan of the batch: chromosome runs (blocks never span chromosomes), longest and shortest read. */
 static int batch_scan(cbcg_ctx *ctx, const cbcg_batch *b) {
@@ -2162,21 +2176,24 @@ extern "C" uint64_t cbcg_cigar_bound(const cbcg_batch *b) {
     if (!b) return 0;
     return 24u + b->n_reads * 16u + (b->cigar_off && b->n_reads ? b->cigar_off[b->n_reads] : 0u);
 }
-extern "C" int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
-    if (!ctx || !batch || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_cigar_pack: bad argument");
-    *out_len = 0;
-    TRY(cbcg_batch_upload(ctx, batch));
+/* K1 and K4's classes over the resident batch */
+static int cigar_classes(cbcg_ctx *ctx, std::vector<uint8_t> &cls) {
     const uint64_t n = ctx->db.n_reads;
-    std::vector<uint8_t> cls(n);
-    if (n) {
-        TRY(run_extract(ctx));
-        TRY(ensure(ctx, ctx->cig_cls, n + 64));
-        if (launch_cigar_class(n, ctx->recs.as<cbcg_read_rec>(), ctx->edits.as<uint16_t>(), ctx->db.cigar_off, ctx->db.cigar,
-                               ctx->cig_cls.as<uint8_t>(), ctx->st))
-            return fail(ctx, CBCG_ERR_CUDA, "CIGAR class launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-        CU(cudaMemcpyAsync(cls.data(), ctx->cig_cls.p, n, cudaMemcpyDeviceToHost, ctx->st));
-        CU(cudaStreamSynchronize(ctx->st));
-    }
+    cls.assign(n, 0);
+    if (!n) return 0;
+    TRY(run_extract(ctx));
+    TRY(ensure(ctx, ctx->cig_cls, n + 64));
+    if (launch_cigar_class(n, ctx->recs.as<cbcg_read_rec>(), ctx->edits.as<uint16_t>(), ctx->db.cigar_off, ctx->db.cigar,
+                           ctx->cig_cls.as<uint8_t>(), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "CIGAR class launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    CU(cudaMemcpyAsync(cls.data(), ctx->cig_cls.p, n, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    return 0;
+}
+/* the section of those classes; cigar_off / cigar: the batch's CIGAR text on the host */
+static int cigar_section(cbcg_ctx *ctx, const std::vector<uint8_t> &cls, const uint64_t *cigar_off, const uint8_t *cigar, uint8_t *out,
+                         uint64_t out_cap, uint64_t *out_len) {
+    const uint64_t n = cls.size();
     std::vector<uint8_t> sec(24);
     uint64_t entries = 0, prev = 0;
     for (uint64_t r = 0; r < n; r++) {
@@ -2184,9 +2201,9 @@ extern "C" int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *
         put_varint(sec, r - prev); prev = r;
         sec.push_back(cls[r]);
         if (cls[r] >= 4u) {
-            const uint64_t a = batch->cigar_off[r], l = batch->cigar_off[r + 1] - a;
+            const uint64_t a = cigar_off[r], l = cigar_off[r + 1] - a;
             put_varint(sec, l);
-            sec.insert(sec.end(), batch->cigar + a, batch->cigar + a + l);
+            sec.insert(sec.end(), cigar + a, cigar + a + l);
         }
         entries++;
     }
@@ -2196,6 +2213,38 @@ extern "C" int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *
     if (!out || sec.size() > out_cap) return fail(ctx, CBCG_ERR_CAPACITY, "CIGAR section is %llu bytes, room for %llu", (unsigned long long)sec.size(), (unsigned long long)out_cap);
     memcpy(out, sec.data(), sec.size());
     return CBCG_OK;
+}
+extern "C" int cbcg_cigar_pack(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!ctx || !batch || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_cigar_pack: bad argument");
+    *out_len = 0;
+    TRY(cbcg_batch_upload(ctx, batch));
+    std::vector<uint8_t> cls;
+    TRY(cigar_classes(ctx, cls));
+    return cigar_section(ctx, cls, batch->cigar_off, batch->cigar, out, out_cap, out_len);
+}
+/* The same for the resident batch, whose CIGAR text may exist only on the device (a BAM upload): the texts of verbatim
+   reads come back from there. */
+extern "C" int cbcg_cigar_pack_resident(cbcg_ctx *ctx, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!ctx || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_cigar_pack_resident: bad argument");
+    *out_len = 0;
+    if (!ctx->have_batch) return fail(ctx, CBCG_ERR_ARG, "no resident batch");
+    CU(cudaSetDevice(ctx->device));
+    std::vector<uint8_t> cls;
+    TRY(cigar_classes(ctx, cls));
+    const uint64_t n = cls.size();
+    std::vector<uint64_t> off;
+    std::vector<uint8_t> text;
+    if (std::any_of(cls.begin(), cls.end(), [](uint8_t c) { return c >= 4u; })) {
+        off.resize(n + 1);
+        CU(cudaMemcpyAsync(off.data(), ctx->db.cigar_off, (n + 1) * 8, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        text.resize(off[n] - off[0] + 1);
+        if (off[n] > off[0]) CU(cudaMemcpyAsync(text.data(), ctx->db.cigar + off[0], off[n] - off[0], cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        const uint64_t base = off[0];
+        for (uint64_t &o : off) o -= base;
+    }
+    return cigar_section(ctx, cls, off.data(), text.data(), out, out_cap, out_len);
 }
 /* A CIGAR side section (layout above cbcg_cigar_bound) for a container of n reads -> a class per read and the class-4 texts. */
 static int parse_cigar_section(cbcg_ctx *ctx, const uint8_t *section, uint64_t section_len, uint64_t n, std::vector<uint8_t> &cls,
@@ -2774,5 +2823,260 @@ extern "C" int cbcg_reconstruct(cbcg_ctx *ctx, uint64_t n_reads, const cbcg_read
     CU(cudaMemcpyAsync(seq_out, ctx->seq_out.p, bytes, cudaMemcpyDeviceToHost, ctx->st));
     CU(cudaStreamSynchronize(ctx->st));
     ctx->stats.n_reads = n_reads; ctx->stats.n_edits = n_edits;
+    return CBCG_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------ BAM input (DESIGN.md 5g)
+ * BGZF members (SAMv1 4.1) are walked on the host, header to header, and inflated on the device (k10_bam_in.cu); the record
+ * stream they form is cut into records and parsed into the resident batch there, so the batch never exists on the host. */
+static uint32_t le16(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8; }
+static uint32_t le32(const uint8_t *p) { return le16(p) | le16(p + 2) << 16; }
+
+/* The members of in[0, in_len), at most max_members of them: a gzip member with FLG.FEXTRA and a 'BC' subfield holding
+ * BSIZE (the member's size - 1), ISIZE <= 65 536. Outputs follow each other from out_base. *used: the bytes walked. */
+static int bgzf_members(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, uint64_t out_base, std::vector<BgzfMember> &m,
+                        uint64_t *used, uint64_t *out_end, uint64_t max_members = ~0ull) {
+    m.clear();
+    uint64_t o = 0, out = out_base;
+    while (o < in_len && m.size() < max_members) {
+        const uint8_t *h = in + o;
+        if (in_len - o < 18) return fail(ctx, CBCG_ERR_FORMAT, "BGZF: member header truncated at byte %llu", (unsigned long long)o);
+        if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || h[3] != 4)
+            return fail(ctx, CBCG_ERR_FORMAT, "BGZF: no BGZF member header at byte %llu", (unsigned long long)o);
+        const uint32_t xlen = le16(h + 10);
+        if (12ull + xlen > in_len - o) return fail(ctx, CBCG_ERR_FORMAT, "BGZF: extra field past the input at byte %llu", (unsigned long long)o);
+        int64_t bsize = -1;
+        for (uint32_t x = 12; x + 4 <= 12 + xlen; x += 4 + le16(h + x + 2))
+            if (h[x] == 'B' && h[x + 1] == 'C' && le16(h + x + 2) == 2 && x + 6 <= 12 + xlen) bsize = le16(h + x + 4);
+        if (bsize < 0) return fail(ctx, CBCG_ERR_FORMAT, "BGZF: gzip member without the BC field at byte %llu", (unsigned long long)o);
+        const uint64_t total = (uint64_t)bsize + 1;
+        if (total < 12ull + xlen + 8 || total > in_len - o)
+            return fail(ctx, CBCG_ERR_FORMAT, "BGZF: BSIZE of the member at byte %llu runs past the input", (unsigned long long)o);
+        const uint32_t isize = le32(h + total - 4);
+        if (isize > 65536u) return fail(ctx, CBCG_ERR_FORMAT, "BGZF: ISIZE %u above 65536 at byte %llu", isize, (unsigned long long)o);
+        m.push_back(BgzfMember{ o + 12 + xlen, out, (uint32_t)(total - 12 - xlen - 8), isize, le32(h + total - 8), 0u });
+        out += isize; o += total;
+    }
+    *used = o; *out_end = out;
+    return 0;
+}
+/* carry (host) then the members of in, inflated into bi_stream[0, out_end); the stream keeps POOL_PAD bytes of slack */
+static int bgzf_inflate_into_stream(cbcg_ctx *ctx, const uint8_t *carry, uint64_t carry_len, const uint8_t *in, uint64_t in_bytes,
+                                    const std::vector<BgzfMember> &m, uint64_t out_end) {
+    TRY(ensure(ctx, ctx->bi_stream, out_end + POOL_PAD));
+    TRY(ensure(ctx, ctx->bi_in, in_bytes + 16));
+    TRY(ensure(ctx, ctx->bi_mem, (m.size() + 1) * sizeof(BgzfMember)));
+    if (carry_len) CU(cudaMemcpyAsync(ctx->bi_stream.p, carry, carry_len, cudaMemcpyHostToDevice, ctx->st));
+    if (in_bytes) CU(cudaMemcpyAsync(ctx->bi_in.p, in, in_bytes, cudaMemcpyHostToDevice, ctx->st));
+    if (!m.empty()) CU(cudaMemcpyAsync(ctx->bi_mem.p, m.data(), m.size() * sizeof(BgzfMember), cudaMemcpyHostToDevice, ctx->st));
+    CU(cudaMemsetAsync(ctx->bi_stream.as<uint8_t>() + out_end, 0, POOL_PAD, ctx->st));
+    TRY(reset_words(ctx));
+    if (launch_inflate(ctx->bi_in.as<uint8_t>(), ctx->bi_mem.as<BgzfMember>(), (uint32_t)m.size(), ctx->bi_stream.as<uint8_t>(),
+                       wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "inflate launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    ctx->stats.kernel_launches++;
+    TRY(fetch_words(ctx));                                   /* synchronises: the caller's buffers may go */
+    return device_error(ctx, "BGZF inflate");
+}
+
+extern "C" int cbcg_bgzf_inflate(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+    if (!ctx || (!in && in_len) || !out_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_bgzf_inflate: bad argument");
+    *out_len = 0;
+    std::vector<BgzfMember> m;
+    uint64_t used = 0, total = 0;
+    TRY(bgzf_members(ctx, in, in_len, 0, m, &used, &total));
+    *out_len = total;
+    if (total > out_cap || (!out && total)) return fail(ctx, CBCG_ERR_CAPACITY, "inflated size %llu, room for %llu", (unsigned long long)total, (unsigned long long)out_cap);
+    CU(cudaSetDevice(ctx->device));
+    ctx->stats = cbcg_stats();
+    CU(cudaEventRecord(ctx->ev[0], ctx->st));
+    TRY(bgzf_inflate_into_stream(ctx, nullptr, 0, in, in_len, m, total));
+    if (total) CU(cudaMemcpyAsync(out, ctx->bi_stream.p, total, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaEventRecord(ctx->ev[1], ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    cudaEventElapsedTime(&ctx->stats.ms_total, ctx->ev[0], ctx->ev[1]);
+    ctx->stats.h2d_bytes = in_len; ctx->stats.d2h_bytes = total;
+    return CBCG_OK;
+}
+
+/* The BAM header (SAMv1 4.2: magic, l_text, text, n_ref, then l_name, name, l_ref per reference) at the start of h[0, n):
+ * 1 when it does not end inside n bytes, else 0 with its size and names, or CBCG_ERR_FORMAT. */
+static int parse_bam_header(cbcg_ctx *ctx, const uint8_t *h, uint64_t n, uint64_t *size, std::vector<std::string> &names) {
+    names.clear();
+    if (n < 4) return 1;
+    if (memcmp(h, "BAM\1", 4)) return fail(ctx, CBCG_ERR_FORMAT, "BAM: no BAM magic");
+    if (n < 8) return 1;
+    const int32_t l_text = (int32_t)le32(h + 4);
+    if (l_text < 0) return fail(ctx, CBCG_ERR_FORMAT, "BAM: negative l_text");
+    uint64_t o = 8 + (uint64_t)l_text;
+    if (o + 4 > n) return 1;
+    const int32_t n_ref = (int32_t)le32(h + o);
+    if (n_ref < 0) return fail(ctx, CBCG_ERR_FORMAT, "BAM: negative n_ref");
+    o += 4;
+    for (int32_t i = 0; i < n_ref; i++) {
+        if (o + 4 > n) return 1;
+        const int32_t l_name = (int32_t)le32(h + o);
+        if (l_name < 1) return fail(ctx, CBCG_ERR_FORMAT, "BAM: reference %d has l_name %d", i, l_name);
+        if (o + 4 + (uint64_t)l_name + 4 > n) return 1;
+        if (h[o + 4 + l_name - 1] != 0) return fail(ctx, CBCG_ERR_FORMAT, "BAM: reference name %d is not NUL-terminated", i);
+        names.emplace_back(reinterpret_cast<const char *>(h + o + 4), strnlen(reinterpret_cast<const char *>(h + o + 4), (size_t)l_name - 1));
+        o += 4 + (uint64_t)l_name + 4;
+    }
+    *size = o;
+    return 0;
+}
+
+extern "C" int cbcg_bam_open(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, uint64_t *used, uint8_t *tail, uint64_t tail_cap, uint64_t *tail_len) {
+    if (!ctx || (!in && in_len) || !used || !tail_len) return fail(ctx, CBCG_ERR_ARG, "cbcg_bam_open: bad argument");
+    *used = 0; *tail_len = 0;
+    ctx->bam_opened = false; ctx->bam_map.clear();
+    if (!ctx->dg.n_chr) return fail(ctx, CBCG_ERR_NO_REFERENCE, "cbcg_bam_open: cbcg_set_reference has not been called");
+    CU(cudaSetDevice(ctx->device));
+    ctx->stats = cbcg_stats();
+    std::vector<BgzfMember> m;
+    std::vector<uint8_t> head;
+    std::vector<std::string> names;
+    uint64_t walked = 0, total = 0, hsize = 0;
+    for (uint64_t k = 1;; k *= 4) {                          /* members from the start until the header ends inside them */
+        TRY(bgzf_members(ctx, in, in_len, 0, m, &walked, &total, k));
+        TRY(bgzf_inflate_into_stream(ctx, nullptr, 0, in, walked, m, total));
+        head.resize(total);
+        if (total) CU(cudaMemcpyAsync(head.data(), ctx->bi_stream.p, total, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        const int rc = parse_bam_header(ctx, head.data(), total, &hsize, names);
+        if (rc < 0) return rc;
+        if (rc == 0) break;
+        if (walked == in_len) return fail(ctx, CBCG_ERR_FORMAT, "BAM: the input ends inside the header");
+    }
+    size_t j = 0;                                            /* the member in which the header ends */
+    while (j + 1 < m.size() && m[j].out_off + m[j].isize < hsize) j++;
+    const uint64_t end = m.empty() ? 0 : m[j].out_off + m[j].isize;
+    *used = m.empty() ? 0 : m[j].in_off + m[j].in_len + 8;
+    *tail_len = end - hsize;
+    if (*tail_len > tail_cap || (!tail && *tail_len))
+        return fail(ctx, CBCG_ERR_CAPACITY, "BAM: %llu record bytes follow the header in its last member, room for %llu", (unsigned long long)*tail_len, (unsigned long long)tail_cap);
+    if (*tail_len) memcpy(tail, head.data() + hsize, *tail_len);
+    std::vector<int32_t> map(names.size(), -1);
+    for (size_t i = 0; i < names.size(); i++)
+        for (size_t c = 0; c < ctx->names.size(); c++) if (ctx->names[c] == names[i]) { map[i] = (int32_t)c; break; }
+    ctx->bam_map.swap(map);
+    ctx->bam_opened = true;
+    return CBCG_OK;
+}
+
+extern "C" int cbcg_batch_upload_bam(cbcg_ctx *ctx, const uint8_t *carry, uint64_t carry_len, const uint8_t *in, uint64_t in_len,
+                                     uint32_t flags, cbcg_bam_info *info, uint8_t *tail, uint64_t tail_cap) {
+    if (!ctx || !info || (!carry && carry_len) || (!in && in_len)) return fail(ctx, CBCG_ERR_ARG, "cbcg_batch_upload_bam: bad argument");
+    memset(info, 0, sizeof *info);
+    if (!ctx->bam_opened) return fail(ctx, CBCG_ERR_ARG, "cbcg_batch_upload_bam: cbcg_bam_open has not been called on this context");
+    CU(cudaSetDevice(ctx->device));
+    const uint32_t derive = (flags & CBCG_BAM_DERIVE_MD) ? 1u : 0u;
+    std::vector<BgzfMember> m;
+    uint64_t walked = 0, T = 0;
+    TRY(bgzf_members(ctx, in, in_len, carry_len, m, &walked, &T));
+    info->inflated_bytes = T;
+    ctx->stats = cbcg_stats();
+    CU(cudaEventRecord(ctx->ev[0], ctx->st));
+    TRY(bgzf_inflate_into_stream(ctx, carry, carry_len, in, in_len, m, T));
+
+    /* record boundaries: a segment per member, the carry in the first */
+    const uint32_t n_seg = (uint32_t)std::max<size_t>(m.size(), 1);
+    std::vector<uint64_t> seg(n_seg + 1);
+    seg[0] = 0;
+    for (uint32_t k = 1; k < n_seg; k++) seg[k] = m[k].out_off;
+    seg[n_seg] = T;
+    const int32_t n_ref = (int32_t)ctx->bam_map.size();
+    TRY(ensure(ctx, ctx->bi_seg, (n_seg + 1) * 8));
+    TRY(ensure(ctx, ctx->bi_work, 5ull * n_seg * 8));
+    const uint64_t rec_cap = T / 36 + 2;                   /* a chain passes only records of >= 36 bytes (k10_next) */
+    TRY(ensure(ctx, ctx->bi_rec, rec_cap * 8));
+    TRY(ensure(ctx, ctx->bi_map, (size_t)std::max(n_ref, 1) * 4));
+    CU(cudaMemcpyAsync(ctx->bi_seg.p, seg.data(), (n_seg + 1) * 8, cudaMemcpyHostToDevice, ctx->st));
+    if (n_ref) CU(cudaMemcpyAsync(ctx->bi_map.p, ctx->bam_map.data(), (size_t)n_ref * 4, cudaMemcpyHostToDevice, ctx->st));
+    TRY(reset_words(ctx));
+    uint64_t *bw = wptr<uint64_t>(ctx, W_OFF(bam));
+    if (launch_bam_boundaries(ctx->bi_stream.as<uint8_t>(), T, ctx->bi_seg.as<uint64_t>(), n_seg, n_ref, ctx->bi_work.as<uint64_t>(),
+                              ctx->bi_rec.as<uint64_t>(), rec_cap, bw, wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "record boundary launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    ctx->stats.kernel_launches += 3;
+    TRY(fetch_words(ctx));
+    TRY(device_error(ctx, "BAM record boundaries"));      /* a block_size below 32 on the chain: CBCG_ERR_FORMAT, item the record */
+    const uint64_t R = ctx->hw->bam[0], tail_at = ctx->hw->bam[1], tail_len = T - tail_at;
+    info->n_records = R; info->tail_len = tail_len;
+    if ((flags & CBCG_BAM_LAST) && tail_len)
+        return fail(ctx, CBCG_ERR_FORMAT, "BAM: the input ends inside a record (%llu bytes after the last whole record)", (unsigned long long)tail_len);
+    if (tail_len > tail_cap || (!tail && tail_len))
+        return fail(ctx, CBCG_ERR_CAPACITY, "BAM: %llu bytes after the last whole record, room for %llu", (unsigned long long)tail_len, (unsigned long long)tail_cap);
+
+    /* the records -> the resident batch (as batch_prepare, sized for every record; the pools once their sizes are counted) */
+    ctx->have_batch = false; ctx->have_encoded = false;
+    ctx->batch_no_md = derive != 0;
+    ctx->runs.clear();
+    if (R) {
+        TRY(ensure(ctx, ctx->b_pos, R * 4)); TRY(ensure(ctx, ctx->b_flag, R * 2)); TRY(ensure(ctx, ctx->b_len, R * 2));
+        TRY(ensure(ctx, ctx->b_chr, R * 4));
+        TRY(ensure(ctx, ctx->b_soff, (R + 1) * 8)); TRY(ensure(ctx, ctx->b_coff, (R + 1) * 8)); TRY(ensure(ctx, ctx->b_moff, (R + 1) * 8));
+        TRY(ensure(ctx, ctx->bi_src, R * 16 + 16));
+        TRY(ensure(ctx, ctx->tile_desc, (4 * bam_in_num_tiles(R) + 1) * 8));
+    }
+    ctx->db = DevBatch{};
+    ctx->db.n_reads = R;
+    ctx->db.pos = ctx->b_pos.as<uint32_t>(); ctx->db.flag = ctx->b_flag.as<uint16_t>(); ctx->db.seq_len = ctx->b_len.as<uint16_t>();
+    ctx->db.chr = ctx->b_chr.as<uint32_t>();
+    ctx->db.seq_off = ctx->b_soff.as<uint64_t>(); ctx->db.cigar_off = ctx->b_coff.as<uint64_t>(); ctx->db.md_off = ctx->b_moff.as<uint64_t>();
+    uint64_t *src = ctx->bi_src.as<uint64_t>(), *md_at = src + R;
+    if (R && launch_bam_count(ctx->bi_stream.as<uint8_t>(), ctx->bi_rec.as<uint64_t>(), R, ctx->bi_map.as<int32_t>(), n_ref, derive, ctx->db,
+                              src, md_at, ctx->tile_desc.as<uint64_t>(), wptr<uint32_t>(ctx, W_OFF(ticket)), bw,
+                              wptr<uint32_t>(ctx, W_OFF(bam_len)), wptr<unsigned long long>(ctx, W_OFF(err)), ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "BAM record count launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (R) ctx->stats.kernel_launches++;
+    TRY(fetch_words(ctx));
+    TRY(device_error(ctx, "BAM records"));
+    const uint64_t n = ctx->hw->bam[3], seq_b = ctx->hw->bam[4], cig_b = ctx->hw->bam[5], md_b = derive ? md_bytes_guess(seq_b, n) : ctx->hw->bam[6];
+    info->n_reads = n; info->n_unmapped = R - n;
+    info->len_first = ctx->hw->bam_len[0]; info->len_second = R > 1 ? ctx->hw->bam_len[1] : 0;
+    const uint32_t min_len = n ? 0xffffffffu - ctx->hw->bam_len[2] : 0, max_len = n ? ctx->hw->bam_len[3] : 0;
+    info->min_len = min_len; info->max_len = max_len;
+    TRY(ensure(ctx, ctx->b_seq, seq_b + POOL_PAD)); TRY(ensure(ctx, ctx->b_cigar, cig_b + POOL_PAD)); TRY(ensure(ctx, ctx->b_md, md_b + POOL_PAD));
+    TRY(ensure(ctx, ctx->bi_runs, 4 * n * 8 + 16));
+    ctx->db.n_reads = n;
+    ctx->db.seq = ctx->b_seq.as<uint8_t>(); ctx->db.cigar = ctx->b_cigar.as<uint8_t>(); ctx->db.md = ctx->b_md.as<uint8_t>();
+    uint64_t *run_first = ctx->bi_runs.as<uint64_t>(), *run_last = run_first + 2 * n;
+    if (n && launch_bam_write(ctx->bi_stream.as<uint8_t>(), ctx->db, derive, src, md_at, run_first, run_last, bw, ctx->st))
+        return fail(ctx, CBCG_ERR_CUDA, "BAM record write launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (n) ctx->stats.kernel_launches++;
+    TRY(fetch_words(ctx));
+    const uint64_t n_runs = ctx->hw->bam[7];
+    if (n_runs != ctx->hw->bam[8] || n_runs > n) return fail(ctx, CBCG_ERR_INTERNAL, "BAM: chromosome run lists disagree");
+
+    /* what batch_scan learns from a host batch: runs, lengths, bases, the window and the indel hint */
+    struct RunEnd { uint64_t key, pos; };                  /* (first read | chromosome << 32, its POS) / (last read, its POS) */
+    std::vector<RunEnd> rf(n_runs), rl(n_runs);
+    if (n_runs) {                                          /* two copies whatever the run count (unsorted input has many) */
+        CU(cudaMemcpyAsync(rf.data(), run_first, n_runs * 16, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaMemcpyAsync(rl.data(), run_last, n_runs * 16, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        std::sort(rf.begin(), rf.end(), [](const RunEnd &a, const RunEnd &b) { return (uint32_t)a.key < (uint32_t)b.key; });
+        std::sort(rl.begin(), rl.end(), [](const RunEnd &a, const RunEnd &b) { return a.key < b.key; });
+    }
+    uint64_t span = 0;
+    for (uint64_t k = 0; k < n_runs; k++) {
+        ctx->runs.push_back(ChrRun{ (uint32_t)rf[k].key, rl[k].key - (uint32_t)rf[k].key + 1, (uint32_t)(rf[k].key >> 32) });
+        if (rl[k].pos > rf[k].pos) span += rl[k].pos - rf[k].pos;
+    }
+    ctx->db.max_len = max_len;
+    ctx->db.ref_cap = n ? ref_window_from_span(span, n, max_len) : 0u;
+    ctx->batch_indel_heavy = n && cig_b > n * 6ull;
+    ctx->batch_min_len = min_len;
+    ctx->total_bases = seq_b;
+    if (n && (min_len == 0 || max_len > CBCG_MAX_READ_LEN))
+        return fail(ctx, CBCG_ERR_INPUT, "read length outside 1..%u (shortest %u, longest %u)", CBCG_MAX_READ_LEN, min_len, max_len);
+    if (n && derive) TRY(derive_md(ctx, 0));
+    if (tail_len) CU(cudaMemcpyAsync(tail, ctx->bi_stream.as<uint8_t>() + tail_at, tail_len, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaEventRecord(ctx->ev[1], ctx->st));
+    CU(cudaStreamSynchronize(ctx->st));
+    ctx->have_batch = true;
+    float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]);
+    ctx->stats.ms_h2d = ms; ctx->stats.h2d_bytes = in_len + carry_len; ctx->stats.n_reads = n;
     return CBCG_OK;
 }

@@ -2,12 +2,16 @@
  * cbc_main.c -- the reference's command line over the B200 path.
  *
  *   cbc -c <sam> <out> <ref.fa>     compress   (README.md:59;  checked-in spelling `-c <ratio> ...`, src/main.c:114-123, also accepted)
+ *                                   <sam> may be BAM (BGZF, recognised by its first bytes): its members are inflated and its
+ *                                   records parsed on the GPU (cbcg_batch_upload_bam), with the same container as the SAM text
+ *                                   a BAM reader prints for it
  *   cbc -d <in>  <out> <ref.fa>     decompress (README.md:67;  checked-in spelling `-x`, src/main.c:136-139, also accepted)
  * options: -b N     reads per block (default: sized by the library, CBCG_BLOCK_AUTO; the container is the blocked "CBCB" format)
  *          -1       single-block mode: the reference's own stream, byte-identical to `program -c 1` built with -DDEBUG
  *          -l       variable-length reads: header read length = longest SEQ (src/main.c -l)
  *          -g LIST  CUDA devices, e.g. `-g 0,1,2,3`: batches (region shards of the sorted input) are dealt out to them
- *          -B MB    SAM text per batch (default 2048): memory is bounded by three batches whatever the file size
+ *          -B MB    SAM text per batch (default 2048; BAM: inflated bytes, in runs of whole BGZF members, from their ISIZE):
+ *                   memory is bounded by three batches whatever the file size
  *          -M       -c only: the input's MD:Z tags are not read (records need none); every read's MD is derived on the GPU from its
  *                   CIGAR, SEQ and the reference (cbcg.h, "a batch without MD"), so an aligner's output without --MD codes as it
  *                   would after `samtools calmd`. The container is the one the derived MD gives, and nothing in it records -M.
@@ -62,10 +66,23 @@
 #define CBCS_MAGIC 0x53434243u
 
 static uint32_t rd_u32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
+/* The size of the BGZF member at p (n bytes left): BSIZE + 1 from the BC subfield of its extra field, wherever that sits
+   among the subfields; 0 when it is not a whole BGZF member (the library then reports the broken member). */
+static uint64_t bgzf_member_size(const uint8_t *p, uint64_t n) {
+    if (n < 18 || p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || p[3] != 4) return 0;
+    const uint32_t xlen = (uint32_t)(p[10] | p[11] << 8);
+    if (12ull + xlen > n) return 0;
+    for (uint32_t x = 12; x + 4 <= 12 + xlen; x += 4 + (uint32_t)(p[x + 2] | p[x + 3] << 8))
+        if (p[x] == 'B' && p[x + 1] == 'C' && (p[x + 2] | p[x + 3] << 8) == 2 && x + 6 <= 12 + xlen) {
+            const uint64_t total = (uint64_t)(p[x + 4] | p[x + 5] << 8) + 1;
+            return total >= 12ull + xlen + 8 && total <= n ? total : 0;
+        }
+    return 0;
+}
 static double now(void) { struct timespec t; clock_gettime(CLOCK_MONOTONIC, &t); return (double)t.tv_sec + 1e-9 * (double)t.tv_nsec; }
 
 static int usage(void) {
-    fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-M] [-b reads_per_block] [-g devices] [-B batch_MB] <sam> <out> <ref.fa>\n"
+    fprintf(stderr, "usage: cbc -c [-1] [-l] [-C] [-M] [-b reads_per_block] [-g devices] [-B batch_MB] <sam|bam> <out> <ref.fa>\n"
                     "       cbc -d [-C] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -r NAME[:START[-END]] [-r ...] [-g devices] <in> <out> <ref.fa>\n"
                     "       cbc -d -S [-C] [-r NAME[:START[-END]] ...] [-g devices] <in> <out.sam> <ref.fa>\n"
@@ -90,6 +107,8 @@ typedef struct job {
     int done, written;
     uint64_t bound, seq_bases; uint32_t header_len;
     uint8_t *bam_head; uint64_t bam_head_len;   /* -Z, batch 0: the BAM header blocks */
+    /* BAM input: the record bytes after this batch's last whole record (the next batch's carry), once uploaded */
+    uint8_t *tail; uint64_t tail_len; int uploaded; uint64_t n_unmapped;
 } job;
 
 typedef struct shared {
@@ -102,10 +121,71 @@ typedef struct shared {
     int mode, single, var_length, with_cigar, sam, bam, derive_md, pileup; uint32_t block_reads, flag_exclude;
     const cbch_fasta *fa; int fa_ready;
     const cbcg_region *regions; uint32_t n_regions;     /* -r: region decode */
+    int bam_in; const uint8_t *file; uint64_t file_len;  /* -c of a BAM file: the whole mapped file (every context reads its header) */
     double t_gpu_ready;
 } shared;
 
-typedef struct devthread { shared *S; int device; pthread_t th; int rc; char err[256]; double create_s, setref_s, call_s, alloc_s; } devthread;
+typedef struct devthread { shared *S; int device; pthread_t th; int rc; char err[256]; double create_s, setref_s, call_s, alloc_s;
+                           uint64_t bam_used; uint8_t *bam_tail; uint64_t bam_tail_len; } devthread;
+
+/* -c of a BAM file, batch J: runs of whole BGZF members, inflated and parsed on the device. Its upload waits for the previous
+ * batch's tail (the bytes of the record that crosses into this batch); only the uploads are serialised, encodes overlap. */
+static void compress_bam_job(shared *S, devthread *D, cbcg_ctx *ctx, job *J) {
+    const uint64_t k = J->index;
+    job *P = k ? S->jobs[k - 1] : NULL;
+    pthread_mutex_lock(&S->mu);
+    while (P && !P->uploaded) pthread_cond_wait(&S->cv, &S->mu);
+    pthread_mutex_unlock(&S->mu);
+    uint64_t a = (uint64_t)(J->in - S->file), e = a + J->in_len;   /* the header's members belong to no batch */
+    if (a < D->bam_used) a = D->bam_used;
+    if (e < a) e = a;
+    cbcg_bam_info info; memset(&info, 0, sizeof info);
+    int rc = 0;
+    if (P && P->rc) { rc = P->rc; snprintf(J->err, sizeof J->err, "%s", P->err); }
+    else {
+        const uint8_t *carry = P ? P->tail : D->bam_tail; const uint64_t carry_len = P ? P->tail_len : D->bam_tail_len;
+        const uint32_t flags = (S->derive_md ? CBCG_BAM_DERIVE_MD : 0u) | (k + 1 == S->n_jobs ? CBCG_BAM_LAST : 0u);
+        uint64_t cap = 1u << 17;
+        for (;;) {
+            J->tail = (uint8_t *)malloc(cap);
+            rc = J->tail ? cbcg_batch_upload_bam(ctx, carry, carry_len, S->file + a, e - a, flags, &info, J->tail, cap) : CBCG_ERR_NOMEM;
+            if (rc != CBCG_ERR_CAPACITY || info.tail_len <= cap) break;
+            free(J->tail); J->tail = NULL; cap = info.tail_len;
+        }
+        if (rc) snprintf(J->err, sizeof J->err, "%s", cbcg_last_error(ctx));
+        J->tail_len = info.tail_len;
+        /* as the SAM path: -l each batch's longest read; else the first batch holding a record fixes it (its second record,
+           or its only one) and every later batch takes that */
+        uint32_t h = 0;
+        for (uint64_t j = 0; j < k && !h && !S->var_length; j++) h = S->jobs[j]->header_len;
+        J->header_len = S->var_length ? info.max_len : h ? h : info.n_records >= 2 ? info.len_second : info.len_first;
+        J->n_reads = info.n_reads; J->n_unmapped = info.n_unmapped;
+    }
+    pthread_mutex_lock(&S->mu);
+    J->rc = rc; J->uploaded = 1;
+    if (P) { free(P->tail); P->tail = NULL; }
+    pthread_cond_broadcast(&S->cv);
+    pthread_mutex_unlock(&S->mu);
+    if (rc) return;
+    cbcg_encode_opts o = { J->header_len ? J->header_len : 1u, S->single ? 0u : S->block_reads, S->single ? 0u : 1u, 0u };
+    uint64_t n = 0;
+    const double tq = now();
+    rc = cbcg_encode_resident(ctx, &o);
+    if (!rc) {
+        rc = cbcg_fetch_container(ctx, NULL, 0, &n);
+        if (rc == CBCG_ERR_CAPACITY) rc = (J->out = (uint8_t *)malloc(n ? n : 1)) ? cbcg_fetch_container(ctx, J->out, n, &n) : CBCG_ERR_NOMEM;
+    }
+    J->out_len = n;
+    D->call_s += now() - tq;
+    cbcg_stats st; cbcg_get_stats(ctx, &st); J->device_ms = st.ms_total; J->n_blocks = st.n_blocks;
+    if (!rc && S->with_cigar) {                                   /* the batch exists only on the device */
+        uint64_t cn = 0;
+        rc = cbcg_cigar_pack_resident(ctx, NULL, 0, &cn);
+        if (rc == CBCG_ERR_CAPACITY) rc = (J->cig = (uint8_t *)malloc(cn)) ? cbcg_cigar_pack_resident(ctx, J->cig, cn, &cn) : CBCG_ERR_NOMEM;
+        J->cig_len = cn;
+    }
+    if (rc) { J->rc = rc; snprintf(J->err, sizeof J->err, "%s", cbcg_last_error(ctx)); }
+}
 
 static void *device_main(void *arg) {
     devthread *D = (devthread *)arg;
@@ -123,6 +203,11 @@ static void *device_main(void *arg) {
         rc = cbcg_set_reference(ctx, S->fa->n, (const char *const *)S->fa->names, (const uint8_t *const *)S->fa->bases, S->fa->len);
         if (rc) { snprintf(D->err, sizeof D->err, "device %d: %s", D->device, cbcg_last_error(ctx)); D->rc = rc; }
     }
+    if (!rc && S->bam_in) {                                      /* every context reads the header: its refID map */
+        D->bam_tail = (uint8_t *)malloc(1u << 17);
+        rc = D->bam_tail ? cbcg_bam_open(ctx, S->file, S->file_len, &D->bam_used, D->bam_tail, 1u << 17, &D->bam_tail_len) : CBCG_ERR_NOMEM;
+        if (rc) { snprintf(D->err, sizeof D->err, "device %d: %s", D->device, cbcg_last_error(ctx)); D->rc = rc; }
+    }
     D->setref_s = now() - tq;
     pthread_mutex_lock(&S->mu);
     if (S->t_gpu_ready == 0) S->t_gpu_ready = now();
@@ -133,7 +218,11 @@ static void *device_main(void *arg) {
         if (S->next_take >= S->n_jobs || (S->producer_failed && S->next_take >= S->produced)) { pthread_mutex_unlock(&S->mu); break; }
         job *J = S->jobs[S->next_take++];
         pthread_mutex_unlock(&S->mu);
-        if (D->rc) { J->rc = D->rc; snprintf(J->err, sizeof J->err, "%s", D->err); }
+        if (D->rc) {
+            J->rc = D->rc; snprintf(J->err, sizeof J->err, "%s", D->err);
+            pthread_mutex_lock(&S->mu); J->uploaded = 1; pthread_cond_broadcast(&S->cv); pthread_mutex_unlock(&S->mu);
+        }
+        else if (S->mode == 'c' && S->bam_in) compress_bam_job(S, D, ctx, J);
         else if (S->mode == 'c') {
             cbcg_encode_opts o = { J->header_len ? J->header_len : 1u, S->single ? 0u : S->block_reads, S->single ? 0u : 1u, 0u };
             cbcg_batch v; cbch_batch_view(&J->hb, &v);
@@ -250,6 +339,7 @@ static void *device_main(void *arg) {
         pthread_mutex_unlock(&S->mu);
     }
     if (ctx) cbcg_destroy(ctx);
+    free(D->bam_tail);
     return NULL;
 }
 
@@ -500,13 +590,32 @@ int main(int argc, char **argv) {
         printf("Compressing...\n");
         const uint64_t batch_bytes = batch_mb << 20;
         if (cbch_map(files[0], 0, &map)) { fprintf(stderr, "cbc: cannot open %s\n", files[0]); return 1; }
-        S.n_jobs = single ? 1 : (map.n + batch_bytes - 1) / batch_bytes;
-        if (S.n_jobs == 0) S.n_jobs = 1;
-        cut = (const uint8_t **)calloc(S.n_jobs + 1, sizeof *cut);
         const uint8_t *end = map.p + map.n;
-        cut[0] = map.p;
-        for (uint64_t k = 1; k < S.n_jobs; k++) { const uint8_t *g = map.p + k * batch_bytes; cut[k] = g < end ? cbch_next_line(g, end) : end; if (cut[k] < cut[k - 1]) cut[k] = cut[k - 1]; }
-        cut[S.n_jobs] = end;
+        S.bam_in = bgzf_member_size(map.p, map.n) != 0;
+        if (S.bam_in) {                                        /* BGZF: batches of whole members, about batch_MB inflated, from the trailers' ISIZE */
+            S.file = map.p; S.file_len = map.n;
+            uint64_t cap = 64, n = 0, o = 0, acc = 0;
+            cut = (const uint8_t **)calloc(cap, sizeof *cut);
+            cut[n++] = map.p;
+            while (cut && o < map.n) {
+                const uint64_t total = bgzf_member_size(map.p + o, map.n - o);
+                if (!total) break;                                          /* the library reports the broken member */
+                acc += rd_u32(map.p + o + total - 4); o += total;
+                if (!single && acc >= batch_bytes && o < map.n) {
+                    if (n + 2 > cap) { cap *= 2; cut = (const uint8_t **)realloc(cut, cap * sizeof *cut); if (!cut) break; }
+                    cut[n++] = map.p + o; acc = 0;
+                }
+            }
+            if (!cut) { fprintf(stderr, "cbc: out of memory\n"); return 1; }
+            S.n_jobs = n; cut[n] = end;
+        } else {
+            S.n_jobs = single ? 1 : (map.n + batch_bytes - 1) / batch_bytes;
+            if (S.n_jobs == 0) S.n_jobs = 1;
+            cut = (const uint8_t **)calloc(S.n_jobs + 1, sizeof *cut);
+            cut[0] = map.p;
+            for (uint64_t k = 1; k < S.n_jobs; k++) { const uint8_t *g = map.p + k * batch_bytes; cut[k] = g < end ? cbch_next_line(g, end) : end; if (cut[k] < cut[k - 1]) cut[k] = cut[k - 1]; }
+            cut[S.n_jobs] = end;
+        }
     } else {
         printf("Decompressing...\n");
         /* mapped, not read: the payload pages a region query does not need are never read from disk */
@@ -519,6 +628,10 @@ int main(int argc, char **argv) {
     }
     S.jobs = (job **)calloc(S.n_jobs, sizeof *S.jobs);
     for (uint64_t k = 0; k < S.n_jobs; k++) { S.jobs[k] = (job *)calloc(1, sizeof(job)); S.jobs[k]->index = k; }
+    if (S.bam_in) {
+        for (uint64_t k = 0; k < S.n_jobs; k++) { S.jobs[k]->in = cut[k]; S.jobs[k]->in_len = (uint64_t)(cut[k + 1] - cut[k]); }
+        S.produced = S.n_jobs;
+    }
     if (mode == 'd') {
         uint64_t nr, cap;
         if (S.n_jobs == 1 && !(in_len >= 16 && rd_u32(in) == CBCS_MAGIC)) {
@@ -572,7 +685,7 @@ int main(int argc, char **argv) {
     ingest_arg IA; memset(&IA, 0, sizeof IA);
     pthread_t ith; int have_ith = 0;
     const double t1 = now();
-    if (mode == 'c' && !status) {
+    if (mode == 'c' && !status && !S.bam_in) {
         IA.S = &S; IA.map = &map; IA.cut = cut; IA.window = (uint64_t)n_dev + 2;
         pthread_create(&ith, NULL, ingest_main, &IA); have_ith = 1;
     }
@@ -617,7 +730,7 @@ int main(int argc, char **argv) {
             cig_bytes += 8 + J->cig_len;
         }
         if (sharded) { shard_off[k] = filepos; shard_len[k] = J->out_len; filepos += J->out_len; }
-        total_reads += J->n_reads; total_out += J->out_len; total_blocks += J->n_blocks; device_ms += J->device_ms;
+        total_reads += J->n_reads; total_out += J->out_len; total_blocks += J->n_blocks; device_ms += J->device_ms; IA.n_unmapped += J->n_unmapped;
         if (mode == 'c') { seq_bases += J->seq_bases; cbch_free_batch(&J->hb); }
         pthread_mutex_lock(&S.mu);
         free(J->out); J->out = NULL; free(J->cig); J->cig = NULL; J->written = 1;     /* frees a slot of the ingest window */
@@ -645,10 +758,16 @@ int main(int argc, char **argv) {
             printf("Final Size: %llu\n", (unsigned long long)total_out);
             if (with_cigar) printf("CIGAR sections: %llu bytes\n", (unsigned long long)cig_bytes);
             printf("Compression took %f\n", t2 - t1);
-            printf("reads %llu (unmapped skipped %llu), blocks %llu, batches %llu on %d device(s), %.4f bits/base, fasta %.3f s, ingest %.3f s (%.2f GB/s), gpu ready %.3f s, device %.3f ms\n",
-                   (unsigned long long)total_reads, (unsigned long long)IA.n_unmapped, (unsigned long long)total_blocks, (unsigned long long)S.n_jobs, n_dev,
-                   seq_bases ? 8.0 * (double)total_out / (double)seq_bases : 0.0, fasta_s, IA.ingest_s, IA.ingest_s > 0 ? (double)map.n / IA.ingest_s / 1e9 : 0.0,
-                   S.t_gpu_ready - t0, device_ms);
+            if (S.bam_in) {                                    /* the batches exist only on the devices: no host ingest, no host base count */
+                printf("reads %llu (unmapped skipped %llu), blocks %llu, batches %llu on %d device(s), BAM input %.3f MB, fasta %.3f s, gpu ready %.3f s, device %.3f ms\n",
+                       (unsigned long long)total_reads, (unsigned long long)IA.n_unmapped, (unsigned long long)total_blocks, (unsigned long long)S.n_jobs, n_dev,
+                       (double)map.n / 1e6, fasta_s, S.t_gpu_ready - t0, device_ms);
+            } else {
+                printf("reads %llu (unmapped skipped %llu), blocks %llu, batches %llu on %d device(s), %.4f bits/base, fasta %.3f s, ingest %.3f s (%.2f GB/s), gpu ready %.3f s, device %.3f ms\n",
+                       (unsigned long long)total_reads, (unsigned long long)IA.n_unmapped, (unsigned long long)total_blocks, (unsigned long long)S.n_jobs, n_dev,
+                       seq_bases ? 8.0 * (double)total_out / (double)seq_bases : 0.0, fasta_s, IA.ingest_s, IA.ingest_s > 0 ? (double)map.n / IA.ingest_s / 1e9 : 0.0,
+                       S.t_gpu_ready - t0, device_ms);
+            }
         } else {
             printf("Decompression took %f\n", t2 - t1);
             printf("reads %llu, shards %llu on %d device(s), gpu ready %.3f s, device %.3f ms\n", (unsigned long long)total_reads, (unsigned long long)S.n_jobs, n_dev, S.t_gpu_ready - t0, device_ms);
@@ -656,7 +775,7 @@ int main(int argc, char **argv) {
     }
     if (getenv("CBC_TRACE")) for (int d = 0; d < n_dev; d++)
         fprintf(stderr, "[cbc] device %d: context %.3f s, reference upload %.3f s, coding calls %.3f s; writer done at %.3f s\n", dev[d], D[d].create_s, D[d].setref_s, D[d].call_s, t2 - t0);
-    for (uint64_t k = 0; k < S.n_jobs; k++) { free(S.jobs[k]->out); free(S.jobs[k]->cig); free(S.jobs[k]->bam_head); free(S.jobs[k]); }
+    for (uint64_t k = 0; k < S.n_jobs; k++) { free(S.jobs[k]->out); free(S.jobs[k]->cig); free(S.jobs[k]->bam_head); free(S.jobs[k]->tail); free(S.jobs[k]); }
     free(S.jobs); free(cut); free(cig_file); free(shard_off); free(shard_len);
     for (uint32_t k = 0; k < n_regions; k++) free((void *)regions[k].name);
     free(regions);

@@ -201,3 +201,25 @@ int launch_bam_records(uint64_t n_reads, const cbcg_read_rec *recs, const uint32
                        uint64_t *totals, unsigned long long *err, cudaStream_t st);
 int launch_bgzf(const uint8_t *stream, const uint64_t *rec_off, const uint32_t *block_first, uint32_t n_blocks, uint8_t *out,
                 uint64_t *tile_desc, uint32_t *ticket, uint64_t *total_bytes, unsigned long long *err, cudaStream_t st);
+/* k10_bam_in.cu: BAM input (DESIGN.md 5g). BgzfMember: one BGZF member, found by the host's walk of the header chain: its raw
+   deflate bytes in[in_off, + in_len), its output out[out_off, + isize) and its CRC32. launch_inflate: a warp per member;
+   CBCG_ERR_CORRUPT (item: the member) on any deflate, ISIZE or CRC problem. launch_bam_boundaries: the whole records of the
+   stream [0, T) cut into n_seg segments at seg[0 .. n_seg] (seg[0] = 0, seg[n_seg] = T); work: 5 n_seg words; rec_start: the
+   offset of every whole record (rec_cap entries; T / 36 + 1 suffice: a chain stops at a block_size below 32, and one that
+   reaches it is CBCG_ERR_FORMAT); words[0] receives the record count, [1] the start of the bytes after the last whole
+   record, [2] the segments walked again. launch_bam_count / launch_bam_write: the mapped records (map: refID ->
+   genome ordinal, -1 for none) into the batch b (b.n_reads records' room for launch_bam_count, then the pools sized from
+   words[3..6]: reads, SEQ, CIGAR and MD bytes; derive: no MD is looked for); tile_desc: 4 x bam_in_num_tiles words; lens:
+   l_seq of records 0 and 1, 0xffffffff - the shortest and the longest read. src / md_at: a word per record. run_first /
+   run_last: room for b.n_reads pairs of words each ((first read | chromosome << 32, POS), (last read, POS)); words[7] / [8]
+   receive their counts. */
+struct BgzfMember { uint64_t in_off, out_off; uint32_t in_len, isize, crc, pad; };
+int launch_inflate(const uint8_t *in, const BgzfMember *mem, uint32_t n_members, uint8_t *out, unsigned long long *err, cudaStream_t st);
+int launch_bam_boundaries(const uint8_t *stream, uint64_t T, const uint64_t *seg, uint32_t n_seg, int32_t n_ref, uint64_t *work,
+                          uint64_t *rec_start, uint64_t rec_cap, uint64_t *words, unsigned long long *err, cudaStream_t st);
+uint64_t bam_in_num_tiles(uint64_t n_records);
+int launch_bam_count(const uint8_t *stream, const uint64_t *rec_start, uint64_t n_rec, const int32_t *map, int32_t n_ref, uint32_t derive,
+                     const DevBatch &b, uint64_t *src, uint64_t *md_at, uint64_t *tile_desc, uint32_t *ticket, uint64_t *words, uint32_t *lens,
+                     unsigned long long *err, cudaStream_t st);
+int launch_bam_write(const uint8_t *stream, const DevBatch &b, uint32_t derive, const uint64_t *src, const uint64_t *md_at, uint64_t *run_first,
+                     uint64_t *run_last, uint64_t *words, cudaStream_t st);

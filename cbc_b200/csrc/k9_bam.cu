@@ -28,7 +28,7 @@
  *   k9_bgzf_kernel: one CTA of K9_BGZF_THREADS per BGZF block (tile order from an atomic ticket). The block's records come
  *     in by one TMA bulk copy. Each thread takes a contiguous chunk of the block's bytes: a pass computes the chunk's raw
  *     CRC32 and its deflate bit cost (8 or 9 bits per literal, the QUAL match's code and extra bits on the byte after the
- *     first 0xff, 0 on the rest of the run); the chunk CRCs are combined by GF(2) shifts (zlib's crc32_combine), a CTA scan
+ *     first 0xff, 0 on the rest of the run); the chunk CRCs are combined by GF(2) shifts (zlib's crc32_combine, bgzf.cuh), a CTA scan
  *     of the costs gives each chunk's bit offset, and a second pass writes the codes into a zeroed shared-memory bit image
  *     (shared atomicOr on the words a chunk shares with its neighbours). A decoupled look-back over the block sizes gives
  *     its output offset; the block leaves by 16-byte vector stores.
@@ -36,6 +36,7 @@
 #include "common.cuh"
 #include "internal.h"
 #include "sam_fields.cuh"
+#include "bgzf.cuh"
 
 #define K9_TILE 128u
 #define K9_MAX_RECORD 8192u
@@ -307,30 +308,6 @@ k9_bam_record_kernel(uint64_t n_reads, const cbcg_read_rec *__restrict__ recs, c
 }
 
 /* ---------------------------------------------------------------- BGZF blocks */
-#define K9_CRC_POLY 0xedb88320u
-/* x^(2^k) mod P, reflected (zlib's x2n_table) */
-__constant__ uint32_t k9_x2n[32] = {
-    0x40000000u, 0x20000000u, 0x08000000u, 0x00800000u, 0x00008000u, 0xedb88320u, 0xb1e6b092u, 0xa06a2517u, 0xed627daeu, 0x88d14467u,
-    0xd7bbfe6au, 0xec447f11u, 0x8e7ea170u, 0x6427800eu, 0x4d47bae0u, 0x09fe548fu, 0x83852d0fu, 0x30362f1au, 0x7b5a9cc3u, 0x31fec169u,
-    0x9fec022au, 0x6c8dedc4u, 0x15d6874du, 0x5fde7a4eu, 0xbad90e37u, 0x2e4e5eefu, 0x4eaba214u, 0xa8a472c0u, 0x429a969eu, 0x148d302au,
-    0xc40ba6d0u, 0xc4e22c3cu };
-
-/* a * b mod P, reflected (zlib's multmodp) */
-__device__ __forceinline__ uint32_t k9_multmodp(uint32_t a, uint32_t b) {
-    uint32_t p = 0;
-    for (uint32_t m = 1u << 31; m; m >>= 1) {
-        if (a & m) p ^= b;
-        b = (b & 1u) ? (b >> 1) ^ K9_CRC_POLY : b >> 1;
-    }
-    return p;
-}
-/* crc * x^(8 n) mod P: a raw CRC followed by n more bytes of zeros */
-__device__ __forceinline__ uint32_t k9_crc_shift(uint32_t crc, uint32_t n) {
-    uint32_t op = 1u << 31, k = 3;
-    for (; n; n >>= 1, k++) if (n & 1u) op = k9_multmodp(k9_x2n[k & 31u], op);
-    return k9_multmodp(op, crc);
-}
-
 /* A length symbol of the fixed code: its code reversed for LSB-first output, the code's bits, extra bits and their value. */
 __device__ __forceinline__ void k9_len_sym(uint32_t L, uint32_t &code, uint32_t &nb, uint32_t &eb, uint32_t &ev) {
     uint32_t sym;
@@ -409,9 +386,7 @@ k9_bgzf_kernel(const uint8_t *__restrict__ stream, const uint64_t *__restrict__ 
         tma_load_1d(stage, stream + (S.in_base - head), bytes, &S.bar);
     }
     for (uint32_t k = tid; k < 256u; k += K9_BGZF_THREADS) {
-        uint32_t c = k;
-        for (int j = 0; j < 8; j++) c = (c & 1u) ? (c >> 1) ^ K9_CRC_POLY : c >> 1;
-        S.crc_tab[k] = c;
+        S.crc_tab[k] = bgzf_crc_table_entry(k);
     }
     if (B) for (uint32_t k = tid; k <= nrec; k += K9_BGZF_THREADS) S.rs[k] = (uint16_t)(rec_off[S.first + k] - S.in_base);
     for (uint32_t k = tid; k < K9_IMG_BYTES / 4u; k += K9_BGZF_THREADS) reinterpret_cast<uint32_t *>(blk)[k] = 0u;
@@ -434,7 +409,7 @@ k9_bgzf_kernel(const uint8_t *__restrict__ stream, const uint64_t *__restrict__ 
         } else bits += k9_lit_bits(v);
     }
     /* the block's CRC: each chunk's raw CRC shifted past the bytes after it, the initial value's shifted past the block */
-    uint32_t part = a < b ? k9_crc_shift(crc, B - b) : 0u;
+    uint32_t part = a < b ? bgzf_crc_shift(crc, B - b) : 0u;
     for (int o = 16; o > 0; o >>= 1) part ^= __shfl_xor_sync(FULL_MASK, part, o);
     const uint32_t incl = warp_incl_scan(bits);
     if (lane == 31u) { S.warp_bits[warp] = incl; S.warp_crc[warp] = part; }
@@ -477,7 +452,7 @@ k9_bgzf_kernel(const uint8_t *__restrict__ stream, const uint64_t *__restrict__ 
     if (tid == 0) {
         const uint8_t h18[18] = { 0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, (uint8_t)(size - 1u), (uint8_t)((size - 1u) >> 8) };
         for (int j = 0; j < 18; j++) blk[2 + j] = h18[j];
-        const uint32_t crc32 = crc_all ^ k9_crc_shift(0xffffffffu, B) ^ 0xffffffffu;
+        const uint32_t crc32 = bgzf_crc_finish(crc_all, B);
         uint8_t *f = blk + 20 + dbytes;
         st_le32(f, crc32); st_le32(f + 4, B);
     }

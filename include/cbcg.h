@@ -337,6 +337,45 @@ int cbcg_pileup(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, int legacy,
  * derived MD), as cbcg_batch_upload. */
 int cbcg_derive_md(cbcg_ctx *ctx, const cbcg_batch *batch, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 
+/* ---- BAM input (DESIGN.md 5g): coordinate-sorted BAM (SAMv1 4.2 in BGZF, 4.1) as the resident batch, inflated and parsed on the
+ * device. The batch is the one cbch_read_sam gives for the SAM text a BAM reader prints for the same records: FLAG & 4 records
+ * are skipped (counted as unmapped); POS = pos + 1; chr = the loaded-reference ordinal of the refID's header name; SEQ spelled
+ * in =ACMGRSVTWYHKDBN; CIGAR as "%u%c" per operation (MIDNSHP=X), "*" for none; MD the MD:Z payload. QNAME, MAPQ, the mate
+ * fields, QUAL and the other aux fields are parsed past and dropped. Every refusal of cbcg_batch_upload then applies.
+ *   cbcg_bgzf_inflate: whole BGZF members -> their inflated concatenation (out_cap too small: CBCG_ERR_CAPACITY, *out_len the
+ *     size). Not BGZF (no gzip member with FLG.FEXTRA and a BC subfield), a BSIZE past the input or an ISIZE above 65 536:
+ *     CBCG_ERR_FORMAT; a bad deflate stream (block type 3, a bad code, a distance before the member's start, too little input,
+ *     more output than ISIZE), an ISIZE or CRC32 mismatch: CBCG_ERR_CORRUPT.
+ *   cbcg_bam_open: needs cbcg_set_reference (else CBCG_ERR_NO_REFERENCE), which also forgets what it read. `in` may be the whole
+ *     file: members are inflated from the start until the header (magic, l_text, text, n_ref, names and lengths) ends inside
+ *     them; *used receives those members' bytes, tail the record bytes after the header in the last of them (tail_cap too
+ *     small: CBCG_ERR_CAPACITY with *tail_len set). The context keeps the refID -> reference map; a name the reference lacks
+ *     is an error only when a mapped record uses it.
+ *   cbcg_batch_upload_bam: the stream carry[0, carry_len) followed by the inflated members of `in` (whole members), parsed from
+ *     offset 0, becomes the resident batch, as cbcg_batch_upload (CBCG_BAM_DERIVE_MD: a batch without MD). The bytes after the
+ *     last whole record go to tail (info->tail_len): the next call's carry, so a file can be fed in runs of whole members.
+ *     tail_cap too small: CBCG_ERR_CAPACITY with info->tail_len set, nothing made resident. Errors: no cbcg_bam_open on the
+ *     context CBCG_ERR_ARG; framing, a record whose fields do not fit its block_size, a malformed aux field before MD:Z, or a
+ *     partial record under CBCG_BAM_LAST CBCG_ERR_FORMAT; deflate, CRC or ISIZE CBCG_ERR_CORRUPT; a mapped record whose refID
+ *     is not in the reference CBCG_ERR_NO_REFERENCE; a mapped record without MD:Z (flag not set) or with l_seq 0
+ *     CBCG_ERR_INPUT. cbcg_last_error names the record's ordinal in the call's stream (the member's, for deflate errors).
+ *     Statistics: ms_h2d covers the copies, inflate, parse and K7; h2d_bytes counts `in` and the carry.
+ *   cbcg_cigar_pack_resident: cbcg_cigar_pack of the resident batch, without an upload (byte-identical for the same batch). */
+typedef struct cbcg_bam_info {
+    uint64_t n_records, n_unmapped, n_reads;   /* whole records in this call's stream; FLAG & 4 skipped; the batch */
+    uint32_t len_first, len_second;            /* l_seq of the call's first / second record, mapped or not (get_read_length); 0: none */
+    uint32_t max_len, min_len;                 /* over the batch */
+    uint64_t inflated_bytes, tail_len;         /* carry + inflated members; bytes after the last whole record */
+} cbcg_bam_info;
+#define CBCG_BAM_DERIVE_MD 1u   /* MD:Z not looked for: the batch is a batch without MD and K7 derives it (as cbch's CBCH_DERIVE_MD) */
+#define CBCG_BAM_LAST      2u   /* the members end the file: a partial record at the end is CBCG_ERR_FORMAT */
+int cbcg_bgzf_inflate(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+int cbcg_bam_open(cbcg_ctx *ctx, const uint8_t *in, uint64_t in_len, uint64_t *used,
+                  uint8_t *tail, uint64_t tail_cap, uint64_t *tail_len);
+int cbcg_batch_upload_bam(cbcg_ctx *ctx, const uint8_t *carry, uint64_t carry_len, const uint8_t *in, uint64_t in_len,
+                          uint32_t flags, cbcg_bam_info *info, uint8_t *tail, uint64_t tail_cap);
+int cbcg_cigar_pack_resident(cbcg_ctx *ctx, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+
 /* ---- device-resident variants (inputs already in HBM when the timed region starts): upload once,
  * run many times. Results stay on the device until fetched. Used by bench.py for `value`. */
 int cbcg_batch_upload(cbcg_ctx *ctx, const cbcg_batch *batch);                 /* replaces the resident batch */
